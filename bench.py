@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """Benchmark of the MapAnything feed-forward inference hot path (BASELINE.json metric: views/sec @518 px).
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--views V] [--impl ours|reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--views V] [--impl ours|reference] [--dump-outputs DIR]
     python -m torch.distributed.run --nnodes=1 --nproc-per-node N ... bench.py --gpus N ...
 
 One "step" = one forward pass over one synthetic V-view 518x518 image-only scene (random-init ViT-L + 24-layer
@@ -28,6 +28,11 @@ FLOP-normalised picture.  `--multi replicas` runs N independent 8-view scenes in
   N > 1     sharded_vs_single_rel (the sharded scene against the same scene run on each GPU alone, before timing; the run
             fails above 1e-2) and `strong` (the fixed 100-view scene of BASELINE config[3] timed on N GPUs and on one)
 `--impl reference` times the CPU oracle alone on the same scene (N = 1: the V views of the config), same metric/config.
+`--dump-outputs DIR` writes what the last timed forward step returned (see dump_outputs), so that two builds can be compared
+output for output on the same arm: an arm's inputs and weights are seeded, identical from run to run.  The two arms are not
+comparable this way: the repo arm keeps the constructors' default init, the reference arm draws init_reference_style
+weights.  The stream-K GEMM tail adds partial sums in arrival order, so the repo arm's outputs repeat to rounding only
+(amplified through the bf16 layers); MA_GEMM_STREAMK=0 makes them repeat bit for bit.
 """
 from __future__ import annotations
 
@@ -179,6 +184,32 @@ def make_host_geometry(v: int, seed: int, first_view_identity: bool = True, pin:
     return out
 
 
+DUMP_BYTES = 64 << 20  # all arrays of one --dump-outputs together
+
+
+def dump_outputs(preds, out_dir: str) -> None:
+    """Writes the per-view output dicts of one forward step as <out_dir>/<key>.npy in float32, views stacked on axis 0
+    (masks as 0 / 1).  When everything would exceed DUMP_BYTES, the per-pixel maps keep one fixed, seeded sample of pixel
+    positions (the same for every view and key, in raster order); per-view vectors are always written whole."""
+    import numpy as np
+    import torch
+
+    arrays = {k: torch.cat([p[k] for p in preds]).float().cpu().numpy() for k in preds[0]}
+    dense = [k for k, a in arrays.items() if a.shape[1:3] == (IMG, IMG)]
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_BYTES:
+        per_pixel = sum(arrays[k].nbytes for k in dense) // (IMG * IMG)
+        keep = (DUMP_BYTES - (total - per_pixel * IMG * IMG)) // per_pixel
+        pix = np.sort(np.random.default_rng(0).choice(IMG * IMG, size=keep, replace=False))
+        for k in dense:
+            a = arrays[k]
+            arrays[k] = a.reshape(a.shape[0], IMG * IMG, *a.shape[3:])[:, pix]
+    out = Path(out_dir)
+    out.mkdir(parents=True, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(out / f"{k}.npy", a)
+
+
 def bench_config(v: int, gpus: int, multi: str, multimodal: bool, shard: bool):
     """The `config` object: identical for both arms of the same invocation."""
     v_scene = v * gpus if shard else v
@@ -198,7 +229,7 @@ def build_oracle():
 
 def run_reference(args):
     """The reference arm: the fp32 CPU oracle of the path on the host cores, all threads, on the SAME scene as the repo arm
-    at N = 1 (all args.views views; the number of steps shrinks to fit the time budget, not the scene).  For N > 1 the
+    at N = 1 (all args.views views; the warm-up shrinks to fit a time budget, the timed steps are --steps).  For N > 1 the
     repo arm's scene has views x N views; the CPU arm runs the first `args.views` of them and says so."""
     import torch
 
@@ -220,20 +251,27 @@ def run_reference(args):
                                              "cam_prob": 1.0})
     else:
         views = [{"img": im, "data_norm_type": ["dinov2"]} for im in imgs]
+    preds = []   # --dump-outputs: what the latest step returned
 
     def step():
+        preds.clear()
         t0 = time.perf_counter()
         with torch.no_grad():
-            model(views)
-        return time.perf_counter() - t0
+            out = model(views)
+        t = time.perf_counter() - t0
+        if args.dump_outputs:
+            preds.append(out)
+        return t
 
-    t_first = step()  # warm-up (also sizes the run: the whole arm must end within a few minutes)
+    t_first = step()  # warm-up (also sizes the rest of the warm-up: a CPU step takes tens of seconds)
     budget = 200.0
     warm = max(0, min(args.warmup - 1, int(0.25 * budget / max(t_first, 1e-3))))
     for _ in range(warm):
         step()
-    steps = max(1, min(args.steps, int(0.75 * budget / max(t_first, 1e-3))))
+    steps = args.steps
     times = [step() for _ in range(steps)]
+    if preds:
+        dump_outputs(preds.pop(), args.dump_outputs)
     t = sum(times) / len(times)
     vps = sample_views / t
     same = sample_views == scene
@@ -483,6 +521,12 @@ def run_ours(args):
     def fwd_step():
         return model(dev_views)
 
+    kept = []   # --dump-outputs: what the latest timed forward step returned
+
+    def fwd_step_kept():
+        kept.clear()   # the previous step's outputs are freed before this step runs, as with fwd_step
+        kept.append(fwd_step())
+
     d2h_keys = ("pts3d", "conf", "mask", "camera_poses", "intrinsics", "metric_scaling_factor")
 
     host_out = []   # pinned result buffers, allocated on the first step and reused (what a serving loop does)
@@ -525,7 +569,7 @@ def run_ours(args):
         fwd_step()
     with ClockSampler(local_rank) as clocks:
         launches0 = ops.LAUNCHES
-        ms_fwd = timed(fwd_step, args.steps)
+        ms_fwd = timed(fwd_step_kept if args.dump_outputs else fwd_step, args.steps)
         launches = ops.LAUNCHES - launches0
         # instrumented pass of the same step for the per-kernel roofline (events around every GEMM launch)
         # (single stream for this pass: with the encoder's two view groups on two streams the kernels overlap and the
@@ -543,6 +587,9 @@ def run_ours(args):
         for _ in range(2):
             e2e_step()
         ms_e2e = timed(e2e_step, args.steps)
+    if kept and rank == 0:
+        dump_outputs(kept[0], args.dump_outputs)
+    kept.clear()
     ms_step = ms_fwd / args.steps
     vps = world * V / (ms_step * 1e-3)
     e2e_ms_step = ms_e2e / args.steps
@@ -672,7 +719,14 @@ def main():
                     help="N = 1: replay the step as one captured CUDA graph (model.enable_cuda_graphs(); small scenes are launch-bound)")
     ap.add_argument("--no-strong", action="store_true", help="N > 1: skip the fixed 100-view strong-scaling record")
     ap.add_argument("--profile-mode", action="store_true", help="1 warm-up + 1 step only, for ncu captures (prints no bench line)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the outputs of the last timed forward step (rank 0's views) as DIR/<key>.npy, float32, "
+                         f"at most {DUMP_BYTES >> 20} MB in all")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.profile_mode:
+        ap.error("--profile-mode times nothing: there are no outputs for --dump-outputs")
     if args.impl == "reference":
         # torchrun exports OMP_NUM_THREADS=1; the reference arm gets every host core (set before torch is imported)
         os.environ["OMP_NUM_THREADS"] = str(os.cpu_count() or 1)

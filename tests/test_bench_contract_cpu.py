@@ -45,3 +45,41 @@ def test_roofline_denominators_and_traffic_lookup(bench):
     # the committed ncu summary of the dominant GEMM launch: within 1.5x of its algorithmic 120.6 MB
     assert traffic is not None and 0.5 * 120.6e6 < traffic < 1.5 * 120.6e6, (traffic, note)
     assert "profiles/" in note
+
+
+def test_dump_outputs_fits_the_budget_with_a_fixed_pixel_sample(bench, tmp_path):
+    """--dump-outputs on the forward() dicts of 5 views at 518 px (70 MB of outputs): float32 files within the budget, the
+    same seeded pixel sample for every view and key, per-view vectors whole, identical from run to run."""
+    import numpy as np
+    import torch
+
+    V, S = 5, bench.IMG
+    P = S * S
+
+    def view(i):
+        px = (torch.arange(P, dtype=torch.float32) + i * P).view(1, S, S)   # every value names its view and pixel
+        return {"pts3d": px[..., None].repeat(1, 1, 1, 3), "pts3d_cam": px[..., None].repeat(1, 1, 1, 3),
+                "ray_directions": px[..., None].repeat(1, 1, 1, 3), "depth_along_ray": px[..., None], "conf": px.clone(),
+                "non_ambiguous_mask_logits": -px, "non_ambiguous_mask": px % 2 == 1,
+                "cam_trans": torch.full((1, 3), float(i)), "cam_quats": torch.full((1, 4), float(i)),
+                "metric_scaling_factor": torch.ones(1, 1)}
+
+    preds = [view(i) for i in range(V)]
+    bench.dump_outputs(preds, str(tmp_path / "a"))
+    bench.dump_outputs(preds, str(tmp_path / "b"))
+    got = {f.stem: np.load(f) for f in (tmp_path / "a").glob("*.npy")}
+    assert set(got) == set(preds[0])
+    assert all(a.dtype == np.float32 for a in got.values())
+    assert 0.95 * bench.DUMP_BYTES < sum(a.nbytes for a in got.values()) <= bench.DUMP_BYTES
+    for k, a in got.items():
+        assert np.array_equal(a, np.load(tmp_path / "b" / f"{k}.npy")), k
+    assert np.array_equal(got["cam_quats"], np.repeat(np.arange(V, dtype=np.float32)[:, None], 4, 1))
+    assert got["metric_scaling_factor"].shape == (V, 1)
+    pix = got["conf"][0]
+    n = pix.size
+    assert 0 < n < P and np.all(np.diff(pix) > 0)
+    for i in range(V):
+        assert np.array_equal(got["conf"][i], pix + i * P)
+        assert np.array_equal(got["pts3d"][i], np.repeat((pix + i * P)[:, None], 3, 1))
+        assert np.array_equal(got["non_ambiguous_mask"][i], (pix + i * P) % 2)
+    assert got["depth_along_ray"].shape == (V, n, 1)
