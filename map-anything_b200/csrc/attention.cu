@@ -1,21 +1,19 @@
 // Flash-style attention forward for sm_100a (head_dim 64, bf16 in/out, fp32 softmax + accumulate).
 //
-// One CTA = one 128-row query tile of one head of one sequence; two CTAs are resident per SM (<=113 KB
-// smem, 256 TMEM columns each) so that one CTA's softmax overlaps the other's tensor-core work.
-//
-//   warp 0      : TMEM alloc + TMA producer (Q once, K/V tiles through a 2-stage mbarrier ring)
-//   warp 1      : MMA issuer.  S = Q.K^T  (tcgen05.mma 128x128x16, K-major A/B, 4 per tile) into TMEM,
-//                 PV = P.V      (tcgen05.mma 128x64x16, A = P from smem, B = V MN-major, 8 per tile)
-//   warps 2..5  : softmax / accumulate, one query row per thread.  Pass 1 reads S from TMEM for the row
-//                 max, pass 2 re-reads it, exponentiates, writes P (bf16) into the 128B-swizzled smem
-//                 operand buffer.  The PV product of the PREVIOUS tile is folded into the fp32 register
-//                 accumulator (O = O*alpha + PV) while the tensor core works on the current tile.
+// Three forward kernels share one pipeline: a TMA producer warp streams Q once and K / V tiles through an mbarrier ring, an
+// MMA issuer warp computes S = Q.K^T (tcgen05.mma, K-major A / B) into tensor memory and accumulates O += P.V in tensor
+// memory (A = P from tensor memory, B = V MN-major), and a softmax warpgroup -- one query row per thread -- reads S into
+// registers, exponentiates it against a lazily updated integer reference maximum and writes P (bf16 pairs) to tensor memory.
+//   v2  two 128-row query tiles per CTA sharing every K / V tile, one CTA per SM, 128-key steps, the exponential phases of
+//       the two softmax warpgroups alternating (ping-pong): long sequences, key segments, carried state, kv split;
+//   v3  one query tile per CTA, three CTAs per SM, 64-key steps: up to 4096 keys when v5 does not apply;
+//   v5  persistent CTAs with two independent query-tile streams in ping-pong: plain attention over many short sequences.
+// attention_merge_kernel joins partial softmax states (kv split, view-sharded global attention).  ma_attention_fwd_ex picks
+// the kernel from the call's shape (the measurements behind each threshold are given there).
 //
 // Sequences are contiguous row ranges of a token-major matrix ([tokens][heads*64] slices of the fused
 // qkv GEMM output, so no head permute/copy is ever materialised).  Keys past kv_len are masked to -inf
 // (TMA zero-fills rows beyond the tensor; rows that belong to the next sequence are masked the same way).
-#include <stdlib.h>
-
 #include "host_common.h"
 #include "ptx.cuh"
 
@@ -24,11 +22,7 @@ namespace ma {
 constexpr int ATT_BM = 128;
 constexpr int ATT_BN = 128;
 constexpr int ATT_D = 64;
-constexpr int ATT_THREADS = 192;
-constexpr int ATT_STAGES = 2;
-constexpr int ATT_TILE_BYTES = 128 * 64 * 2;  // 16 KB: Q, one K stage, one V stage, half of P
-constexpr int ATT_SMEM_BYTES = ATT_TILE_BYTES * (1 + 2 * ATT_STAGES + 2) + 256;
-constexpr int ATT_TMEM_COLS = 256;            // S: [0,128)  PV0: [128,192)  PV1: [192,256)
+constexpr int ATT_TILE_BYTES = 128 * 64 * 2;  // 16 KB: a Q tile or a 128-row K / V stage
 
 struct AttnParams {
   __nv_bfloat16* out;
@@ -53,18 +47,22 @@ struct AttnParams {
   // kv_split > 1: the kv tile range is cut into kv_split equal parts, each handled by its own CTA, which writes its
   // partial softmax state to state_o + part * split_stride_o / state_m + part * split_stride_m (ma_attention_merge joins
   // them).  Doubles / triples the CTA count when (query blocks x heads) fills the last wave of SMs badly.
-  int pingpong;              // two-tile kernel: alternate the exponential phases of the two softmax warpgroups
+  // v2 alternates the exponential phases of its two query tiles whenever it has two; the host always sets 1.  Read at run
+  // time on purpose: with the condition known at compile time ptxas schedules v2's exponential phase differently and the
+  // kernel measured ~1.3 % slower on the global-attention shapes (B200, same-box A/B).
+  int pingpong;
   int kv_split, split_from;  // CTAs of slots >= split_from are split (tail-only splitting); 0 = every slot
   int64_t split_stride_o, split_stride_m;
 };
 
-// Cursor over the kv tiles of all segments, in segment order.
+// Cursor over the BN-row kv tiles of all segments, in segment order.
+template <int BN>
 struct KvCursor {
   int seg = 0, jj = 0;
-  __device__ __forceinline__ int row0(const AttnParams& p) const { return p.seg_row0[seg] + jj * ATT_BN; }
-  __device__ __forceinline__ int valid(const AttnParams& p) const { return p.seg_len[seg] - jj * ATT_BN; }
+  __device__ __forceinline__ int row0(const AttnParams& p) const { return p.seg_row0[seg] + jj * BN; }
+  __device__ __forceinline__ int valid(const AttnParams& p) const { return p.seg_len[seg] - jj * BN; }
   __device__ __forceinline__ void next(const AttnParams& p) {
-    if ((jj + 1) * ATT_BN < p.seg_len[seg]) ++jj;
+    if ((jj + 1) * BN < p.seg_len[seg]) ++jj;
     else { ++seg; jj = 0; }
   }
   __device__ __forceinline__ void skip(const AttnParams& p, int n) {
@@ -72,381 +70,36 @@ struct KvCursor {
   }
 };
 
-__global__ void __launch_bounds__(ATT_THREADS, 2)
-attention_fwd_tcgen05_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
-                             const __grid_constant__ CUtensorMap tmap_v, const AttnParams p) {
-  extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sQ = smem;
-  uint8_t* sK = sQ + ATT_TILE_BYTES;
-  uint8_t* sV = sK + ATT_STAGES * ATT_TILE_BYTES;
-  uint8_t* sP = sV + ATT_STAGES * ATT_TILE_BYTES;  // two 16 KB K-major sub-tiles (kv 0..63, 64..127)
-  uint64_t* bars = reinterpret_cast<uint64_t*>(sP + 2 * ATT_TILE_BYTES);
-  uint64_t* q_full = bars;
-  uint64_t* k_full = bars + 1;
-  uint64_t* k_empty = k_full + ATT_STAGES;
-  uint64_t* v_full = k_empty + ATT_STAGES;
-  uint64_t* v_empty = v_full + ATT_STAGES;
-  uint64_t* s_full = v_empty + ATT_STAGES;
-  uint64_t* s_empty = s_full + 1;
-  uint64_t* p_full = s_empty + 1;
-  uint64_t* p_empty = p_full + 1;
-  uint64_t* pv_full = p_empty + 1;   // [2]
-  uint64_t* pv_empty = pv_full + 2;  // [2]
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(pv_empty + 2);
-
-  const int warp = __shfl_sync(0xffffffff, threadIdx.x >> 5, 0);
-  const int lane = lane_id();
-  const int q0 = blockIdx.x * ATT_BM;
-  const int head = blockIdx.y;
-  const int seq = blockIdx.z;
-  const int n_kv_tiles = p.n_kv_tiles;
-
-  if (threadIdx.x == 0 && (smem_u32(smem) & 1023u) != 0) {
-    printf("[ma] attention: dynamic smem base not 1024-byte aligned\n");
-    __trap();
-  }
-  if (warp == 1 && lane == 0) {
-    mbar_init(q_full, 1);
-    for (int s = 0; s < ATT_STAGES; ++s) {
-      mbar_init(&k_full[s], 1);
-      mbar_init(&k_empty[s], 1);
-      mbar_init(&v_full[s], 1);
-      mbar_init(&v_empty[s], 1);
-    }
-    mbar_init(s_full, 1);
-    mbar_init(s_empty, 4);
-    mbar_init(p_full, 4);
-    mbar_init(p_empty, 1);
-    for (int i = 0; i < 2; ++i) {
-      mbar_init(&pv_full[i], 1);
-      mbar_init(&pv_empty[i], 4);
-    }
-    fence_barrier_init();
-  }
-  if (warp == 0) {
-    if (lane == 0) {
-      prefetch_tmap(&tmap_q);
-      prefetch_tmap(&tmap_k);
-      prefetch_tmap(&tmap_v);
-    }
-    __syncwarp();
-    tmem_alloc(tmem_slot, ATT_TMEM_COLS);
-    tmem_relinquish();
-  }
-  tc_fence_before();
-  __syncthreads();
-  tc_fence_after();
-  const uint32_t tmem_base = *tmem_slot;
-  const uint32_t tmem_s = tmem_base;
-  const uint32_t tmem_pv = tmem_base + 128;
-
-  if (warp == 0) {
-    if (lane == 0) {
-      const int q_row = static_cast<int>(seq * p.q_seq_stride) + q0;
-      const int kv_row0 = static_cast<int>(seq * p.kv_seq_stride);
-      mbar_arrive_expect_tx(q_full, ATT_TILE_BYTES);
-      tma_load_2d(sQ, &tmap_q, q_full, p.q_col0 + head * ATT_D, q_row);
-      KvCursor cur;
-      for (int j = 0; j < n_kv_tiles; ++j, cur.next(p)) {
-        const int st = j % ATT_STAGES;
-        const uint32_t ph = (j / ATT_STAGES) & 1;
-        const int row = kv_row0 + cur.row0(p);
-        mbar_wait(&k_empty[st], ph ^ 1);
-        mbar_arrive_expect_tx(&k_full[st], ATT_TILE_BYTES);
-        tma_load_2d(sK + st * ATT_TILE_BYTES, &tmap_k, &k_full[st], p.k_col0 + head * ATT_D, row);
-        mbar_wait(&v_empty[st], ph ^ 1);
-        mbar_arrive_expect_tx(&v_full[st], ATT_TILE_BYTES);
-        tma_load_2d(sV + st * ATT_TILE_BYTES, &tmap_v, &v_full[st], p.v_col0 + head * ATT_D, row);
-      }
-    }
-  } else if (warp == 1) {
-    if (lane == 0) {
-      constexpr uint32_t idesc_s = make_idesc_bf16(ATT_BM, ATT_BN, 0, 0);
-      constexpr uint32_t idesc_pv = make_idesc_bf16(ATT_BM, ATT_D, 0, 1);  // B (= V) is MN-major
-      const uint32_t q_addr = smem_u32(sQ);
-      const uint32_t p_addr = smem_u32(sP);
-
-      auto issue_s = [&](int j) {
-        const int st = j % ATT_STAGES;
-        const uint32_t ph = (j / ATT_STAGES) & 1;
-        mbar_wait(&k_full[st], ph);
-        mbar_wait(s_empty, (j & 1) ^ 1);  // softmax has drained S of tile j-1
-        tc_fence_after();
-        const uint32_t k_addr = smem_u32(sK + st * ATT_TILE_BYTES);
-#pragma unroll
-        for (int k = 0; k < ATT_D / 16; ++k) {
-          umma_bf16_ss(tmem_s, make_smem_desc_sw128(q_addr + k * 32, 16, 1024),
-                       make_smem_desc_sw128(k_addr + k * 32, 16, 1024), idesc_s, k != 0 ? 1u : 0u);
-        }
-        umma_commit(&k_empty[st]);
-        umma_commit(s_full);
-      };
-
-      mbar_wait(q_full, 0);
-      issue_s(0);
-      for (int j = 0; j < n_kv_tiles; ++j) {
-        if (j + 1 < n_kv_tiles) issue_s(j + 1);
-        const int st = j % ATT_STAGES;
-        const uint32_t ph = (j / ATT_STAGES) & 1;
-        const int buf = j & 1;
-        mbar_wait(p_full, j & 1);
-        mbar_wait(&v_full[st], ph);
-        mbar_wait(&pv_empty[buf], ((j >> 1) & 1) ^ 1);
-        tc_fence_after();
-        const uint32_t v_addr = smem_u32(sV + st * ATT_TILE_BYTES);
-#pragma unroll
-        for (int k = 0; k < ATT_BN / 16; ++k) {
-          const uint64_t adesc = make_smem_desc_sw128(p_addr + (k >> 2) * ATT_TILE_BYTES + (k & 3) * 32, 16, 1024);
-          const uint64_t bdesc = make_smem_desc_sw128(v_addr + k * 2048, 1024, 1024);
-          umma_bf16_ss(tmem_pv + buf * ATT_D, adesc, bdesc, idesc_pv, k != 0 ? 1u : 0u);
-        }
-        umma_commit(&v_empty[st]);
-        umma_commit(p_empty);
-        umma_commit(&pv_full[buf]);
-      }
-    }
-  } else {
-    // ---- softmax / accumulate warps: thread <-> query row -------------------------------------
-    const int quarter = warp & 3;
-    const int row = quarter * 32 + lane;
-    const uint32_t lane_base = static_cast<uint32_t>(quarter * 32) << 16;
-    float o_acc[ATT_D];
-#pragma unroll
-    for (int i = 0; i < ATT_D; ++i) o_acc[i] = 0.f;
-    float m_run = -INFINITY;  // running max of raw scores
-    float l_run = 0.f;
-    float alpha_prev = 1.f;
-    const int q_idx = q0 + row;
-    const int64_t q_grow = static_cast<int64_t>(seq) * p.q_seq_stride + q_idx;
-    if ((p.flags & MA_ATTN_STATE_IN) && q_idx < p.q_len) {
-      const float4* so = reinterpret_cast<const float4*>(p.state_o + q_grow * p.ld_state_o + head * ATT_D);
-#pragma unroll
-      for (int i = 0; i < ATT_D / 4; ++i) {
-        const float4 t = so[i];
-        o_acc[4 * i] = t.x; o_acc[4 * i + 1] = t.y; o_acc[4 * i + 2] = t.z; o_acc[4 * i + 3] = t.w;
-      }
-      m_run = p.state_m[q_grow * p.num_heads + head];
-      l_run = 1.f;
-    }
-    const uint32_t sw = static_cast<uint32_t>(row & 7);
-    uint8_t* p_row = sP + row * 128;
-
-    auto fold_pv = [&](int j, float alpha) {
-      const int buf = j & 1;
-      mbar_wait(&pv_full[buf], (j >> 1) & 1);
-      tc_fence_after();
-#pragma unroll
-      for (int c = 0; c < ATT_D; c += 32) {
-        uint32_t v[32];
-        tmem_ld_32x32b_x32(tmem_pv + lane_base + buf * ATT_D + c, v);
-        tmem_ld_wait();
-#pragma unroll
-        for (int i = 0; i < 32; ++i) o_acc[c + i] = fmaf(o_acc[c + i], alpha, __uint_as_float(v[i]));
-      }
-      tc_fence_before();
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&pv_empty[buf]);
-    };
-
-    KvCursor cur;
-    for (int j = 0; j < n_kv_tiles; ++j, cur.next(p)) {
-      const int kv_valid = cur.valid(p);  // >= 1; < 128 only on the last tile of a segment
-      mbar_wait(s_full, j & 1);
-      tc_fence_after();
-      // pass 1: row max
-      float m_tile = -INFINITY;
-#pragma unroll 1
-      for (int c = 0; c < ATT_BN; c += 32) {
-        uint32_t v[32];
-        tmem_ld_32x32b_x32(tmem_s + lane_base + c, v);
-        tmem_ld_wait();
-        if (kv_valid >= c + 32) {
-#pragma unroll
-          for (int i = 0; i < 32; ++i) m_tile = fmaxf(m_tile, __uint_as_float(v[i]));
-        } else {
-#pragma unroll
-          for (int i = 0; i < 32; ++i)
-            if (c + i < kv_valid) m_tile = fmaxf(m_tile, __uint_as_float(v[i]));
-        }
-      }
-      const float m_new = fmaxf(m_run, m_tile);
-      const float alpha = fast_exp2((m_run - m_new) * p.scale_log2);
-      const float m_scaled = m_new * p.scale_log2;
-      m_run = m_new;
-
-      mbar_wait(p_empty, (j & 1) ^ 1);  // PV of tile j-1 has finished reading P
-      // pass 2: probabilities -> bf16 -> swizzled smem operand
-      float l_tile = 0.f;
-#pragma unroll 1
-      for (int c = 0; c < ATT_BN; c += 32) {
-        uint32_t v[32];
-        tmem_ld_32x32b_x32(tmem_s + lane_base + c, v);
-        tmem_ld_wait();
-        float e[32];
-#pragma unroll
-        for (int i = 0; i < 32; ++i) {
-          float x = fast_exp2(fmaf(__uint_as_float(v[i]), p.scale_log2, -m_scaled));
-          if (c + i >= kv_valid) x = 0.f;
-          e[i] = x;
-          l_tile += x;
-        }
-        uint8_t* dst = p_row + (c >> 6) * ATT_TILE_BYTES;
-        const uint32_t chunk0 = static_cast<uint32_t>((c & 63) >> 3);  // 16-byte chunk index inside the 128 B row
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-          uint4 pk = make_uint4(pack_bf16x2(e[8 * q + 0], e[8 * q + 1]), pack_bf16x2(e[8 * q + 2], e[8 * q + 3]),
-                                pack_bf16x2(e[8 * q + 4], e[8 * q + 5]), pack_bf16x2(e[8 * q + 6], e[8 * q + 7]));
-          *reinterpret_cast<uint4*>(dst + (((chunk0 + q) ^ sw) << 4)) = pk;
-        }
-      }
-      l_run = l_run * alpha + l_tile;
-      tc_fence_before();        // S reads are complete before the MMA warp may overwrite S
-      fence_proxy_async_smem(); // P writes visible to the tensor core (async proxy)
-      __syncwarp();
-      if (lane == 0) {
-        mbar_arrive(s_empty);
-        mbar_arrive(p_full);
-      }
-      // fold the previous tile's PV while the tensor core computes S_{j+1} and PV_j
-      if (j > 0) fold_pv(j - 1, alpha_prev);
-      alpha_prev = alpha;  // O_j = O_{j-1} * alpha_j + PV_j is applied when PV_j is folded (next iteration)
-    }
-    fold_pv(n_kv_tiles - 1, alpha_prev);
-
-    if (q_idx < p.q_len && (p.flags & MA_ATTN_STATE_OUT)) {
-      const float inv_l = 1.0f / l_run;
-      float4* so = reinterpret_cast<float4*>(p.state_o + q_grow * p.ld_state_o + head * ATT_D);
-#pragma unroll
-      for (int i = 0; i < ATT_D / 4; ++i)
-        so[i] = make_float4(o_acc[4 * i] * inv_l, o_acc[4 * i + 1] * inv_l, o_acc[4 * i + 2] * inv_l, o_acc[4 * i + 3] * inv_l);
-      p.state_m[q_grow * p.num_heads + head] = m_run + __log2f(l_run) / p.scale_log2;
-    } else if (q_idx < p.q_len) {
-      const float inv_l = 1.0f / l_run;
-      __nv_bfloat16* optr = p.out + q_grow * p.ldo + p.o_col0 + head * ATT_D;
-#pragma unroll
-      for (int q = 0; q < ATT_D / 8; ++q) {
-        uint4 pk = make_uint4(pack_bf16x2(o_acc[8 * q + 0] * inv_l, o_acc[8 * q + 1] * inv_l),
-                              pack_bf16x2(o_acc[8 * q + 2] * inv_l, o_acc[8 * q + 3] * inv_l),
-                              pack_bf16x2(o_acc[8 * q + 4] * inv_l, o_acc[8 * q + 5] * inv_l),
-                              pack_bf16x2(o_acc[8 * q + 6] * inv_l, o_acc[8 * q + 7] * inv_l));
-        reinterpret_cast<uint4*>(optr)[q] = pk;
-      }
-    }
-  }
-
-  tc_fence_before();
-  __syncthreads();
-  if (warp == 0) {
-    tc_fence_after();
-    tmem_dealloc(tmem_base, ATT_TMEM_COLS);
-  }
-}
-
-
 // ================================================================================================================
-// v2: one CTA per SM works on TWO 128-row query tiles (A, B) that share every K/V tile, with
-//   * 8 softmax warps (4 per query tile), one thread per query ROW: the 128 scores of the row are read from TMEM ONCE
-//     into registers and S is released immediately (the tensor core starts Q.K^T of the next tile while the
-//     exponentials of this one are computed); row maximum and row sum are thread-local, so the softmax warps never
-//     synchronise with each other -- the two query tiles are free-running streams whose TMEM-read and MUFU phases
-//     interleave on each SM sub-partition (TMEM reads, 64 B/clk/SM, cost as many cycles as the exponentials);
-//   * the output accumulator O kept in TMEM (PV accumulates in place) with LAZY rescaling: O and the running sum are
-//     rescaled only when the row maximum grew by more than 2^8; until then probabilities are computed against the stale
-//     maximum (they stay <= 256, exact in fp32 / bf16 range), so the common tile does no correction work at all;
-//   * P written by the softmax warps straight into TENSOR MEMORY (tcgen05.st, two bf16 per 32-bit column) and consumed
-//     by the P.V MMA as a TMEM A operand: shared memory carries only Q, K and V.  With P staged in shared memory the
-//     kernel was bound by shared-memory bandwidth (Q.K^T reads 8 KB and P.V 6 KB per MMA, plus 32 KB of P writes per
-//     tile -- about as many cycles as the exponentials themselves on a 128 B/clk port);
-//   * a 4-deep K and V ring shared by both query tiles (half the L2 -> smem traffic per query row).
-// Same interface / masking / segment / carried-state semantics as the v1 kernel above.
+// Softmax-row steps shared by the kernels.  A softmax thread owns one query row; mref is the row's reference maximum in
+// log2 units (score * scale * log2 e), kept INTEGER valued.  Any reference works (it cancels in O / l), so the true running
+// maximum is only tracked to within the lazy-rescale slack.
 // ================================================================================================================
-// NQT = query tiles per CTA.  2: one CTA per SM, the layout described above (long sequences: K/V shared by 256 query
-// rows).  1: one tile per CTA and TWO CTAs per SM (half the TMEM / smem / warps each): the same two free-running softmax
-// streams per SM, but a CTA's prologue (TMEM allocation, Q / first K,V loads, pipeline ramp) and epilogue overlap the other
-// CTA's steady state, and work is scheduled in 128-row units -- better for the 11-tile sequences of a single view.
-template <int NQT>
-struct A2Cfg {
-  static constexpr int THREADS = NQT == 2 ? 11 * 32 : 6 * 32;  // warp 0 TMA, warp 1 (/10) MMA issuer of tile A (/B), then softmax
-  static constexpr int KV_STAGES = NQT == 2 ? 4 : 3;
-  static constexpr int SMEM_BYTES = (NQT + 2 * KV_STAGES) * ATT_TILE_BYTES + 512;
-  static constexpr int TMEM_COLS = NQT * 256;  // S tiles [0, 128 NQT), O tiles [128 NQT, 192 NQT), P tiles [192 NQT, 256 NQT)
-  static constexpr int O_COL0 = NQT * 128, P_COL0 = NQT * 192;
-  static constexpr int BMQ = NQT * ATT_BM;     // query rows per CTA
-};
 constexpr float A2_RESCALE_LOG2 = 8.0f;
-constexpr int A2_DEFAULT_POLY = 0;  // of 16 score pairs on the FMA pipe: 0 measured fastest (DESIGN.md section 5)
 
 // Exponentials of one 32-column chunk of a score row (16 register pairs) -> 16 packed bf16x2 probabilities + row-sum
-// contribution.  NPOLY of every 16 pairs are evaluated on the FMA pipe (exp2_poly_pair), the rest on the MUFU; all
-// arithmetic that can be is issued as packed fp32x2 (half the issue slots).  mref is an integer-valued reference maximum
-// in log2 units: p = 2^(s * sl2 - mref).
-__host__ __device__ constexpr bool a2_poly_slot(int i, int npoly) { return ((i * npoly) & 15) < npoly; }
-
-template <int NPOLY>
-__device__ __forceinline__ void a2_exp_chunk(const uint32_t (&v)[32], uint32_t* dst, uint64_t sl2_2, uint64_t nm2, uint64_t k2,
-                                             float smin, uint64_t (&acc)[4]) {
+// contribution, p = 2^(s * sl2 - mref) on the MUFU; all arithmetic that can be is issued as packed fp32x2 (half the issue
+// slots).
+__device__ __forceinline__ void a2_exp_chunk(const uint32_t (&v)[32], uint32_t* dst, uint64_t sl2_2, uint64_t nm2,
+                                             uint64_t (&acc)[4]) {
   // Written stage by stage over all pairs of the chunk (not pair by pair): every stage is a run of independent
   // instructions.  (ptxas re-schedules the result freely -- the SASS consumes each pair of exponentials two MUFU
   // instructions after issuing them whatever the source order, volatile asm included.)
-  constexpr int NP = NPOLY > 0 ? NPOLY : 1;
   constexpr int AHEAD = 1;
-  uint64_t s2[16], r2[NP], g2[NP];
+  uint64_t s2[16];
   float ea[16], eb[16];
-  int pi = 0;
 #pragma unroll
-  for (int i = 0; i < 16; ++i) {
-    if (a2_poly_slot(i, NPOLY)) {
-      s2[i] = pack2(fmaxf(__uint_as_float(v[2 * i]), smin), fmaxf(__uint_as_float(v[2 * i + 1]), smin));
-    } else {
-      s2[i] = ffma2(pack2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1])), sl2_2, nm2);
-    }
-  }
-  if (NPOLY > 0) {
-    const uint64_t c3 = pack2(0.055205505f, 0.055205505f), c2 = pack2(0.24261397f, 0.24261397f);
-    const uint64_t c1 = pack2(0.69325477f, 0.69325477f), c0 = pack2(0.9999277f, 0.9999277f);
-    pi = 0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i)
-      if (a2_poly_slot(i, NPOLY)) r2[pi++] = ffma2(s2[i], sl2_2, k2);
-    pi = 0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i)
-      if (a2_poly_slot(i, NPOLY)) { g2[pi] = fsub2(k2, r2[pi]); ++pi; }
-    pi = 0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i)
-      if (a2_poly_slot(i, NPOLY)) { g2[pi] = ffma2(s2[i], sl2_2, g2[pi]); ++pi; }
-    pi = 0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i)
-      if (a2_poly_slot(i, NPOLY)) { s2[i] = ffma2(g2[pi], c3, c2); ++pi; }
-    pi = 0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i)
-      if (a2_poly_slot(i, NPOLY)) { s2[i] = ffma2(s2[i], g2[pi], c1); ++pi; }
-    pi = 0;
-#pragma unroll
-    for (int i = 0; i < 16; ++i)
-      if (a2_poly_slot(i, NPOLY)) { s2[i] = ffma2(s2[i], g2[pi], c0); ++pi; }
-  }
-  auto evaluate = [&](int i, int& pidx) {
+  for (int i = 0; i < 16; ++i) s2[i] = ffma2(pack2(__uint_as_float(v[2 * i]), __uint_as_float(v[2 * i + 1])), sl2_2, nm2);
+  auto evaluate = [&](int i) {
     unpack2(s2[i], ea[i], eb[i]);
-    if (a2_poly_slot(i, NPOLY)) {
-      float ra, rb;
-      unpack2(r2[pidx++], ra, rb);
-      ea[i] = __uint_as_float(__float_as_uint(ea[i]) + (__float_as_uint(ra) << 23));
-      eb[i] = __uint_as_float(__float_as_uint(eb[i]) + (__float_as_uint(rb) << 23));
-    } else {
-      ea[i] = fast_exp2(ea[i]);
-      eb[i] = fast_exp2(eb[i]);
-    }
+    ea[i] = fast_exp2(ea[i]);
+    eb[i] = fast_exp2(eb[i]);
   };
-  pi = 0;
 #pragma unroll
-  for (int i = 0; i < AHEAD; ++i) evaluate(i, pi);
+  for (int i = 0; i < AHEAD; ++i) evaluate(i);
 #pragma unroll
   for (int i = 0; i < 16; ++i) {
-    if (i + AHEAD < 16) evaluate(i + AHEAD, pi);
+    if (i + AHEAD < 16) evaluate(i + AHEAD);
     acc[i & 3] = fadd2(acc[i & 3], pack2(ea[i], eb[i]));
     dst[i] = pack_bf16x2(ea[i], eb[i]);
   }
@@ -497,16 +150,164 @@ __device__ __forceinline__ void a2_exp_row_pipelined(uint32_t (&v0)[32], uint32_
   consume(v3, 3);
 }
 
-template <int NQT, int NPOLY>
-__global__ void __launch_bounds__(A2Cfg<NQT>::THREADS, NQT == 2 ? 1 : 2)
+// Carried state (normalised O, m' in raw score units, l = 1) -> the row's O columns in tensor memory, re-expressed against an
+// integer reference maximum (set in mref); returns l.  Rows past the sequence load zeros.
+__device__ __forceinline__ float load_state_row(const AttnParams& p, int64_t q_grow, int head, bool q_ok, uint32_t tmem_o,
+                                                float& mref) {
+  const float sl2 = p.scale_log2;
+  const float m_in = q_ok ? p.state_m[q_grow * p.num_heads + head] : 0.f;
+  mref = rintf(m_in * sl2);
+  const float c_in = q_ok ? fast_exp2(fmaf(m_in, sl2, -mref)) : 0.f;  // in [2^-0.5, 2^0.5]
+  const float* so = p.state_o + q_grow * p.ld_state_o + head * ATT_D;
+#pragma unroll 1
+  for (int c = 0; c < ATT_D; c += 8) {
+    uint32_t o[8];
+#pragma unroll
+    for (int i = 0; i < 8; ++i) o[i] = 0u;
+    if (q_ok) {
+      const float4 x = *reinterpret_cast<const float4*>(so + c), y = *reinterpret_cast<const float4*>(so + c + 4);
+      o[0] = __float_as_uint(x.x * c_in); o[1] = __float_as_uint(x.y * c_in); o[2] = __float_as_uint(x.z * c_in);
+      o[3] = __float_as_uint(x.w * c_in); o[4] = __float_as_uint(y.x * c_in); o[5] = __float_as_uint(y.y * c_in);
+      o[6] = __float_as_uint(y.z * c_in); o[7] = __float_as_uint(y.w * c_in);
+    }
+    tmem_st_32x32b_x8(tmem_o + c, o);
+  }
+  tmem_st_wait();
+  tc_fence_before();
+  return c_in;
+}
+
+// The 128 scores of the row (S in tensor memory, four 32-column loads) -> v0..v3, and their maximum.  Columns at or past
+// kv_valid are set to -inf (ex2(-inf) = 0 exactly).  The maximum is reduced chunk by chunk UNDER the tensor-memory loads
+// of the following chunks (a warp reads tensor memory at ~45 B/clk: the four 4 KB loads take ~360 clk whatever the order),
+// and S is released (s_empty) as soon as it is in registers, so the tensor core may overwrite it with the next Q.K^T.
+__device__ __forceinline__ float read_scores_max(uint32_t tmem_s, int kv_valid, uint64_t* s_empty, int lane, uint32_t (&v0)[32],
+                                                 uint32_t (&v1)[32], uint32_t (&v2)[32], uint32_t (&v3)[32]) {
+  float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
+  auto chunk_max = [&](uint32_t (&v)[32], int c0, float& m) {
+    if (kv_valid < c0 + 32) {
+#pragma unroll
+      for (int i = 0; i < 32; ++i)
+        if (c0 + i >= kv_valid) v[i] = __float_as_uint(-INFINITY);
+    }
+    float a = -INFINITY, b = -INFINITY;
+#pragma unroll
+    for (int i = 0; i < 16; ++i) {
+      a = fmaxf(a, __uint_as_float(v[i]));
+      b = fmaxf(b, __uint_as_float(v[16 + i]));
+    }
+    m = fmaxf(a, b);
+  };
+  tmem_ld_32x32b_x32(tmem_s, v0);
+  tmem_ld_wait();
+  tmem_ld_32x32b_x32(tmem_s + 32, v1);
+  chunk_max(v0, 0, mx4[0]);
+  tmem_ld_wait();
+  tmem_ld_32x32b_x32(tmem_s + 64, v2);
+  chunk_max(v1, 32, mx4[1]);
+  tmem_ld_wait();
+  tmem_ld_32x32b_x32(tmem_s + 96, v3);
+  chunk_max(v2, 64, mx4[2]);
+  tmem_ld_wait();
+  tc_fence_before();
+  __syncwarp();
+  if (lane == 0) mbar_arrive(s_empty);
+  chunk_max(v3, 96, mx4[3]);
+  return fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
+}
+
+// Lazy rescale: mref moves to the tile maximum mt2 (log2 units) on the row's first tile, and afterwards only when mt2 exceeds
+// it by more than 2^8; until then probabilities are computed against the stale reference (they stay <= 256, exact in fp32
+// and in bf16's range), so the common tile does no correction work at all.  When any row of the warp moves, O (tensor
+// memory) and l are scaled by the exact power of two 2^(old - new), after P.V of the previous tile has completed (p_empty
+// with parity prev_parity, waited for when has_prev).  Returns whether it waited for that P.V.
+__device__ __forceinline__ bool lazy_rescale(float mt2, bool first, bool has_prev, uint64_t* p_empty, uint32_t prev_parity,
+                                             uint32_t tmem_o, float& mref, float& l_run) {
+  float m_new = mref;
+  bool need = false;
+  if (first) m_new = rintf(mt2);
+  else if (mt2 - mref > A2_RESCALE_LOG2) { need = true; m_new = rintf(mt2); }
+  bool waited = false;
+  if (__any_sync(0xffffffffu, need)) {
+    if (has_prev) { mbar_wait(p_empty, prev_parity); waited = true; }
+    tc_fence_after();
+    const float alpha = need ? fast_exp2(mref - m_new) : 1.f;
+#pragma unroll 1
+    for (int c = 0; c < ATT_D; c += 8) {  // rare path
+      uint32_t o[8];
+      tmem_ld_32x32b_x8(tmem_o + c, o);
+      tmem_ld_wait();
+#pragma unroll
+      for (int i = 0; i < 8; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
+      tmem_st_32x32b_x8(tmem_o + c, o);
+    }
+    tmem_st_wait();
+    tc_fence_before();
+    l_run *= alpha;
+  }
+  mref = m_new;
+  return waited;
+}
+
+// Row epilogue, once the row's last P.V has completed: O (tensor memory) / l -> the bf16 output row, or, with write_state,
+// the fp32 state row of partial `part` and m' = (mref + log2 l) / (scale log2 e).  Rows past the sequence store nothing.
+__device__ __forceinline__ void store_row(const AttnParams& p, uint32_t tmem_o, bool q_ok, bool write_state, int part,
+                                          int64_t q_grow, int head, float mref, float l_run) {
+  const float inv_l = 1.0f / l_run;
+  uint32_t o[32];
+#pragma unroll 1
+  for (int c = 0; c < ATT_D; c += 32) {
+    tmem_ld_32x32b_x32(tmem_o + c, o);
+    tmem_ld_wait();
+    if (q_ok && write_state) {
+      float4* so = reinterpret_cast<float4*>(p.state_o + part * p.split_stride_o + q_grow * p.ld_state_o + head * ATT_D + c);
+#pragma unroll
+      for (int i = 0; i < 8; ++i)
+        so[i] = make_float4(__uint_as_float(o[4 * i]) * inv_l, __uint_as_float(o[4 * i + 1]) * inv_l,
+                            __uint_as_float(o[4 * i + 2]) * inv_l, __uint_as_float(o[4 * i + 3]) * inv_l);
+    } else if (q_ok) {
+      __nv_bfloat16* optr = p.out + q_grow * p.ldo + p.o_col0 + head * ATT_D + c;
+#pragma unroll
+      for (int q = 0; q < 4; ++q)
+        reinterpret_cast<uint4*>(optr)[q] =
+            make_uint4(pack_bf16x2(__uint_as_float(o[8 * q]) * inv_l, __uint_as_float(o[8 * q + 1]) * inv_l),
+                       pack_bf16x2(__uint_as_float(o[8 * q + 2]) * inv_l, __uint_as_float(o[8 * q + 3]) * inv_l),
+                       pack_bf16x2(__uint_as_float(o[8 * q + 4]) * inv_l, __uint_as_float(o[8 * q + 5]) * inv_l),
+                       pack_bf16x2(__uint_as_float(o[8 * q + 6]) * inv_l, __uint_as_float(o[8 * q + 7]) * inv_l));
+    }
+  }
+  if (q_ok && write_state)
+    p.state_m[part * p.split_stride_m + q_grow * p.num_heads + head] = (mref + __log2f(l_run)) * (1.0f / p.scale_log2);
+}
+
+
+// ================================================================================================================
+// v2: one CTA per SM works on TWO 128-row query tiles (A, B) that share every K/V tile, with
+//   * 8 softmax warps (4 per query tile), one thread per query ROW: the 128 scores of the row are read from TMEM ONCE
+//     into registers and S is released immediately (the tensor core starts Q.K^T of the next tile while the
+//     exponentials of this one are computed); row maximum and row sum are thread-local, and the two query tiles' softmax
+//     warpgroups meet only at a pair of named barriers that make their exponential phases alternate (ping-pong);
+//   * the output accumulator O kept in TMEM (PV accumulates in place) with LAZY rescaling (lazy_rescale);
+//   * P written by the softmax warps straight into TENSOR MEMORY (tcgen05.st, two bf16 per 32-bit column) and consumed
+//     by the P.V MMA as a TMEM A operand: shared memory carries only Q, K and V.  With P staged in shared memory the
+//     kernel was bound by shared-memory bandwidth (Q.K^T reads 8 KB and P.V 6 KB per MMA, plus 32 KB of P writes per
+//     tile -- about as many cycles as the exponentials themselves on a 128 B/clk port);
+//   * a 4-deep K and V ring shared by both query tiles (half the L2 -> smem traffic per query row).
+// Handles key segments, carried state (in and out) and the kv split.
+// ================================================================================================================
+constexpr int A2_THREADS = 11 * 32;  // warp 0 TMA, warp 1 (/10) MMA issuer of tile A (/B), warps 2..9 softmax
+constexpr int A2_KV_STAGES = 4;
+constexpr int A2_SMEM_BYTES = (2 + 2 * A2_KV_STAGES) * ATT_TILE_BYTES + 512;
+constexpr int A2_TMEM_COLS = 512;  // S tiles [0, 256), O tiles [256, 384), P tiles [384, 512)
+constexpr int A2_O_COL0 = 256, A2_P_COL0 = 384;
+constexpr int A2_BMQ = 2 * ATT_BM;  // query rows per CTA
+
+__global__ void __launch_bounds__(A2_THREADS, 1)
 attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                         const __grid_constant__ CUtensorMap tmap_v, const AttnParams p) {
-  using Cfg = A2Cfg<NQT>;
-  constexpr int A2_KV_STAGES = Cfg::KV_STAGES;
-  constexpr int A2_TMEM_COLS = Cfg::TMEM_COLS;
   extern __shared__ __align__(1024) uint8_t smem[];
-  uint8_t* sQ = smem;                                     // [NQT] tiles
-  uint8_t* sK = sQ + NQT * ATT_TILE_BYTES;                // [stages]
+  uint8_t* sQ = smem;                                     // [2] tiles
+  uint8_t* sK = sQ + 2 * ATT_TILE_BYTES;                  // [stages]
   uint8_t* sV = sK + A2_KV_STAGES * ATT_TILE_BYTES;       // [stages]
   uint64_t* bars = reinterpret_cast<uint64_t*>(sV + A2_KV_STAGES * ATT_TILE_BYTES);
   uint64_t* q_full = bars;
@@ -525,9 +326,8 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
   // 1-D grid over (query block, head, sequence).  All FULL 256-row query blocks come first, the ragged last block of
   // every (head, sequence) -- cheaper, often a single 128-row tile -- is scheduled at the end where it fills the tail
   // wave instead of occupying an SM slot for a full block's duration in the middle (1370-token views: 5 full + 1 ragged).
-  const int n_full = p.q_len / (Cfg::BMQ);
+  const int n_full = p.q_len / A2_BMQ;
   const int hs_count = p.num_heads * p.num_seqs;
-  const int n_slots = ((p.q_len + Cfg::BMQ - 1) / (Cfg::BMQ)) * hs_count;
   // slots [0, split_from) run as one CTA each; every later slot -- the ones that would form the badly filled last wave
   // of SMs -- is cut into kv_split CTAs that each take a share of the key range and leave a partial softmax state
   int bid = blockIdx.x, part = 0, nparts = 1;
@@ -537,7 +337,6 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     part = r % p.kv_split;
     nparts = p.kv_split;
   }
-  (void)n_slots;
   int qb, hs;
   if (bid < n_full * hs_count) {
     qb = bid % n_full;
@@ -546,13 +345,13 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     qb = n_full;
     hs = bid - n_full * hs_count;
   }
-  const int q0 = qb * Cfg::BMQ;
+  const int q0 = qb * A2_BMQ;
   const int head = hs % p.num_heads;
   const int seq = hs / p.num_heads;
   const int kv_tile0 = static_cast<int>((static_cast<int64_t>(part) * p.n_kv_tiles) / nparts);
   const int n_kv_tiles = static_cast<int>((static_cast<int64_t>(part + 1) * p.n_kv_tiles) / nparts) - kv_tile0;
   const bool write_state = (p.flags & MA_ATTN_STATE_OUT) != 0 || nparts > 1;
-  const int n_qt = (NQT == 2 && q0 + ATT_BM < p.q_len) ? 2 : 1;  // query tile B is skipped when it lies past the sequence
+  const int n_qt = q0 + ATT_BM < p.q_len ? 2 : 1;  // query tile B is skipped when it lies past the sequence
   const bool state_in = (p.flags & MA_ATTN_STATE_IN) != 0;
 
   if (threadIdx.x == 0 && (smem_u32(smem) & 1023u) != 0) {
@@ -595,10 +394,10 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     if (lane == 0) {
       const int q_row = static_cast<int>(seq * p.q_seq_stride) + q0;
       const int kv_row0 = static_cast<int>(seq * p.kv_seq_stride);
-      mbar_arrive_expect_tx(q_full, NQT * ATT_TILE_BYTES);
+      mbar_arrive_expect_tx(q_full, 2 * ATT_TILE_BYTES);
       tma_load_2d(sQ, &tmap_q, q_full, p.q_col0 + head * ATT_D, q_row);
-      if (NQT == 2) tma_load_2d(sQ + ATT_TILE_BYTES, &tmap_q, q_full, p.q_col0 + head * ATT_D, q_row + ATT_BM);
-      KvCursor cur;
+      tma_load_2d(sQ + ATT_TILE_BYTES, &tmap_q, q_full, p.q_col0 + head * ATT_D, q_row + ATT_BM);
+      KvCursor<ATT_BN> cur;
       cur.skip(p, kv_tile0);
       for (int j = 0; j < n_kv_tiles; ++j, cur.next(p)) {
         const int st = j % A2_KV_STAGES;
@@ -621,8 +420,8 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
       constexpr uint32_t idesc_pv = make_idesc_bf16(ATT_BM, ATT_D, 0, 1);  // B (= V) is MN-major
       const uint32_t q_addr = smem_u32(sQ + t * ATT_TILE_BYTES);
       const uint32_t tmem_s = tmem_base + t * ATT_BN;
-      const uint32_t tmem_o = tmem_base + Cfg::O_COL0 + t * ATT_D;
-      const uint32_t p_tmem = tmem_base + Cfg::P_COL0 + t * 64;  // 128 kv x bf16 = 64 columns, 8 columns per K = 16 step
+      const uint32_t tmem_o = tmem_base + A2_O_COL0 + t * ATT_D;
+      const uint32_t p_tmem = tmem_base + A2_P_COL0 + t * 64;  // 128 kv x bf16 = 64 columns, 8 columns per K = 16 step
       auto issue_qk = [&](int j) {
         const int st = j % A2_KV_STAGES;
         const uint32_t ph = (j / A2_KV_STAGES) & 1;
@@ -663,91 +462,33 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
       const int row = quarter * 32 + lane;
       const uint32_t lane_base = static_cast<uint32_t>(quarter * 32) << 16;
       const uint32_t tmem_s = tmem_base + lane_base + t * ATT_BN;
-      const uint32_t tmem_o = tmem_base + lane_base + Cfg::O_COL0 + t * ATT_D;
-      const uint32_t tmem_p = tmem_base + lane_base + Cfg::P_COL0 + t * 64;
+      const uint32_t tmem_o = tmem_base + lane_base + A2_O_COL0 + t * ATT_D;
+      const uint32_t tmem_p = tmem_base + lane_base + A2_P_COL0 + t * 64;
       const int q_idx = q0 + t * ATT_BM + row;
       const bool q_ok = q_idx < p.q_len;
       const int64_t q_grow = static_cast<int64_t>(seq) * p.q_seq_stride + q_idx;
       const float sl2 = p.scale_log2;
 
-      // mref: reference maximum of the row in log2 units (score * scale * log2 e), kept INTEGER valued so that the
-      // polynomial exp2 path needs no per-row fraction; any reference works (it cancels in O / l), so the true running
-      // maximum is only tracked to within the lazy-rescale slack
       float mref = 0.f, l_run = 0.f;
-      if (state_in) {
-        // carried state = (normalised O, m' in raw score units, l = 1): re-express it against the integer reference
-        const float m_in = q_ok ? p.state_m[q_grow * p.num_heads + head] : 0.f;
-        mref = rintf(m_in * sl2);
-        const float c_in = q_ok ? fast_exp2(fmaf(m_in, sl2, -mref)) : 0.f;  // in [2^-0.5, 2^0.5]
-        const float* so = p.state_o + q_grow * p.ld_state_o + head * ATT_D;
-#pragma unroll 1
-        for (int c = 0; c < ATT_D; c += 8) {
-          uint32_t o[8];
-#pragma unroll
-          for (int i = 0; i < 8; ++i) o[i] = 0u;
-          if (q_ok) {
-            const float4 x = *reinterpret_cast<const float4*>(so + c), y = *reinterpret_cast<const float4*>(so + c + 4);
-            o[0] = __float_as_uint(x.x * c_in); o[1] = __float_as_uint(x.y * c_in); o[2] = __float_as_uint(x.z * c_in);
-            o[3] = __float_as_uint(x.w * c_in); o[4] = __float_as_uint(y.x * c_in); o[5] = __float_as_uint(y.y * c_in);
-            o[6] = __float_as_uint(y.z * c_in); o[7] = __float_as_uint(y.w * c_in);
-          }
-          tmem_st_32x32b_x8(tmem_o + c, o);
-        }
-        l_run = c_in;
-        tmem_st_wait();
-        tc_fence_before();
-      }
-      const uint64_t sl2_2 = pack2(sl2, sl2);
-      const float inv_sl2 = 1.0f / sl2;
-      // Ping-pong (two-tile form only): left free-running, the two softmax warps of a scheduler settle IN PHASE -- both read
+      if (state_in) l_run = load_state_row(p, q_grow, head, q_ok, tmem_o, mref);
+      // Ping-pong: left free-running, the two softmax warps of a scheduler settle IN PHASE -- both read
       // S and reduce maxima together, then share the MUFU pipe at half rate each: period n + 2e per tile pair (n ~ 1150 clk
       // outside the exponential phase, e = 1024 clk of MUFU work; ncu: MUFU 71 % = 2e / (n + 2e)).  Two named barriers force
       // the exponential phases of the two warpgroups to ALTERNATE, so one owns the pipe at full rate while the other does its
-      // tensor-memory reads, maximum and stores: period n + e.
-      const bool pingpong = NQT == 2 && n_qt == 2 && p.pingpong != 0;
+      // tensor-memory reads, maximum and stores: period n + e.  (p.pingpong is always 1; see AttnParams.)
+      const bool pingpong = n_qt == 2 && p.pingpong != 0;
 
-      KvCursor cur;
+      KvCursor<ATT_BN> cur;
       cur.skip(p, kv_tile0);
       for (int j = 0; j < n_kv_tiles; ++j, cur.next(p)) {
         const int kv_valid = cur.valid(p);
         mbar_wait(&s_full[t], j & 1);
         tc_fence_after();
         uint32_t v0[32], v1[32], v2[32], v3[32];  // the 128 scores of this thread's row
-        // the row maximum is reduced chunk by chunk UNDER the tensor-memory loads of the following chunks (a warp reads
-        // tensor memory at ~45 B/clk: the four 4 KB loads take ~360 clk whatever the order)
-        float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-        auto chunk_max = [&](uint32_t (&v)[32], int c0, float& m) {
-          if (kv_valid < c0 + 32) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (c0 + i >= kv_valid) v[i] = __float_as_uint(-INFINITY);
-          }
-          float a = -INFINITY, b = -INFINITY;
-#pragma unroll
-          for (int i = 0; i < 16; ++i) {
-            a = fmaxf(a, __uint_as_float(v[i]));
-            b = fmaxf(b, __uint_as_float(v[16 + i]));
-          }
-          m = fmaxf(a, b);
-        };
-        tmem_ld_32x32b_x32(tmem_s, v0);
-        tmem_ld_wait();
-        tmem_ld_32x32b_x32(tmem_s + 32, v1);
-        chunk_max(v0, 0, mx4[0]);
-        tmem_ld_wait();
-        tmem_ld_32x32b_x32(tmem_s + 64, v2);
-        chunk_max(v1, 32, mx4[1]);
-        tmem_ld_wait();
-        tmem_ld_32x32b_x32(tmem_s + 96, v3);
-        chunk_max(v2, 64, mx4[2]);
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(&s_empty[t]);  // S is in registers: the tensor core may overwrite it
-        chunk_max(v3, 96, mx4[3]);
-        const float m_tile = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
+        const float m_tile = read_scores_max(tmem_s, kv_valid, &s_empty[t], lane, v0, v1, v2, v3);
 
-        // lazy rescale: adopt the new maximum only when it grew by more than 2^8
+        // lazy rescale (the steps of lazy_rescale, written out: called as a function here, ptxas schedules the
+        // exponential phase below differently and the kernel measured ~1 % slower)
         const float mt2 = m_tile * sl2;
         float m_new = mref;
         bool need = false;
@@ -774,39 +515,22 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
         mref = m_new;
 
         // exponentials -> bf16 pairs (two per 32-bit P column), stored to tensor memory chunk by chunk (16 columns = 32
-        // scores at a time, so the packed probabilities never occupy more than 16 registers).  P.V of the previous tile
-        // still reads the single P buffer: it was issued a whole tile ago, so this wait is normally already satisfied
-        // P.V of tile j-1 still reads the single P buffer.  Measured placements of this wait (TFLOP/s, 8- / 24-view global
-        // shape, two-tile ping-pong form): here, before the exponential phase 756 / 850; at the first P store inside the phase
-        // 665 / 751; after the phase with all four stores deferred 592 / 668.
+        // scores at a time, so the packed probabilities never occupy more than 16 registers).  P.V of tile j-1 still reads
+        // the single P buffer: it was issued a whole tile ago, so this wait is normally already satisfied.  Measured
+        // placements of this wait (TFLOP/s, 8- / 24-view global shape): here, before the exponential phase 756 / 850; at the
+        // first P store inside the phase 665 / 751; after the phase with all four stores deferred 592 / 668.
         if (!waited && j > 0) mbar_wait(&p_empty[t], (j - 1) & 1);
         tc_fence_after();
         uint64_t acc[4] = {0ull, 0ull, 0ull, 0ull};
-        const uint64_t nm2 = pack2(-mref, -mref);
-        if (NPOLY == 0 || kv_valid < ATT_BN) {  // masked columns are -inf: MUFU only (ex2(-inf) = 0 exactly)
-          float mref_turn = mref;
-          // wait for the turn; the barrier carries the reference maximum so that no exponential can be scheduled above it
-          if (pingpong && (t == 1 || j > 0)) asm volatile("bar.sync %1, 256;" : "+f"(mref_turn) : "r"(1 + t) : "memory");
-          a2_exp_row_pipelined(v0, v1, v2, v3, sl2, mref_turn, acc,
-                               [&](int chunk, const uint32_t (&pk)[16]) { tmem_st_32x32b_x16(tmem_p + 16 * chunk, pk); },
-                               [&](uint32_t& last) {
-                                 if (pingpong && (t == 0 || j + 1 < n_kv_tiles))
-                                   asm volatile("bar.arrive %1, 256;" : "+r"(last) : "r"(2 - t) : "memory");
-                               });
-        } else {
-          const float kk = 12582912.0f - mref;           // 1.5 * 2^23 - mref, exact for |mref| < 2^22
-          const uint64_t k2 = pack2(kk, kk);
-          const float smin = (mref - 120.0f) * inv_sl2;  // keeps the exponent field of 2^n in range
-          uint32_t pk[16];
-          a2_exp_chunk<NPOLY>(v0, pk, sl2_2, nm2, k2, smin, acc);
-          tmem_st_32x32b_x16(tmem_p, pk);
-          a2_exp_chunk<NPOLY>(v1, pk, sl2_2, nm2, k2, smin, acc);
-          tmem_st_32x32b_x16(tmem_p + 16, pk);
-          a2_exp_chunk<NPOLY>(v2, pk, sl2_2, nm2, k2, smin, acc);
-          tmem_st_32x32b_x16(tmem_p + 32, pk);
-          a2_exp_chunk<NPOLY>(v3, pk, sl2_2, nm2, k2, smin, acc);
-          tmem_st_32x32b_x16(tmem_p + 48, pk);
-        }
+        float mref_turn = mref;
+        // wait for the turn; the barrier carries the reference maximum so that no exponential can be scheduled above it
+        if (pingpong && (t == 1 || j > 0)) asm volatile("bar.sync %1, 256;" : "+f"(mref_turn) : "r"(1 + t) : "memory");
+        a2_exp_row_pipelined(v0, v1, v2, v3, sl2, mref_turn, acc,
+                             [&](int chunk, const uint32_t (&pk)[16]) { tmem_st_32x32b_x16(tmem_p + 16 * chunk, pk); },
+                             [&](uint32_t& last) {
+                               if (pingpong && (t == 0 || j + 1 < n_kv_tiles))
+                                 asm volatile("bar.arrive %1, 256;" : "+r"(last) : "r"(2 - t) : "memory");
+                             });
         {
           float a0, a1, a2, a3;
           unpack2(fadd2(acc[0], acc[1]), a0, a1);
@@ -819,34 +543,9 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
         if (lane == 0) mbar_arrive(&p_full[t]);
       }
 
-      // ---- finish: normalise, store ----
       mbar_wait(&p_empty[t], (n_kv_tiles - 1) & 1);
       tc_fence_after();
-      const float inv_l = 1.0f / l_run;
-      uint32_t o[32];
-#pragma unroll 1
-      for (int c = 0; c < ATT_D; c += 32) {
-        tmem_ld_32x32b_x32(tmem_o + c, o);
-        tmem_ld_wait();
-        if (q_ok && write_state) {
-          float4* so = reinterpret_cast<float4*>(p.state_o + part * p.split_stride_o + q_grow * p.ld_state_o + head * ATT_D + c);
-#pragma unroll
-          for (int i = 0; i < 8; ++i)
-            so[i] = make_float4(__uint_as_float(o[4 * i]) * inv_l, __uint_as_float(o[4 * i + 1]) * inv_l,
-                                __uint_as_float(o[4 * i + 2]) * inv_l, __uint_as_float(o[4 * i + 3]) * inv_l);
-        } else if (q_ok) {
-          __nv_bfloat16* optr = p.out + q_grow * p.ldo + p.o_col0 + head * ATT_D + c;
-#pragma unroll
-          for (int q = 0; q < 4; ++q)
-            reinterpret_cast<uint4*>(optr)[q] =
-                make_uint4(pack_bf16x2(__uint_as_float(o[8 * q]) * inv_l, __uint_as_float(o[8 * q + 1]) * inv_l),
-                           pack_bf16x2(__uint_as_float(o[8 * q + 2]) * inv_l, __uint_as_float(o[8 * q + 3]) * inv_l),
-                           pack_bf16x2(__uint_as_float(o[8 * q + 4]) * inv_l, __uint_as_float(o[8 * q + 5]) * inv_l),
-                           pack_bf16x2(__uint_as_float(o[8 * q + 6]) * inv_l, __uint_as_float(o[8 * q + 7]) * inv_l));
-        }
-      }
-      if (q_ok && write_state)
-        p.state_m[part * p.split_stride_m + q_grow * p.num_heads + head] = (mref + __log2f(l_run)) * inv_sl2;
+      store_row(p, tmem_o, q_ok, write_state, part, q_grow, head, mref, l_run);
     }
   }
 
@@ -863,11 +562,11 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
 // v5: persistent CTAs, two INDEPENDENT attention streams per CTA with ping-pong (many short sequences: encoder / frame
 // attention, 1370 keys = 11 steps per 128-row query tile).
 //   * a work item is one 128-row query tile of one (sequence, head); stream t of CTA c takes the items r * 2G + 2c + t
-//     (G = grid size = number of SMs), so 1408 items fill 296 streams in 4.76 -> 5 rounds (the one-tile-per-CTA kernels:
+//     (G = grid size = number of SMs), so 1408 items fill 296 streams in 4.76 -> 5 rounds (v3, three CTAs per SM:
 //     3.17 -> 4 waves of 444 resident CTAs);
 //   * each stream has its own Q tile, its own 3-stage K / V ring, its own TMA producer warp, MMA issuer warp and softmax
-//     warpgroup, its own S / O / P tensor-memory columns -- two v2<1> pipelines inside one CTA.  What the CTA buys is the
-//     ping-pong of v2<2>: the two softmax warps of a scheduler alternate their exponential phases through a pair of named
+//     warpgroup, its own S / O / P tensor-memory columns (v2's column map) -- two one-tile pipelines inside one CTA.  What
+//     the CTA buys is v2's ping-pong: the two softmax warps of a scheduler alternate their exponential phases through a pair of named
 //     barriers instead of falling into step (MUFU 82 % instead of 63 - 71 % busy);
 //   * every barrier phase runs on across items (global step counters), the producer loads the next item's Q as soon as the
 //     last Q.K^T of the current one is issued, and the MMA issuer issues the next item's first Q.K^T right after the current
@@ -875,7 +574,7 @@ attention_fwd_v2_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
 //     OTHER stream's exponential phase.
 //   * both streams execute the same number of ping-pong turns (equal steps per item; a stream without an item in the last
 //     round only passes the turn), so every bar.sync has its bar.arrive.
-// No key segments, carried state or kv split here (ma_attention_fwd routes those to v2).
+// No key segments, carried state or kv split here (ma_attention_fwd_ex routes those to v3 / v2).
 // ================================================================================================================
 constexpr int A5_THREADS = 12 * 32;  // warp 0 / 11: TMA producer of stream 0 / 1; warp 1 / 10: MMA issuer; warps 2-5 / 6-9: softmax
 constexpr int A5_KV_STAGES = 3;
@@ -885,7 +584,6 @@ constexpr int A5_BARS_PER_STREAM = 6 + 4 * A5_KV_STAGES;
 __global__ void __launch_bounds__(A5_THREADS, 1)
 attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                         const __grid_constant__ CUtensorMap tmap_v, const AttnParams p) {
-  using Cfg = A2Cfg<2>;  // tensor-memory column map of the two-tile kernel
   extern __shared__ __align__(1024) uint8_t smem[];
   uint8_t* sQ = smem;                                              // [2] tiles
   uint8_t* sKV = sQ + 2 * ATT_TILE_BYTES;                          // per stream: K[stages], V[stages]
@@ -927,7 +625,7 @@ attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
       prefetch_tmap(&tmap_v);
     }
     __syncwarp();
-    tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
+    tmem_alloc(tmem_slot, A2_TMEM_COLS);
     tmem_relinquish();
   }
   tc_fence_before();
@@ -994,8 +692,8 @@ attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
       constexpr uint32_t idesc_pv = make_idesc_bf16(ATT_BM, ATT_D, 0, 1);  // B (= V) is MN-major
       const uint32_t q_addr = smem_u32(sQt);
       const uint32_t tmem_s = tmem_base + t * ATT_BN;
-      const uint32_t tmem_o = tmem_base + Cfg::O_COL0 + t * ATT_D;
-      const uint32_t p_tmem = tmem_base + Cfg::P_COL0 + t * 64;
+      const uint32_t tmem_o = tmem_base + A2_O_COL0 + t * ATT_D;
+      const uint32_t p_tmem = tmem_base + A2_P_COL0 + t * 64;
       auto issue_qk = [&](int gs, bool last_of_item) {
         const int st = gs % A5_KV_STAGES;
         const uint32_t ph = (gs / A5_KV_STAGES) & 1;
@@ -1051,8 +749,8 @@ attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     const int row = quarter * 32 + lane;
     const uint32_t lane_base = static_cast<uint32_t>(quarter * 32) << 16;
     const uint32_t tmem_s = tmem_base + lane_base + t * ATT_BN;
-    const uint32_t tmem_o = tmem_base + lane_base + Cfg::O_COL0 + t * ATT_D;
-    const uint32_t tmem_p = tmem_base + lane_base + Cfg::P_COL0 + t * 64;
+    const uint32_t tmem_o = tmem_base + lane_base + A2_O_COL0 + t * ATT_D;
+    const uint32_t tmem_p = tmem_base + lane_base + A2_P_COL0 + t * 64;
     const float sl2 = p.scale_log2;
     const int kv_len = p.seg_len[0];
     int gs0 = 0;
@@ -1080,64 +778,9 @@ attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
         mbar_wait(s_full, gs & 1);
         tc_fence_after();
         uint32_t v0[32], v1[32], v2[32], v3[32];  // the 128 scores of this thread's row
-        float mx4[4] = {-INFINITY, -INFINITY, -INFINITY, -INFINITY};
-        auto chunk_max = [&](uint32_t (&v)[32], int c0, float& m) {
-          if (kv_valid < c0 + 32) {
-#pragma unroll
-            for (int i = 0; i < 32; ++i)
-              if (c0 + i >= kv_valid) v[i] = __float_as_uint(-INFINITY);
-          }
-          float a = -INFINITY, bb = -INFINITY;
-#pragma unroll
-          for (int i = 0; i < 16; ++i) {
-            a = fmaxf(a, __uint_as_float(v[i]));
-            bb = fmaxf(bb, __uint_as_float(v[16 + i]));
-          }
-          m = fmaxf(a, bb);
-        };
-        tmem_ld_32x32b_x32(tmem_s, v0);
-        tmem_ld_wait();
-        tmem_ld_32x32b_x32(tmem_s + 32, v1);
-        chunk_max(v0, 0, mx4[0]);
-        tmem_ld_wait();
-        tmem_ld_32x32b_x32(tmem_s + 64, v2);
-        chunk_max(v1, 32, mx4[1]);
-        tmem_ld_wait();
-        tmem_ld_32x32b_x32(tmem_s + 96, v3);
-        chunk_max(v2, 64, mx4[2]);
-        tmem_ld_wait();
-        tc_fence_before();
-        __syncwarp();
-        if (lane == 0) mbar_arrive(s_empty);  // S is in registers: the tensor core may overwrite it
-        chunk_max(v3, 96, mx4[3]);
-        const float m_tile = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3]));
-
-        // lazy rescale: adopt the new maximum only when it grew by more than 2^8
-        const float mt2 = m_tile * sl2;
-        float m_new = mref;
-        bool need = false;
-        if (j == 0) m_new = rintf(mt2);
-        else if (mt2 - mref > A2_RESCALE_LOG2) { need = true; m_new = rintf(mt2); }
-        bool waited = false;
-        if (__any_sync(0xffffffffu, need)) {
-          mbar_wait(p_empty, (gs - 1) & 1);  // j > 0 here: P.V of the previous step has completed
-          waited = true;
-          tc_fence_after();
-          const float alpha = need ? fast_exp2(mref - m_new) : 1.f;  // an exact power of two
-#pragma unroll 1
-          for (int cc = 0; cc < ATT_D; cc += 8) {  // rare path
-            uint32_t o[8];
-            tmem_ld_32x32b_x8(tmem_o + cc, o);
-            tmem_ld_wait();
-#pragma unroll
-            for (int i = 0; i < 8; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-            tmem_st_32x32b_x8(tmem_o + cc, o);
-          }
-          tmem_st_wait();
-          tc_fence_before();
-          l_run *= alpha;
-        }
-        mref = m_new;
+        const float m_tile = read_scores_max(tmem_s, kv_valid, s_empty, lane, v0, v1, v2, v3);
+        // no row moves on an item's first step, so the previous step's P.V exists whenever the rescale waits for it
+        const bool waited = lazy_rescale(m_tile * sl2, j == 0, true, p_empty, (gs - 1) & 1, tmem_o, mref, l_run);
 
         // P.V of the previous step (of this item, or the last one of the previous item -- whose completion the epilogue has
         // already waited for) still reads the single P buffer
@@ -1169,23 +812,7 @@ attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
       // ---- finish the item: normalise, store (runs under the other stream's exponential phase) ----
       mbar_wait(p_empty, (gs0 - 1) & 1);
       tc_fence_after();
-      const float inv_l = 1.0f / l_run;
-      uint32_t o[32];
-#pragma unroll 1
-      for (int cc = 0; cc < ATT_D; cc += 32) {
-        tmem_ld_32x32b_x32(tmem_o + cc, o);
-        tmem_ld_wait();
-        if (q_ok) {
-          __nv_bfloat16* optr = p.out + q_grow * p.ldo + p.o_col0 + head * ATT_D + cc;
-#pragma unroll
-          for (int q = 0; q < 4; ++q)
-            reinterpret_cast<uint4*>(optr)[q] =
-                make_uint4(pack_bf16x2(__uint_as_float(o[8 * q]) * inv_l, __uint_as_float(o[8 * q + 1]) * inv_l),
-                           pack_bf16x2(__uint_as_float(o[8 * q + 2]) * inv_l, __uint_as_float(o[8 * q + 3]) * inv_l),
-                           pack_bf16x2(__uint_as_float(o[8 * q + 4]) * inv_l, __uint_as_float(o[8 * q + 5]) * inv_l),
-                           pack_bf16x2(__uint_as_float(o[8 * q + 6]) * inv_l, __uint_as_float(o[8 * q + 7]) * inv_l));
-        }
-      }
+      store_row(p, tmem_o, q_ok, false, 0, q_grow, head, mref, l_run);
       tc_fence_before();   // the tensor-memory reads of O are ordered before the p_full arrive that lets the next P.V overwrite it
     }
   }
@@ -1194,14 +821,14 @@ attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
   __syncthreads();
   if (warp == 0) {
     tc_fence_after();
-    tmem_dealloc(tmem_base, Cfg::TMEM_COLS);
+    tmem_dealloc(tmem_base, A2_TMEM_COLS);
   }
 }
 
 
 // ================================================================================================================
 // v3: three CTAs per SM.
-//   * one 128-row query tile per CTA as in v2<1>, but key / value steps of 64 rows: a softmax thread holds 64 scores
+//   * one 128-row query tile per CTA, and key / value steps of 64 rows: a softmax thread holds 64 scores
 //     (112 registers instead of 168) and a CTA needs 64 (S) + 64 (O) + 32 (P) = 160 tensor-memory columns, taken as TWO
 //     allocations (128 + 32; a single allocation must be a power of two), so THREE CTAs fit an SM (480 of 512 columns,
 //     3 x 64 KB shared memory, 3 x 192 x 112 registers).  Every scheduler then holds three softmax warps from three
@@ -1213,9 +840,8 @@ attention_fwd_v5_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
 //     without that pipeline -- P written in place over S, 128 columns, the chain S_j -> softmax -> P_j V_j -> S_{j+1}
 //     strictly serial per CTA -- measured 494 TFLOP/s on the 8-view global shape against 766 for v2: three CTAs do not
 //     hide ~2000 clk of barrier / MMA latency per step.)
-//   * same exponentials as v2 (a2_exp_chunk): packed fp32x2 arithmetic, integer reference maximum, NPOLY of 16 pairs on
-//     the FMA pipe.
-// Same interface / masking / segment / carried-state semantics; kv_split stays with the v2 two-tile kernel.
+//   * exponentials 32 scores at a time (a2_exp_chunk): packed fp32x2 arithmetic, integer reference maximum.
+// Same interface / masking / segment / carried-state semantics as v2; the kv split is v2's alone.
 // ================================================================================================================
 constexpr int A3_BN = 64;
 constexpr int A3_STAGES = 3;
@@ -1225,20 +851,9 @@ constexpr int A3_THREADS = 6 * 32;  // warp 0: TMA producer, warp 1: MMA issuer,
 constexpr int A3_TMEM_COLS = 128;   // first allocation: S [0, 64), O [64, 128)
 constexpr int A3_TMEM_P_COLS = 32;  // second allocation: P (64 probabilities as bf16 pairs)
 
-struct Kv64Cursor {
-  int seg = 0, jj = 0;
-  __device__ __forceinline__ int row0(const AttnParams& p) const { return p.seg_row0[seg] + jj * A3_BN; }
-  __device__ __forceinline__ int valid(const AttnParams& p) const { return p.seg_len[seg] - jj * A3_BN; }
-  __device__ __forceinline__ void next(const AttnParams& p) {
-    if ((jj + 1) * A3_BN < p.seg_len[seg]) ++jj;
-    else { ++seg; jj = 0; }
-  }
-};
-
 // Registers: a scheduler (SM sub-partition) owns 16 K registers and the warps of the resident CTAs are spread over the four
 // schedulers: 3 CTAs x 6 warps = 18 warps -> one scheduler holds 5 of them -> at most 16384 / (5 x 32) = 102 registers per
 // thread, i.e. 96.  (At 104-112 registers only TWO CTAs were resident: launch__occupancy_limit_registers = 2.)
-template <int NPOLY>
 __global__ void __maxnreg__(96)
 attention_fwd_v3_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid_constant__ CUtensorMap tmap_k,
                         const __grid_constant__ CUtensorMap tmap_v, const AttnParams p) {
@@ -1324,7 +939,7 @@ attention_fwd_v3_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
       const int kv_row0 = static_cast<int>(seq * p.kv_seq_stride);
       mbar_arrive_expect_tx(q_full, ATT_TILE_BYTES);
       tma_load_2d(sQ, &tmap_q, q_full, p.q_col0 + head * ATT_D, q_row);
-      Kv64Cursor cur;
+      KvCursor<A3_BN> cur;
       for (int j = 0; j < n_kv_tiles; ++j, cur.next(p)) {
         const int st = j % A3_STAGES;
         const uint32_t ph = (j / A3_STAGES) & 1;
@@ -1386,32 +1001,10 @@ attention_fwd_v3_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
     const int64_t q_grow = static_cast<int64_t>(seq) * p.q_seq_stride + q_idx;
     const float sl2 = p.scale_log2;
     float mref = 0.f, l_run = 0.f;
-    if (state_in) {
-      const float m_in = q_ok ? p.state_m[q_grow * p.num_heads + head] : 0.f;
-      mref = rintf(m_in * sl2);
-      const float c_in = q_ok ? fast_exp2(fmaf(m_in, sl2, -mref)) : 0.f;
-      const float* so = p.state_o + q_grow * p.ld_state_o + head * ATT_D;
-#pragma unroll 1
-      for (int c = 0; c < ATT_D; c += 8) {
-        uint32_t o[8];
-#pragma unroll
-        for (int i = 0; i < 8; ++i) o[i] = 0u;
-        if (q_ok) {
-          const float4 x = *reinterpret_cast<const float4*>(so + c), y = *reinterpret_cast<const float4*>(so + c + 4);
-          o[0] = __float_as_uint(x.x * c_in); o[1] = __float_as_uint(x.y * c_in); o[2] = __float_as_uint(x.z * c_in);
-          o[3] = __float_as_uint(x.w * c_in); o[4] = __float_as_uint(y.x * c_in); o[5] = __float_as_uint(y.y * c_in);
-          o[6] = __float_as_uint(y.z * c_in); o[7] = __float_as_uint(y.w * c_in);
-        }
-        tmem_st_32x32b_x8(tmem_o + c, o);
-      }
-      l_run = c_in;
-      tmem_st_wait();
-      tc_fence_before();
-    }
+    if (state_in) l_run = load_state_row(p, q_grow, head, q_ok, tmem_o, mref);
     const uint64_t sl2_2 = pack2(sl2, sl2);
-    const float inv_sl2 = 1.0f / sl2;
 
-    Kv64Cursor cur;
+    KvCursor<A3_BN> cur;
     for (int j = 0; j < n_kv_tiles; ++j, cur.next(p)) {
       const int kv_valid = cur.valid(p);
       mbar_wait(s_full, j & 1);
@@ -1439,52 +1032,18 @@ attention_fwd_v3_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
         mx4[3] = fmaxf(mx4[3], __uint_as_float(v1[16 + i]));
       }
       const float mt2 = fmaxf(fmaxf(mx4[0], mx4[1]), fmaxf(mx4[2], mx4[3])) * sl2;
-      float m_new = mref;
-      bool need = false;
-      if (j == 0 && !state_in) m_new = rintf(mt2);
-      else if (mt2 - mref > A2_RESCALE_LOG2) { need = true; m_new = rintf(mt2); }
-      bool waited = false;
-      if (__any_sync(0xffffffffu, need)) {  // rare
-        if (j > 0) { mbar_wait(p_empty, (j - 1) & 1); waited = true; }  // P_{j-1} V_{j-1} has completed: O is quiescent
-        tc_fence_after();
-        const float alpha = need ? fast_exp2(mref - m_new) : 1.f;
-#pragma unroll 1
-        for (int c = 0; c < ATT_D; c += 8) {
-          uint32_t o[8];
-          tmem_ld_32x32b_x8(tmem_o + c, o);
-          tmem_ld_wait();
-#pragma unroll
-          for (int i = 0; i < 8; ++i) o[i] = __float_as_uint(__uint_as_float(o[i]) * alpha);
-          tmem_st_32x32b_x8(tmem_o + c, o);
-        }
-        tmem_st_wait();
-        tc_fence_before();
-        l_run *= alpha;
-      }
-      mref = m_new;
+      const bool waited = lazy_rescale(mt2, j == 0 && !state_in, j > 0, p_empty, (j - 1) & 1, tmem_o, mref, l_run);
 
       uint64_t acc[4] = {0ull, 0ull, 0ull, 0ull};
       const uint64_t nm2 = pack2(-mref, -mref);
       uint32_t pk[16];
       // the single P buffer is still read by P_{j-1} V_{j-1}: wait for it only once the first 32 exponentials are done
-      if (NPOLY == 0 || kv_valid < A3_BN) {
-        a2_exp_chunk<0>(v0, pk, sl2_2, nm2, 0ull, 0.f, acc);
-        if (!waited && j > 0) mbar_wait(p_empty, (j - 1) & 1);
-        tc_fence_after();
-        tmem_st_32x32b_x16(tmem_p, pk);
-        a2_exp_chunk<0>(v1, pk, sl2_2, nm2, 0ull, 0.f, acc);
-        tmem_st_32x32b_x16(tmem_p + 16, pk);
-      } else {
-        const float kk = 12582912.0f - mref;
-        const uint64_t k2 = pack2(kk, kk);
-        const float smin = (mref - 120.0f) * inv_sl2;
-        a2_exp_chunk<NPOLY>(v0, pk, sl2_2, nm2, k2, smin, acc);
-        if (!waited && j > 0) mbar_wait(p_empty, (j - 1) & 1);
-        tc_fence_after();
-        tmem_st_32x32b_x16(tmem_p, pk);
-        a2_exp_chunk<NPOLY>(v1, pk, sl2_2, nm2, k2, smin, acc);
-        tmem_st_32x32b_x16(tmem_p + 16, pk);
-      }
+      a2_exp_chunk(v0, pk, sl2_2, nm2, acc);
+      if (!waited && j > 0) mbar_wait(p_empty, (j - 1) & 1);
+      tc_fence_after();
+      tmem_st_32x32b_x16(tmem_p, pk);
+      a2_exp_chunk(v1, pk, sl2_2, nm2, acc);
+      tmem_st_32x32b_x16(tmem_p + 16, pk);
       {
         float a0, a1, a2, a3;
         unpack2(fadd2(acc[0], acc[1]), a0, a1);
@@ -1499,30 +1058,7 @@ attention_fwd_v3_kernel(const __grid_constant__ CUtensorMap tmap_q, const __grid
 
     mbar_wait(p_empty, (n_kv_tiles - 1) & 1);
     tc_fence_after();
-    const float inv_l = 1.0f / l_run;
-    uint32_t o[32];
-#pragma unroll 1
-    for (int c = 0; c < ATT_D; c += 32) {
-      tmem_ld_32x32b_x32(tmem_o + c, o);
-      tmem_ld_wait();
-      if (q_ok && write_state) {
-        float4* so = reinterpret_cast<float4*>(p.state_o + q_grow * p.ld_state_o + head * ATT_D + c);
-#pragma unroll
-        for (int i = 0; i < 8; ++i)
-          so[i] = make_float4(__uint_as_float(o[4 * i]) * inv_l, __uint_as_float(o[4 * i + 1]) * inv_l,
-                              __uint_as_float(o[4 * i + 2]) * inv_l, __uint_as_float(o[4 * i + 3]) * inv_l);
-      } else if (q_ok) {
-        __nv_bfloat16* optr = p.out + q_grow * p.ldo + p.o_col0 + head * ATT_D + c;
-#pragma unroll
-        for (int q = 0; q < 4; ++q)
-          reinterpret_cast<uint4*>(optr)[q] =
-              make_uint4(pack_bf16x2(__uint_as_float(o[8 * q]) * inv_l, __uint_as_float(o[8 * q + 1]) * inv_l),
-                         pack_bf16x2(__uint_as_float(o[8 * q + 2]) * inv_l, __uint_as_float(o[8 * q + 3]) * inv_l),
-                         pack_bf16x2(__uint_as_float(o[8 * q + 4]) * inv_l, __uint_as_float(o[8 * q + 5]) * inv_l),
-                         pack_bf16x2(__uint_as_float(o[8 * q + 6]) * inv_l, __uint_as_float(o[8 * q + 7]) * inv_l));
-      }
-    }
-    if (q_ok && write_state) p.state_m[q_grow * p.num_heads + head] = (mref + __log2f(l_run)) * inv_sl2;
+    store_row(p, tmem_o, q_ok, write_state, 0, q_grow, head, mref, l_run);
   }
 
   tc_fence_before();
@@ -1634,7 +1170,7 @@ extern "C" int ma_attention_fwd_ex(const void* q, int64_t ldq, int64_t q_rows, i
   p.num_seqs = num_seqs;
   p.flags = flags;
   p.kv_split = 1;
-  p.pingpong = 0;
+  p.pingpong = 1;
   p.split_from = 0;
   p.split_stride_o = 0;
   p.split_stride_m = 0;
@@ -1693,104 +1229,63 @@ extern "C" int ma_attention_fwd_ex(const void* q, int64_t ldq, int64_t q_rows, i
   p.v_col0 = v_col0;
   p.o_col0 = o_col0;
   p.scale_log2 = softmax_scale * 1.4426950408889634f;
-  const int dev = current_device();
-  static const bool use_v1 = [] {
-    const char* e = getenv("MA_ATTN_V1");
-    return e != nullptr && e[0] == '1';
-  }();
-  if (use_v1) {
-    static bool configured[MA_MAX_DEVICES] = {};  // the large-shared-memory opt-in is per device
-    if (!configured[dev]) {
-      MA_CHECK_CUDA(cudaFuncSetAttribute(attention_fwd_tcgen05_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize,
-                                         ATT_SMEM_BYTES));
-      configured[dev] = true;
-    }
-    MA_REQUIRE(p.kv_split == 1, "ma_attention_fwd: kv_split is not supported by the v1 kernel");
-    dim3 grid((q_len + ATT_BM - 1) / ATT_BM, num_heads, num_seqs);
-    attention_fwd_tcgen05_kernel<<<grid, ATT_THREADS, ATT_SMEM_BYTES, static_cast<cudaStream_t>(stream)>>>(tq, tk, tv, p);
+  // Kernel choice (same-box A/B on a B200, tools/bench_kernels.py, TFLOP/s):
+  //  * v5 for plain attention over many short sequences, once the (128-row query tile x head x sequence) items fill the
+  //    2 x SMs streams for at least three rounds.  Against v3: 8 x 16 x 1370 (encoder, 1408 items) 637 vs 572, 8 x 12 x 1369
+  //    (frame, 1056 items) 592 vs 539, 24 x 16 x 1370 698 vs 655; 3 x 12 x 1369 (396 items, 1.3 rounds) 411 vs 468.
+  //  * v3 for other calls with up to 4096 keys and no kv split.  Against one query tile per CTA in the v2 layout:
+  //    1370-key sequences (encoder, frame attention) 586 / 552 vs 572 / 535 at 8 views, 658 / 634 vs 622 / 604 at 24 views;
+  //    one long sequence (global attention) 740 vs 766 at 8 views, 786 vs 799 at 24.
+  //  * v2 otherwise (long sequences, kv split): K / V shared by 256 query rows and ping-pong, MUFU 82 % busy instead of
+  //    71 %: 881 vs 795 for one tile per CTA at 16 views, 850 vs 799 at 24; at 8 views 756 vs 766 as a plain launch (516
+  //    CTAs = 3.5 waves of 148), 860 with the last partial wave split over the key range (Engine._pick_tail_split).
+  using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, AttnParams);
+  const int sms = device_sm_count();
+  const int n_items = ((q_len + ATT_BM - 1) / ATT_BM) * num_heads * num_seqs;
+  const bool short_keys = kv_len <= 4096 && p.kv_split == 1;
+  int kernel;  // index into `configured` below
+  KernelFn fn;
+  int threads, smem_bytes, ctas;
+  if (short_keys && p.n_segs == 1 && p.seg_row0[0] == 0 && !(flags & (MA_ATTN_STATE_IN | MA_ATTN_STATE_OUT)) &&
+      n_items >= 6 * sms) {
+    kernel = 0;
+    fn = attention_fwd_v5_kernel;
+    threads = A5_THREADS;
+    smem_bytes = A5_SMEM_BYTES;
+    ctas = sms < (n_items + 1) / 2 ? sms : (n_items + 1) / 2;
+  } else if (short_keys) {
+    kernel = 1;
+    fn = attention_fwd_v3_kernel;
+    threads = A3_THREADS;
+    smem_bytes = A3_SMEM_BYTES;
+    ctas = n_items;
+    // key / value boxes of 64 rows
+    const uint32_t box64[2] = {ATT_D, A3_BN};
+    uint64_t dims[2] = {(uint64_t)ldk, (uint64_t)kv_rows};
+    uint64_t str[1] = {(uint64_t)ldk * 2};
+    int rc = make_tmap_bf16(&tk, k, 2, dims, str, box64);
+    if (rc != MA_OK) return rc;
+    dims[0] = (uint64_t)ldv;
+    str[0] = (uint64_t)ldv * 2;
+    rc = make_tmap_bf16(&tv, v, 2, dims, str, box64);
+    if (rc != MA_OK) return rc;
   } else {
-    // one query tile per CTA, two CTAs per SM: measured faster than two tiles per CTA on every shape of the path (B200,
-    // same-box A/B: encoder 521-571 vs 446-462, frame 535-540 vs 482, 8-view global 765 vs 709 TFLOP/s); the two-tile
-    // form is kept for the kv-split mode and for A/B runs (MA_ATTN_NQT=2)
-    static const int nqt_env = [] {
-      const char* e = getenv("MA_ATTN_NQT");
-      return e ? atoi(e) : 0;
-    }();
-    // pairs of every 16 whose exponential runs on the FMA pipe (a2_exp_chunk); MA_ATTN_POLY selects a variant for A/B runs
-    static const int poly_env = [] {
-      const char* e = getenv("MA_ATTN_POLY");
-      return e ? atoi(e) : -1;
-    }();
-    using KernelFn = void (*)(CUtensorMap, CUtensorMap, CUtensorMap, AttnParams);
-    struct Variant { int nqt, npoly; KernelFn fn; };  // nqt 3 = the v3 kernel (three CTAs per SM, 64-row kv steps)
-    static const Variant variants[] = {
-        {3, 0, attention_fwd_v3_kernel<0>}, {3, 7, attention_fwd_v3_kernel<7>},
-        {1, 0, attention_fwd_v2_kernel<1, 0>}, {1, 7, attention_fwd_v2_kernel<1, 7>},
-        {2, 0, attention_fwd_v2_kernel<2, 0>},
-    };
-    // Default (same-box A/B on B200, tools/bench_kernels.py, TFLOP/s v3 / v2<1>): 1370-key sequences (encoder, frame
-    // attention) 586 / 572 and 552 / 535 at 8 views, 658 / 622 and 634 / 604 at 24 views -> v3; one long sequence (global
-    // attention) 740 / 766 at 8 views, 786 / 799 at 24 views -> v2<1>.  Every exponential on the MUFU (NPOLY = 0): moving a
-    // share of them to the FMA pipe was slower in both kernels (v2<1>: 766 -> 646 at 7 of 16; v3: 740 -> 720).
-    static const int pingpong_env = [] {
-      const char* e = getenv("MA_ATTN_PINGPONG");
-      return e ? atoi(e) : -1;
-    }();
-    // One long sequence (global attention, > 4096 keys): two query tiles per CTA with ping-pong -- K / V shared by 256 query
-    // rows, MUFU 82 % busy instead of 71 %: 881 vs 795 TFLOP/s at 16 views, 850 vs 799 at 24; at 8 views 756 vs 766 as a plain
-    // launch (516 CTAs = 3.5 waves of 148), 860 with the last partial wave split over the key range (Engine._pick_tail_split).
-    // v5 (persistent, two independent streams per CTA with ping-pong): many short sequences, plain self / cross attention
-    // (MA_ATTN_V5=0 turns it off) when the (query tile x head x sequence) items fill the 2 x SMs streams for at least three
-    // rounds.  Same-box A/B against v3 (TFLOP/s): 8 x 16 x 1370 (encoder, 1408 items) 637 vs 572, 8 x 12 x 1369 (frame, 1056
-    // items) 592 vs 539, 24 x 16 x 1370 698 vs 655; 3 x 12 x 1369 (396 items, 1.3 rounds) 411 vs 468 -> v3 stays for few items.
-    static const int v5_env = [] {
-      const char* e = getenv("MA_ATTN_V5");
-      return e ? atoi(e) : 1;
-    }();
-    const int n_items5 = ((q_len + ATT_BM - 1) / ATT_BM) * num_heads * num_seqs;
-    if (v5_env != 0 && nqt_env == 0 && kv_len <= 4096 && p.n_segs == 1 && p.seg_row0[0] == 0 && p.kv_split == 1 &&
-        !(flags & (MA_ATTN_STATE_IN | MA_ATTN_STATE_OUT)) && n_items5 >= 6 * device_sm_count()) {
-      static bool configured5[MA_MAX_DEVICES] = {};
-      if (!configured5[dev]) {
-        MA_CHECK_CUDA(cudaFuncSetAttribute(attention_fwd_v5_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, A5_SMEM_BYTES));
-        configured5[dev] = true;
-      }
-      const int grid5 = device_sm_count() < (n_items5 + 1) / 2 ? device_sm_count() : (n_items5 + 1) / 2;
-      MA_CHECK_CUDA(launch_kernel(attention_fwd_v5_kernel, dim3(grid5), dim3(A5_THREADS), A5_SMEM_BYTES,
-                                  static_cast<cudaStream_t>(stream), pdl_enabled(), tq, tk, tv, p));
-      MA_CHECK_CUDA(cudaGetLastError());
-      return MA_OK;
-    }
-    const int nqt = p.kv_split > 1 ? 2 : (nqt_env >= 1 && nqt_env <= 3) ? nqt_env : (kv_len <= 4096 ? 3 : 2);
-    p.pingpong = (nqt == 2 && pingpong_env != 0) ? 1 : 0;
-    const int want_poly = poly_env >= 0 ? poly_env : A2_DEFAULT_POLY;
-    const Variant* pick = nullptr;
-    for (const Variant& v : variants)
-      if (v.nqt == nqt && (pick == nullptr || abs(v.npoly - want_poly) < abs(pick->npoly - want_poly))) pick = &v;
-    const int smem_bytes = nqt == 3 ? A3_SMEM_BYTES : nqt == 2 ? A2Cfg<2>::SMEM_BYTES : A2Cfg<1>::SMEM_BYTES;
-    const int threads = nqt == 3 ? A3_THREADS : nqt == 2 ? A2Cfg<2>::THREADS : A2Cfg<1>::THREADS;
-    static bool configured2[MA_MAX_DEVICES][sizeof(variants) / sizeof(variants[0])] = {};
-    const int vi = static_cast<int>(pick - variants);
-    if (!configured2[dev][vi]) {
-      MA_CHECK_CUDA(cudaFuncSetAttribute(pick->fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
-      MA_CHECK_CUDA(cudaFuncSetAttribute(pick->fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
-      configured2[dev][vi] = true;
-    }
-    const int ctas = nqt == 2 ? grid_ctas : ((q_len + ATT_BM - 1) / ATT_BM) * num_heads * num_seqs;
-    if (nqt == 3) {  // key / value boxes of 64 rows
-      const uint32_t box64[2] = {ATT_D, A3_BN};
-      uint64_t dims[2] = {(uint64_t)ldk, (uint64_t)kv_rows};
-      uint64_t str[1] = {(uint64_t)ldk * 2};
-      int rc = make_tmap_bf16(&tk, k, 2, dims, str, box64);
-      if (rc != MA_OK) return rc;
-      dims[0] = (uint64_t)ldv;
-      str[0] = (uint64_t)ldv * 2;
-      rc = make_tmap_bf16(&tv, v, 2, dims, str, box64);
-      if (rc != MA_OK) return rc;
-    }
-    MA_CHECK_CUDA(launch_kernel(pick->fn, dim3(ctas), dim3(threads), smem_bytes, static_cast<cudaStream_t>(stream), pdl_enabled(),
-                                tq, tk, tv, p));
+    kernel = 2;
+    fn = attention_fwd_v2_kernel;
+    threads = A2_THREADS;
+    smem_bytes = A2_SMEM_BYTES;
+    ctas = grid_ctas;
   }
+  static bool configured[3][MA_MAX_DEVICES] = {};  // the large-shared-memory opt-in is per kernel and device
+  const int dev = current_device();
+  if (!configured[kernel][dev]) {
+    MA_CHECK_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_bytes));
+    if (kernel != 0)  // v2 / v3; v5's shared memory leaves no other carveout
+      MA_CHECK_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
+    configured[kernel][dev] = true;
+  }
+  MA_CHECK_CUDA(launch_kernel(fn, dim3(ctas), dim3(threads), smem_bytes, static_cast<cudaStream_t>(stream), pdl_enabled(),
+                              tq, tk, tv, p));
   MA_CHECK_CUDA(cudaGetLastError());
   return MA_OK;
 }

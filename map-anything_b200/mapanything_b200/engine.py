@@ -235,11 +235,6 @@ class Engine:
         # and the persistent two-stream attention kernel, which wants all views in one launch)
         self.encoder_streams = max(1, int(os.environ.get("MA_ENCODER_STREAMS", "1")))
         self.sm_count = torch.cuda.get_device_properties(self.device).multi_processor_count
-        # tail-wave splitting of long attention (the slots of the last, partially filled wave of SMs are cut over the key range,
-        # ma_attention_merge joins them): neutral with the free-running kernels of round 1, but with the ping-pong two-tile
-        # kernel the 8-view global attention drops from 6.34 to 5.67 + 0.15 (merge) ms per step (same-box A/B, 320 -> 332
-        # views/s); MA_ATTN_KV_SPLIT=0 turns it off
-        self.kv_split_enabled = os.environ.get("MA_ATTN_KV_SPLIT", "1") != "0"
         # views per DPT pass (bounds the activation scratch: ~0.6 GB per view at 518 px).  8 instead of 4: same-box A/B at 8
         # views 311.1 vs 301.6 views/s (fewer, larger launches); MA_DPT_CHUNK overrides for A/B runs
         self.dpt_chunk_default = max(1, int(os.environ.get("MA_DPT_CHUNK", "8")))
@@ -377,9 +372,9 @@ class Engine:
         """(first split slot, parts) for a long single-sequence attention, or None.  The (query block x head) CTAs have
         equal cost and fill the SMs in whole waves (8 views: 516 CTAs on 148 SMs = 3 full waves + 72 CTAs on half the
         chip).  Only the slots of that last partial wave are cut into `parts` CTAs, each with a share of the key range and
-        a partial softmax state; ma_attention_merge joins them (touching those rows only)."""
-        if not self.kv_split_enabled:
-            return None
+        a partial softmax state; ma_attention_merge joins them (touching those rows only).  With the ping-pong two-tile
+        kernel this takes the 8-view global attention from 6.34 to 5.67 + 0.15 (merge) ms per step (same-box A/B on a B200,
+        320 -> 332 views/s)."""
         sms = self.sm_count
         slots = -(-q_len // 256) * heads
         rem = slots % sms

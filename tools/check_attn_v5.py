@@ -1,7 +1,7 @@
-"""v5 attention (MA_ATTN_V5=1): correctness against F.scaled_dot_product_attention and TFLOP/s on the short-sequence shapes.
+"""Short-sequence attention: correctness against F.scaled_dot_product_attention and TFLOP/s.  Each shape runs on v5 when its
+(query tile x head x sequence) items number at least 6 per SM, on v3 otherwise (ma_attention_fwd_ex); the kernel is printed.
 python tools/check_attn_v5.py"""
 import json
-import os
 import sys
 
 import torch
@@ -10,7 +10,7 @@ import torch.nn.functional as F
 sys.path.insert(0, "map-anything_b200")
 from mapanything_b200 import ops  # noqa: E402
 
-print("MA_ATTN_V5 =", os.environ.get("MA_ATTN_V5"), flush=True)
+sms = torch.cuda.get_device_properties(0).multi_processor_count
 for nseq, L, H in ((8, 1370, 16), (8, 1369, 12), (3, 1369, 12), (24, 1370, 16), (5, 700, 12), (40, 257, 8), (2, 4096, 16)):
     D = H * 64
     g = torch.Generator(device="cuda").manual_seed(nseq * 1000 + L + H)
@@ -38,5 +38,6 @@ for nseq, L, H in ((8, 1370, 16), (8, 1369, 12), (3, 1369, 12), (24, 1370, 16), 
         torch.cuda.synchronize()
         ts.append(a.elapsed_time(b) / 10)
     ms = sorted(ts)[2]
-    print(json.dumps({"nseq": nseq, "L": L, "H": H, "finite": finite, "max_abs_err": round(err, 5), "us": round(ms * 1e3, 1),
+    kernel = "v5" if -(-L // 128) * H * nseq >= 6 * sms else "v3"
+    print(json.dumps({"nseq": nseq, "L": L, "H": H, "kernel": kernel, "finite": finite, "max_abs_err": round(err, 5), "us": round(ms * 1e3, 1),
                       "tflops": round(4.0 * nseq * H * L * L * 64 / ms / 1e9, 1)}), flush=True)
