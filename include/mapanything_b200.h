@@ -54,8 +54,8 @@ int ma_set_pdl(int enabled);
  * MA_GEMM_STREAMK, else on. */
 int ma_set_stream_k(int enabled);
 /* Which kernel the last ma_gemm_bf16 / ma_conv3x3_bf16 call of THIS thread launched, as a block_n code (64 / 128 / 256 = the
- * one-CTA kernel gemm_bf16_tcgen05_kernel<block_n>, 2128 / 2256 = the CTA-pair kernel gemm_bf16_2cta_kernel<block_n - 2000>);
- * 0 before the first call.  Measurement aid (bench.py names the dominant kernel from it); no reference counterpart. */
+ * one-CTA instantiation gemm_bf16_kernel<1, block_n>, 2128 / 2256 = the CTA-pair instantiation
+ * gemm_bf16_kernel<2, block_n - 2000>); 0 before the first call.  Measurement aid (bench.py names the dominant kernel from it); no reference counterpart. */
 int ma_last_gemm_block(void);
 
 /* ---- GEMM: Y = epilogue(X . W^T) ------------------------------------------------------------
@@ -108,8 +108,7 @@ typedef struct ma_gemm_epilogue {
 #define MA_GEMM_RELU_OUT_BEFORE_RESIDUAL 2
 
 /* block_n: 0 = choose automatically (wave count x measured per-tile cost); 64 / 128 / 256 = one CTA per 128 x block_n
- * tile; 2128 / 2256 = a CTA pair (tcgen05 cta_group::2, cluster of 2) per 256 x 128 / 256 x 256 tile.  Setting the
- * environment variable MA_GEMM_2CTA=0 removes the pair kernels from the automatic choice. */
+ * tile; 2128 / 2256 = a CTA pair (tcgen05 cta_group::2, cluster of 2) per 256 x 128 / 256 x 256 tile. */
 int ma_gemm_bf16(const void* x, int64_t ldx, const void* w, int64_t ldw, int M, int N, int K,
                  const ma_gemm_epilogue* epi, int block_n, void* stream);
 

@@ -30,7 +30,7 @@ def register_algorithmic_shape(w: torch.Tensor, n: int, k: int) -> None:
 
 def _gemm_kernel_name() -> str:
     code = _lib.load().ma_last_gemm_block()
-    return f"gemm_bf16_2cta_kernel<{code - 2000}>" if code > 2000 else f"gemm_bf16_tcgen05_kernel<{code}>"
+    return f"gemm_bf16_kernel<2, {code - 2000}>" if code > 2000 else f"gemm_bf16_kernel<1, {code}>"
 
 
 class launch:

@@ -1,14 +1,14 @@
-"""The stream-K work-unit schedule of the CTA-pair GEMM (csrc/gemm2.cu: UnitWalk + the sk_lo choice in launch_gemm2), mirrored
+"""The stream-K work-unit schedule of the CTA-pair GEMM (csrc/gemm.cu: UnitWalk + the sk_lo choice in launch_gemm<2, BN>), mirrored
 in Python and checked as a property over many shapes: every (tile, K block) is covered exactly once, by contiguous pieces,
 bias goes to exactly one unit per tile, and no cluster does more than its fair share + one tile boundary.  The numerical
 check of the kernel itself is tests/test_gemm_gpu.py::test_gemm_stream_k_residual."""
 import random
 
-SK_MIN_KBLOCKS, SK_MIN_PIECE = 32, 8   # G2_SK_MIN_KBLOCKS, G2_SK_MIN_PIECE
+SK_MIN_KBLOCKS, SK_MIN_PIECE = 32, 8   # GEMM_SK_MIN_KBLOCKS, GEMM_SK_MIN_PIECE
 
 
 def launch_params(tiles: int, kblocks: int, max_clusters: int = 74, reduce_add: bool = True):
-    """-> (clusters, sk_lo) as launch_gemm2 chooses them."""
+    """-> (clusters, sk_lo) as launch_gemm<2, BN> chooses them."""
     clusters = min(tiles, max_clusters)
     sk_lo = tiles
     if reduce_add and kblocks >= SK_MIN_KBLOCKS and tiles % max_clusters != 0:

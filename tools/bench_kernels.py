@@ -36,7 +36,7 @@ def main():
         x = torch.randn(m, k, device="cuda").bfloat16()
         w = torch.randn(n, k, device="cuda").bfloat16()
         o = torch.empty(m, n, device="cuda", dtype=torch.bfloat16)
-        for bn in (0, 128, 256, 2128, 2256):
+        for bn in (0, 64, 128, 256, 2128, 2256):
             t = timeit(lambda: ops.gemm(x, w, o, block_n=bn))
             res.append({"kernel": "gemm", "name": name, "bn": bn, "M": m, "N": n, "K": k, "ms": t, "tflops": 2 * m * n * k / t / 1e9})
         t = timeit(lambda: torch.matmul(x, w.t()))
@@ -46,7 +46,7 @@ def main():
         x = torch.randn(n, H, W, Cc, device="cuda").bfloat16()
         w = torch.randn(Co, 9 * Cc, device="cuda").bfloat16()
         o = torch.empty(n * H * W, Co, device="cuda", dtype=torch.bfloat16)
-        for bn in (0, 128, 256, 2128, 2256):
+        for bn in (0, 64, 128, 256, 2128, 2256):
             if bn % 1000 > Co and bn:
                 continue
             t = timeit(lambda: ops.conv3x3(x, w, o, block_n=bn))
