@@ -72,7 +72,10 @@ int ma_last_gemm_block(void);
  * (`flags` can move the activation after the residual add, or take out_relu before it.)
  * Row mapping (token assembly without copy kernels): when rows_per_group_in > 0,
  *    out_row = (m / rows_per_group_in) * rows_per_group_out + row_offset_out + m % rows_per_group_in
- * else out_row = m.  res_row = m % residual_row_mod when residual_row_mod > 0, else out_row. */
+ * else out_row = m.  res_row = m % residual_row_mod when residual_row_mod > 0, else out_row.
+ * Alignment: when N >= 32 (a multiple of 32 or not), out, residual, out_relu, bias and colscale must be 16-byte aligned and
+ * ldo / ldr / ldo_relu multiples of 16 bytes (full 32-column chunks are loaded and stored as 16-byte vectors); otherwise
+ * the call returns MA_ERR_INVALID.  With N < 32 they need only their element alignment. */
 typedef struct ma_gemm_epilogue {
   void* out;
   int64_t ldo;

@@ -672,28 +672,25 @@ static int run_gemm(const char* who, int block_n, const void* w, int64_t ldw, co
 
 }  // namespace ma
 
+// Every full 32-column chunk of a row takes the vector path (16-byte loads of bias / colscale / residual, 16-byte stores of
+// out / out_relu), also when a ragged last chunk follows it: so with N >= 32 every epilogue operand must be 16-byte
+// aligned at each row.  With N < 32 the only chunk is the scalar path, which has no alignment needs.
 static int check_epilogue(const ma_gemm_epilogue* epi, int N, const char* who) {
-  if (N % 32 == 0) {
-    const int64_t oalign = epi->out_dtype == MA_F32 ? 4 : 8;
-    MA_REQUIRE(epi->ldo % oalign == 0 && (reinterpret_cast<uintptr_t>(epi->out) & 15) == 0,
-               "%s: output not 16-byte aligned (ldo=%lld)", who, (long long)epi->ldo);
-    if (epi->residual) {
-      const int64_t ralign = epi->residual_dtype == MA_F32 ? 4 : 8;
-      MA_REQUIRE(epi->ldr % ralign == 0 && (reinterpret_cast<uintptr_t>(epi->residual) & 15) == 0,
-                 "%s: residual not 16-byte aligned", who);
-    }
-    if (epi->out_relu)
-      MA_REQUIRE(epi->ldo_relu % 8 == 0 && (reinterpret_cast<uintptr_t>(epi->out_relu) & 15) == 0,
-                 "%s: out_relu not 16-byte aligned", who);
-    if (epi->bias) MA_REQUIRE((reinterpret_cast<uintptr_t>(epi->bias) & 15) == 0, "%s: bias not 16-byte aligned", who);
-    if (epi->colscale)
-      MA_REQUIRE((reinterpret_cast<uintptr_t>(epi->colscale) & 15) == 0, "%s: colscale not 16-byte aligned", who);
-  } else {
-    // A ragged last N chunk takes the scalar store path, full chunks before it still use vector stores.
-    const int64_t oalign = epi->out_dtype == MA_F32 ? 4 : 8;
-    MA_REQUIRE(N <= 32 || (epi->ldo % oalign == 0 && (reinterpret_cast<uintptr_t>(epi->out) & 15) == 0),
-               "%s: output not 16-byte aligned (ldo=%lld)", who, (long long)epi->ldo);
+  if (N < 32) return MA_OK;
+  const int64_t oalign = epi->out_dtype == MA_F32 ? 4 : 8;
+  MA_REQUIRE(epi->ldo % oalign == 0 && (reinterpret_cast<uintptr_t>(epi->out) & 15) == 0,
+             "%s: output not 16-byte aligned (ldo=%lld)", who, (long long)epi->ldo);
+  if (epi->residual) {
+    const int64_t ralign = epi->residual_dtype == MA_F32 ? 4 : 8;
+    MA_REQUIRE(epi->ldr % ralign == 0 && (reinterpret_cast<uintptr_t>(epi->residual) & 15) == 0,
+               "%s: residual not 16-byte aligned (ldr=%lld)", who, (long long)epi->ldr);
   }
+  if (epi->out_relu)
+    MA_REQUIRE(epi->ldo_relu % 8 == 0 && (reinterpret_cast<uintptr_t>(epi->out_relu) & 15) == 0,
+               "%s: out_relu not 16-byte aligned (ldo_relu=%lld)", who, (long long)epi->ldo_relu);
+  if (epi->bias) MA_REQUIRE((reinterpret_cast<uintptr_t>(epi->bias) & 15) == 0, "%s: bias not 16-byte aligned", who);
+  if (epi->colscale)
+    MA_REQUIRE((reinterpret_cast<uintptr_t>(epi->colscale) & 15) == 0, "%s: colscale not 16-byte aligned", who);
   return MA_OK;
 }
 

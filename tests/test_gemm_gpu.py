@@ -153,14 +153,17 @@ def test_gemm_row_remap_and_strides():
 
 @pytest.mark.parametrize("n,H,W,C,Cout", [(2, 37, 37, 256, 256), (1, 19, 19, 768, 256), (3, 74, 74, 192, 256), (1, 148, 148, 96, 256),
                                           (2, 40, 56, 128, 128), (1, 5, 3, 64, 32), (1, 130, 70, 128, 6)])
-@pytest.mark.parametrize("bn", [0, 128, 2128, 2256])
+@pytest.mark.parametrize("bn", [0, 64, 128, 256, 2128, 2256])
 def test_conv3x3_implicit_gemm_matches_torch(n, H, W, C, Cout, bn):
     """Implicit-GEMM 3x3 conv (4-D TMA boxes, zero padding by out-of-bounds fill) vs F.conv2d on the same bf16 operands,
-    incl. C not a multiple of 64, ragged pixel tiles, ragged Cout, bias + ReLU + residual + twin ReLU output."""
+    incl. C not a multiple of 64, ragged pixel tiles, ragged Cout, bias + ReLU + residual + twin ReLU output, and the
+    geometric-input encoders' bias + fp32 residual + GELU after the residual into bf16.  The fp32 output and the GELU case
+    are also checked per element against an fp64 reference (the bound of test_gemm_epilogue_gpu.py)."""
     import torch.nn.functional as F
 
-    from mapanything_b200 import ops
-    from mapanything_b200.ops import MA_ACT_RELU
+    from mapanything_b200 import _lib, ops
+    from mapanything_b200.ops import MA_ACT_GELU, MA_ACT_RELU
+    from test_gemm_epilogue_gpu import GELU_SLOPE, _bound, _check as _check_elementwise, _conv_f64, _gelu
 
     torch.backends.cudnn.allow_tf32 = False
     g = torch.Generator(device="cuda").manual_seed(n * 1000 + H + W + C)
@@ -169,10 +172,23 @@ def test_conv3x3_implicit_gemm_matches_torch(n, H, W, C, Cout, bn):
     bias = torch.randn(Cout, device="cuda", generator=g)
     w = w4.permute(0, 2, 3, 1).reshape(Cout, 9 * C).contiguous()  # [Cout][(ky,kx),Cin]
     ref = F.conv2d(x.float().permute(0, 3, 1, 2), w4.float(), bias, padding=1).permute(0, 2, 3, 1).reshape(n * H * W, Cout)
+    ref64 = _conv_f64(x, w4, bias)
+    mag = _conv_f64(x.abs(), w4.abs(), bias.abs())
 
     out = torch.full((n * H * W, Cout), float("nan"), device="cuda")
     ops.conv3x3(x, w, out, bias=bias, block_n=bn)
+    assert bn == 0 or _lib.load().ma_last_gemm_block() == bn
     _check(out, ref, 2e-3, "conv3x3 fp32 out")
+    _check_elementwise(out, ref64, _bound(ref64, mag, None, False, True), f"conv3x3 fp32 out bn={bn}")
+
+    # bias + fp32 residual, then GELU (geometric-input encoders), bf16 out
+    res32 = torch.randn(n * H * W, Cout, device="cuda", generator=g)
+    o4 = torch.full((n * H * W, Cout), float("nan"), device="cuda", dtype=torch.bfloat16)
+    ops.conv3x3(x, w, o4, bias=bias, residual=res32, act=MA_ACT_GELU, act_after_residual=True, block_n=bn)
+    pre = ref64 + res32.double()
+    want = _gelu(pre)
+    _check_elementwise(o4, want, _bound(want, (mag + res32.double().abs()) * GELU_SLOPE, (pre.abs(), 1.0), True, False),
+                       f"conv3x3 + residual, GELU after it, bn={bn}")
 
     if Cout % 32 == 0:
         res = torch.randn(n * H * W, Cout, device="cuda", generator=g).bfloat16()
