@@ -57,6 +57,11 @@ int ma_set_stream_k(int enabled);
  * one-CTA instantiation gemm_bf16_kernel<1, block_n>, 2128 / 2256 = the CTA-pair instantiation
  * gemm_bf16_kernel<2, block_n - 2000>); 0 before the first call.  Measurement aid (bench.py names the dominant kernel from it); no reference counterpart. */
 int ma_last_gemm_block(void);
+/* Which kernel the last ma_attention_fwd / ma_attention_fwd_ex call of THIS thread launched: 5 = attention_fwd_v5_kernel
+ * (plain attention over many short sequences), 3 = attention_fwd_v3_kernel (up to 4096 keys, no kv split), 2 =
+ * attention_fwd_v2_kernel (longer key ranges, kv split); 0 before the first launch.  Lets tests and tools see which kernel
+ * a shape reaches; no reference counterpart. */
+int ma_last_attention_kernel(void);
 
 /* ---- GEMM: Y = epilogue(X . W^T) ------------------------------------------------------------
  * Replaces every nn.Linear / 1x1 conv / im2col'ed conv on the path (cuBLASLt / cuDNN calls in the

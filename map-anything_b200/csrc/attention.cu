@@ -1117,7 +1117,11 @@ __global__ void attention_merge_kernel(const float* __restrict__ state_o, int64_
   *reinterpret_cast<uint32_t*>(out + row * ldo + h * ATT_D + 2 * lane) = pack_bf16x2(ax * inv, ay * inv);
 }
 
+thread_local int g_last_attention_kernel = 0;  // 5 / 3 / 2: the forward kernel this thread launched last
+
 }  // namespace ma
+
+extern "C" int ma_last_attention_kernel(void) { return ma::g_last_attention_kernel; }
 
 extern "C" int ma_attention_fwd(const void* q, int64_t ldq, int64_t q_rows, int q_col0, const void* k, int64_t ldk,
                                 int64_t kv_rows, int k_col0, const void* v, int64_t ldv, int v_col0, void* out,
@@ -1160,10 +1164,15 @@ extern "C" int ma_attention_fwd_ex(const void* q, int64_t ldq, int64_t q_rows, i
     kv_extent = p.seg_row0[s] + p.seg_len[s] > kv_extent ? p.seg_row0[s] + p.seg_len[s] : kv_extent;
   }
   p.state_o = nullptr; p.state_m = nullptr; p.ld_state_o = 0;
-  if (flags & (MA_ATTN_STATE_IN | MA_ATTN_STATE_OUT)) {
-    MA_REQUIRE(ext->state_o && ext->state_m && ext->ld_state_o % 4 == 0 && ext->ld_state_o >= (int64_t)num_heads * ATT_D &&
-                   (reinterpret_cast<uintptr_t>(ext->state_o) & 15) == 0,
-               "ma_attention_fwd: softmax state buffers missing / misaligned");
+  // a kv split writes partial states whether or not STATE_OUT is set (store_row: float4 rows of state_o)
+  if ((flags & (MA_ATTN_STATE_IN | MA_ATTN_STATE_OUT)) || (ext && ext->kv_split > 1)) {
+    MA_REQUIRE(ext->state_o && ext->state_m, "ma_attention_fwd: softmax state buffers missing");
+    MA_REQUIRE((reinterpret_cast<uintptr_t>(ext->state_o) & 15) == 0, "ma_attention_fwd: state_o not 16-byte aligned");
+    MA_REQUIRE(ext->ld_state_o % 4 == 0, "ma_attention_fwd: ld_state_o %lld is not a multiple of 4 floats",
+               (long long)ext->ld_state_o);
+    MA_REQUIRE(ext->ld_state_o >= (int64_t)num_heads * ATT_D, "ma_attention_fwd: ld_state_o %lld is less than heads*64 = %d",
+               (long long)ext->ld_state_o, num_heads * ATT_D);
+    MA_REQUIRE((reinterpret_cast<uintptr_t>(ext->state_m) & 3) == 0, "ma_attention_fwd: state_m not 4-byte aligned");
     p.state_o = ext->state_o; p.state_m = ext->state_m; p.ld_state_o = ext->ld_state_o;
   }
   p.num_heads = num_heads;
@@ -1178,9 +1187,7 @@ extern "C" int ma_attention_fwd_ex(const void* q, int64_t ldq, int64_t q_rows, i
   int grid_ctas = n_slots_host;
   if (ext && ext->kv_split > 1) {
     MA_REQUIRE(!(flags & MA_ATTN_STATE_IN), "ma_attention_fwd: kv_split cannot resume from a state");
-    MA_REQUIRE(ext->state_o && ext->state_m, "ma_attention_fwd: kv_split needs the partial-state buffers");
     MA_REQUIRE(ext->kv_split_from >= 0 && ext->kv_split_from <= n_slots_host, "ma_attention_fwd: kv_split_from out of range");
-    p.state_o = ext->state_o; p.state_m = ext->state_m; p.ld_state_o = ext->ld_state_o;
     p.split_from = ext->kv_split_from;
     grid_ctas = p.split_from + (n_slots_host - p.split_from) * ext->kv_split;
     MA_REQUIRE(ext->kv_split <= p.n_kv_tiles, "ma_attention_fwd: kv_split %d exceeds the %d kv tiles", ext->kv_split, p.n_kv_tiles);
@@ -1284,6 +1291,8 @@ extern "C" int ma_attention_fwd_ex(const void* q, int64_t ldq, int64_t q_rows, i
       MA_CHECK_CUDA(cudaFuncSetAttribute(fn, cudaFuncAttributePreferredSharedMemoryCarveout, cudaSharedmemCarveoutMaxShared));
     configured[kernel][dev] = true;
   }
+  static constexpr int kVersion[3] = {5, 3, 2};
+  g_last_attention_kernel = kVersion[kernel];
   MA_CHECK_CUDA(launch_kernel(fn, dim3(ctas), dim3(threads), smem_bytes, static_cast<cudaStream_t>(stream), pdl_enabled(),
                               tq, tk, tv, p));
   MA_CHECK_CUDA(cudaGetLastError());
@@ -1296,6 +1305,14 @@ extern "C" int ma_attention_merge(const float* state_o, int64_t ld_state_o, int6
   using namespace ma;
   MA_REQUIRE(state_o && state_m && out && n_partials >= 1 && rows > 0 && num_heads > 0, "ma_attention_merge: bad arguments");
   MA_REQUIRE(ld_state_o % 2 == 0 && split_stride_o % 2 == 0 && ldo % 2 == 0, "ma_attention_merge: strides must be even");
+  // one warp per (row, head): float2 loads of state_o, 32-bit (bf16 pair) stores of out
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(state_o) & 7) == 0, "ma_attention_merge: state_o not 8-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(state_m) & 3) == 0, "ma_attention_merge: state_m not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out) & 3) == 0, "ma_attention_merge: out not 4-byte aligned");
+  MA_REQUIRE(ld_state_o >= (int64_t)num_heads * ATT_D, "ma_attention_merge: ld_state_o %lld is less than heads*64 = %d",
+             (long long)ld_state_o, num_heads * ATT_D);
+  MA_REQUIRE(ldo >= (int64_t)num_heads * ATT_D, "ma_attention_merge: ldo %lld is less than heads*64 = %d", (long long)ldo,
+             num_heads * ATT_D);
   int64_t warps = rows * num_heads;
   if (first_slot >= 0) {
     const int64_t n_slots = ((rows + 2 * ATT_BM - 1) / (2 * ATT_BM)) * num_heads;

@@ -262,15 +262,22 @@ def attention(
     is cut into kv_split parts, one CTA each, and `state` holds one partial per part: (fp32 [kv_split, q_rows, heads*64],
     fp32 [kv_split, q_rows, heads], the latter pre-filled with -inf); join them with attention_merge.  kv_split_from: only
     (query block, head) slots from that index on are split (the others write `out` / part 0).  See ma_attention_fwd_ex."""
-    for t in (q, k, v, out):
+    width = num_heads * 64
+    for name, t in (("q", q), ("k", k), ("v", v), ("out", out)):
         if t is None:
             continue
         if t.dtype != torch.bfloat16 or t.dim() != 2 or t.stride(1) != 1:
             raise ValueError("attention operands must be 2-D bf16 with contiguous rows")
+        # the library sees only the row stride: a narrower view would let the heads run into the parent's next columns
+        if t.shape[1] < width:
+            raise ValueError(f"attention: {name} has {t.shape[1]} columns, {num_heads} heads need {width}")
     if q_seq_stride is None:
         q_seq_stride = q_len
     if kv_seq_stride is None:
         kv_seq_stride = kv_len
+    q_rows = (num_seqs - 1) * q_seq_stride + q_len   # query rows the call reads and writes
+    if out is not None and out.shape[0] < q_rows:
+        raise ValueError(f"attention: out has {out.shape[0]} rows, the call writes {q_rows}")
     if scale is None:
         scale = 64 ** -0.5
     lib = _lib.load()
@@ -295,6 +302,8 @@ def attention(
                     or sm.stride(1) != num_heads or so.shape[1] < q.shape[0] or sm.shape[1:] != (so.shape[1], num_heads)
                     or so.shape[0] < kv_split or sm.shape[0] < kv_split):
                 raise ValueError("attention state must be (fp32 [parts, q_rows, >=heads*64], fp32 [parts, q_rows, heads])")
+            if so.shape[2] < width:
+                raise ValueError(f"attention: state_o has {so.shape[2]} columns, {num_heads} heads need {width}")
             ext.flags = (MA_ATTN_STATE_IN if state_in else 0) | (MA_ATTN_STATE_OUT if state_out else 0)
             ext.state_o, ext.ld_state_o, ext.state_m = so.data_ptr(), so.stride(1), sm.data_ptr()
             ext.kv_split, ext.split_stride_o, ext.split_stride_m = kv_split, so.stride(0), sm.stride(0)
@@ -323,6 +332,13 @@ def attention_merge(state, out: torch.Tensor, *, num_heads: int, scale: Optional
     if out.dtype != torch.bfloat16 or out.stride(1) != 1 or sm.stride(1) != num_heads or sm.stride(2) != 1:
         raise ValueError("attention_merge: out must be bf16 with contiguous rows")
     parts, rows = so.shape[0], out.shape[0]
+    width = num_heads * 64
+    if out.shape[1] < width:
+        raise ValueError(f"attention_merge: out has {out.shape[1]} columns, {num_heads} heads need {width}")
+    if so.shape[2] < width or so.shape[1] < rows:
+        raise ValueError(f"attention_merge: state_o is [{so.shape[1]}, {so.shape[2]}] per part, out needs [{rows}, {width}]")
+    if sm.shape[0] < parts or sm.shape[1] < rows:
+        raise ValueError(f"attention_merge: state_m has {sm.shape[0]} parts of {sm.shape[1]} rows, state_o {parts} of {rows}")
     if scale is None:
         scale = 64 ** -0.5
     with launch("attention_merge"):

@@ -1,5 +1,5 @@
-"""Short-sequence attention: correctness against F.scaled_dot_product_attention and TFLOP/s.  Each shape runs on v5 when its
-(query tile x head x sequence) items number at least 6 per SM, on v3 otherwise (ma_attention_fwd_ex); the kernel is printed.
+"""Short-sequence attention: correctness against F.scaled_dot_product_attention and TFLOP/s, with the kernel each shape ran
+on (v5 / v3, as ma_last_attention_kernel reports it).
 python tools/check_attn_v5.py"""
 import json
 import sys
@@ -8,9 +8,8 @@ import torch
 import torch.nn.functional as F
 
 sys.path.insert(0, "map-anything_b200")
-from mapanything_b200 import ops  # noqa: E402
+from mapanything_b200 import _lib, ops  # noqa: E402
 
-sms = torch.cuda.get_device_properties(0).multi_processor_count
 for nseq, L, H in ((8, 1370, 16), (8, 1369, 12), (3, 1369, 12), (24, 1370, 16), (5, 700, 12), (40, 257, 8), (2, 4096, 16)):
     D = H * 64
     g = torch.Generator(device="cuda").manual_seed(nseq * 1000 + L + H)
@@ -22,6 +21,7 @@ for nseq, L, H in ((8, 1370, 16), (8, 1369, 12), (3, 1369, 12), (24, 1370, 16), 
 
     run()
     torch.cuda.synchronize()
+    kernel = f"v{_lib.load().ma_last_attention_kernel()}"
     q, k, v = (qkv[:, i * D:(i + 1) * D].view(nseq, L, H, 64).transpose(1, 2) for i in range(3))
     ref = F.scaled_dot_product_attention(q.float(), k.float(), v.float()).transpose(1, 2).reshape(nseq * L, D)
     err = (out.float() - ref).abs().max().item()
@@ -38,6 +38,5 @@ for nseq, L, H in ((8, 1370, 16), (8, 1369, 12), (3, 1369, 12), (24, 1370, 16), 
         torch.cuda.synchronize()
         ts.append(a.elapsed_time(b) / 10)
     ms = sorted(ts)[2]
-    kernel = "v5" if -(-L // 128) * H * nseq >= 6 * sms else "v3"
     print(json.dumps({"nseq": nseq, "L": L, "H": H, "kernel": kernel, "finite": finite, "max_abs_err": round(err, 5), "us": round(ms * 1e3, 1),
                       "tflops": round(4.0 * nseq * H * L * L * 64 / ms / 1e9, 1)}), flush=True)
