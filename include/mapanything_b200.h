@@ -196,7 +196,9 @@ int ma_patchify(const float* img, void* out, int n, int H, int W, int patch, int
 /* nn.LayerNorm over the last dim (reference: every norm1/norm2/norm of dinov2/layers/block.py:93-119, the
  * fusion_norm_layer model.py:1245-1254, the info-sharing norms).  in/out dtype are ma_dtype; the optional row
  * remap row(r) = (r / rows_per_group) * group_stride + row_offset + r % rows_per_group (separately for in and
- * out; rows_per_group = 0 -> identity) drops the cls token / skips the scale token without a copy. */
+ * out; rows_per_group = 0 -> identity) drops the cls token / skips the scale token without a copy.  C and the row
+ * strides are multiples of 4 with ld_in, ld_out >= C; in and out are 16-byte aligned when fp32 and 8-byte aligned when bf16,
+ * gamma and beta 16-byte aligned. */
 int ma_layernorm(const void* in, int in_dtype, int64_t ld_in, void* out, int out_dtype, int64_t ld_out,
                  const float* gamma, const float* beta, int rows, int C, float eps, int rows_per_group,
                  int64_t in_group_stride, int64_t in_row_offset, int64_t out_group_stride, int64_t out_row_offset,
@@ -207,16 +209,17 @@ int ma_layernorm(const void* in, int in_dtype, int64_t ld_in, void* out, int out
 int ma_fill_f32(float* dst, int64_t n, float value, void* stream);
 
 /* dst[g*group_stride + row_offset][0:C] = a[0:C] + b[0:C] (b may be NULL) for g in [0, groups): cls token +
- * pos_embed[0] (reference vision_transformer.py:252-253), scale token row (model.py:1524-1535). fp32. */
+ * pos_embed[0] (reference vision_transformer.py:252-253), scale token row (model.py:1524-1535). fp32, ld >= C. */
 int ma_set_rows(float* dst, int64_t ld, int groups, int64_t group_stride, int64_t row_offset, const float* a,
                 const float* b, int C, void* stream);
 
 /* im2col of a 3x3 / pad 1 / stride {1,2} convolution over NHWC bf16 (n,H,W,C): out[(i,yo,xo)][(ky*3+kx)*C + c].
- * With ma_gemm_bf16 this replaces the cuDNN convs of the DPT / pose heads (reference model.py:1302-1338). */
+ * With ma_gemm_bf16 this replaces the cuDNN convs of the DPT / pose heads (reference model.py:1302-1338).  C % 8 == 0;
+ * in and out 16-byte aligned. */
 int ma_im2col3x3(const void* in, void* out, int n, int H, int W, int C, int stride, void* stream);
 
 /* ConvTranspose2d with kernel == stride == s as GEMM + this permutation: in[(i,y,x)][(ky*s+kx)*C + c] ->
- * NHWC out[(i, y*s+ky, x*s+kx)][c]  (DPT act_postprocess, SURVEY App. A.4). bf16. */
+ * NHWC out[(i, y*s+ky, x*s+kx)][c]  (DPT act_postprocess, SURVEY App. A.4). bf16, C % 8 == 0, in and out 16-byte aligned. */
 int ma_pixel_shuffle(const void* in, void* out, int n, int h, int w, int C, int s, void* stream);
 
 /* The same permutation in fp32 with row strides: the `linear` prediction head (reference model.py:339-343, a 1x1 conv
@@ -226,7 +229,8 @@ int ma_pixel_shuffle_f32(const float* in, int64_t ld_in, float* out, int64_t ld_
                          void* stream);
 
 /* F.interpolate(mode="bilinear", align_corners=True) over NHWC bf16.  (Hv,Wv) is the full output size that
- * defines the scale; only the top-left (Ho,Wo) window is written (refinenet4 crop 38 -> 37). */
+ * defines the scale; only the top-left (Ho,Wo) window is written (refinenet4 crop 38 -> 37).  C % 8 == 0; in and out
+ * 16-byte aligned. */
 int ma_bilinear_align_corners(const void* in, void* out, int n, int Hin, int Win, int C, int Hv, int Wv, int Ho, int Wo,
                               void* stream);
 
@@ -235,18 +239,21 @@ int ma_token_mean(const void* in, void* out, int n, int T, int C, void* stream);
 
 /* fp32 [rows][C] -> bf16 [rows][3C] = [hi | lo | hi] (hi = bf16(x), lo = bf16(x - hi)).  With weights packed
  * [w_hi | w_hi | w_lo] one ma_gemm_bf16 over K' = 3K evaluates the product to ~2^-16 relative accuracy: used for
- * the pose / scale heads, which the reference runs with autocast disabled (model.py:1599). */
+ * the pose / scale heads, which the reference runs with autocast disabled (model.py:1599).  C and ld_in are multiples of 4
+ * with ld_in >= C; in is 16-byte aligned, out 8-byte aligned. */
 int ma_split_bf16x3(const float* in, int64_t ld_in, void* out, int rows, int C, void* stream);
 
 /* Narrow linear head out[row][0:N] = W[N][K] . x[row] + b (N <= 8, K <= 256, bf16 in, fp32 out): the final 1x1 conv of
- * the DPT regressor (128 -> 6 channels per pixel, SURVEY App. A.4; reference model.py:1326-1332) as a streaming kernel. */
+ * the DPT regressor (128 -> 6 channels per pixel, SURVEY App. A.4; reference model.py:1326-1332) as a streaming kernel.
+ * K % 8 == 0, ldx % 8 == 0, ldx >= K, ldw >= K, ldo >= N; x 16-byte aligned. */
 int ma_head_linear_small(const void* x, int64_t ldx, const void* w, int64_t ldw, const float* bias, float* out, int64_t ldo,
                          int64_t rows, int N, int K, void* stream);
 
 /* fp32 Linear on a handful of rows: out[r][0:N] = act(b + W[N][K] . x[r]), 1 <= rows <= 16, K % 4 == 0, rows * K * 4 <= 48 KB,
  * plain fp32 arithmetic (act: MA_ACT_NONE / MA_ACT_RELU / MA_ACT_GELU, exact erf).  The pooled MLPs of the pose head and the
  * scale head (uniception PoseHead.more_mlps / fc_t / fc_rot and MLPHead on the scale token, invoked at reference
- * model.py:1449-1469 with autocast disabled): 8 x 768 and 1 x 768 inputs. */
+ * model.py:1449-1469 with autocast disabled): 8 x 768 and 1 x 768 inputs.  ldx, ldw multiples of 4 and >= K, ldo >= N; x and w
+ * 16-byte aligned. */
 int ma_linear_rows_f32(const float* x, int64_t ldx, const float* w, int64_t ldw, const float* bias, int act, float* out,
                        int64_t ldo, int rows, int N, int K, void* stream);
 
@@ -257,7 +264,8 @@ int ma_token_mean_f32(const float* in, float* out, int n, int T, int C, void* st
  * model.py:1683-1741, :1874-1907; geometry.py:855-907): raw [n*HW][ld_raw] fp32 = (ray xyz, depth logit,
  * confidence logit, mask logit); pose_raw [n][7] = (t, q xyzw); scale_raw [1] (log metric scale).
  * Writes pts3d, pts3d_cam, rays [n*HW][3]; depth, conf, logits [n*HW]; mask [n*HW] (1 byte bool);
- * cam_trans [n][3] (scaled), cam_quats [n][4] (unit), scale_out [1]. */
+ * cam_trans [n][3] (scaled), cam_quats [n][4] (unit), scale_out [1].  ld_raw >= 6; when ld_raw % 4 == 0 each row is read
+ * as a float4 and a float2, so raw must then be 16-byte aligned. */
 int ma_decode_dense(const float* raw, int ld_raw, const float* pose_raw, const float* scale_raw, int n, int HW,
                     float* pts3d, float* pts3d_cam, float* rays, float* depth, float* conf, float* logits, uint8_t* mask,
                     float* cam_trans, float* cam_quats, float* scale_out, void* stream);

@@ -729,6 +729,15 @@ extern "C" int ma_layernorm(const void* in, int in_dtype, int64_t ld_in, void* o
                             int64_t out_row_offset, void* stream) {
   MA_REQUIRE(in && out && gamma && beta && rows > 0 && C > 0 && C % 4 == 0, "ma_layernorm: bad arguments (rows=%d C=%d)", rows, C);
   MA_REQUIRE(ld_in % 4 == 0 && ld_out % 4 == 0, "ma_layernorm: row strides must be multiples of 4 elements");
+  MA_REQUIRE(ld_in >= C, "ma_layernorm: ld_in (%lld) below C = %d", (long long)ld_in, C);
+  MA_REQUIRE(ld_out >= C, "ma_layernorm: ld_out (%lld) below C = %d", (long long)ld_out, C);
+  // four elements per access: float4 / uint2 loads of in, stores of out, float4 loads of gamma and beta
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(in) & (in_dtype == MA_F32 ? 15 : 7)) == 0, "ma_layernorm: in not %d-byte aligned",
+             in_dtype == MA_F32 ? 16 : 8);
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out) & (out_dtype == MA_F32 ? 15 : 7)) == 0, "ma_layernorm: out not %d-byte aligned",
+             out_dtype == MA_F32 ? 16 : 8);
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(gamma) & 15) == 0, "ma_layernorm: gamma not 16-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(beta) & 15) == 0, "ma_layernorm: beta not 16-byte aligned");
   LnParams p{in, out, gamma, beta, ld_in, ld_out, rows, C, rows_per_group, in_group_stride, in_row_offset,
              out_group_stride, out_row_offset, eps};
   const int wpb = 8;
@@ -751,6 +760,7 @@ extern "C" int ma_layernorm(const void* in, int in_dtype, int64_t ld_in, void* o
 extern "C" int ma_set_rows(float* dst, int64_t ld, int groups, int64_t group_stride, int64_t row_offset, const float* a,
                            const float* b, int C, void* stream) {
   MA_REQUIRE(dst && a && groups > 0 && C > 0, "ma_set_rows: bad arguments");
+  MA_REQUIRE(ld >= C, "ma_set_rows: ld (%lld) below C = %d", (long long)ld, C);
   set_rows_kernel<<<groups, 256, 0, static_cast<cudaStream_t>(stream)>>>(dst, ld, group_stride, row_offset, a, b, C);
   MA_CHECK_CUDA(cudaGetLastError());
   return MA_OK;
@@ -765,6 +775,8 @@ extern "C" int ma_fill_f32(float* dst, int64_t n, float value, void* stream) {
 
 extern "C" int ma_im2col3x3(const void* in, void* out, int n, int H, int W, int C, int stride, void* stream) {
   MA_REQUIRE(in && out && n > 0 && C % 8 == 0 && (stride == 1 || stride == 2), "ma_im2col3x3: bad arguments (C=%d stride=%d)", C, stride);
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(in) & 15) == 0, "ma_im2col3x3: in not 16-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "ma_im2col3x3: out not 16-byte aligned");
   const int Ho = (H + 2 - 3) / stride + 1, Wo = (W + 2 - 3) / stride + 1;
   const int64_t total = (int64_t)n * Ho * Wo * 9 * (C / 8);
   im2col3x3_kernel<<<grid_for(total, 256, device_sm_count() * 16), 256, 0, static_cast<cudaStream_t>(stream)>>>(
@@ -775,6 +787,8 @@ extern "C" int ma_im2col3x3(const void* in, void* out, int n, int H, int W, int 
 
 extern "C" int ma_pixel_shuffle(const void* in, void* out, int n, int h, int w, int C, int s, void* stream) {
   MA_REQUIRE(in && out && n > 0 && C % 8 == 0 && s > 0, "ma_pixel_shuffle: bad arguments");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(in) & 15) == 0, "ma_pixel_shuffle: in not 16-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "ma_pixel_shuffle: out not 16-byte aligned");
   const int64_t total = (int64_t)n * h * w * s * s * (C / 8);
   pixel_shuffle_kernel<<<grid_for(total, 256, device_sm_count() * 16), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       static_cast<const __nv_bfloat16*>(in), static_cast<__nv_bfloat16*>(out), n, h, w, C, s);
@@ -797,6 +811,8 @@ extern "C" int ma_bilinear_align_corners(const void* in, void* out, int n, int H
                                          int Wo, void* stream) {
   MA_REQUIRE(in && out && n > 0 && C % 8 == 0 && Ho <= Hv && Wo <= Wv && Hin > 0 && Win > 0, "ma_bilinear_align_corners: bad arguments");
   MA_REQUIRE((int64_t)n * Ho < (1ll << 31), "ma_bilinear_align_corners: too many output rows");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(in) & 15) == 0, "ma_bilinear_align_corners: in not 16-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out) & 15) == 0, "ma_bilinear_align_corners: out not 16-byte aligned");
   bilinear_ac_kernel<<<n * Ho, 256, 0, static_cast<cudaStream_t>(stream)>>>(
       static_cast<const __nv_bfloat16*>(in), static_cast<__nv_bfloat16*>(out), n, Hin, Win, C, Hv, Wv, Ho, Wo);
   MA_CHECK_CUDA(cudaGetLastError());
@@ -818,6 +834,8 @@ extern "C" int ma_head_linear_small(const void* x, int64_t ldx, const void* w, i
   MA_REQUIRE(N >= 1 && N <= 8 && K >= 8 && K <= 256 && K % 8 == 0 && ldx % 8 == 0 && ldo >= N,
              "ma_head_linear_small: needs N <= 8, K <= 256, K %% 8 == 0 (N=%d K=%d)", N, K);
   MA_REQUIRE((reinterpret_cast<uintptr_t>(x) & 15) == 0, "ma_head_linear_small: x not 16-byte aligned");
+  MA_REQUIRE(ldx >= K, "ma_head_linear_small: ldx (%lld) below K = %d", (long long)ldx, K);
+  MA_REQUIRE(ldw >= K, "ma_head_linear_small: ldw (%lld) below K = %d", (long long)ldw, K);
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   const __nv_bfloat16* xb = static_cast<const __nv_bfloat16*>(x);
   const __nv_bfloat16* wb = static_cast<const __nv_bfloat16*>(w);
@@ -837,6 +855,9 @@ extern "C" int ma_head_linear_small(const void* x, int64_t ldx, const void* w, i
 
 extern "C" int ma_split_bf16x3(const float* in, int64_t ld_in, void* out, int rows, int C, void* stream) {
   MA_REQUIRE(in && out && rows > 0 && C > 0 && C % 4 == 0 && ld_in % 4 == 0, "ma_split_bf16x3: bad arguments (C=%d)", C);
+  MA_REQUIRE(ld_in >= C, "ma_split_bf16x3: ld_in (%lld) below C = %d", (long long)ld_in, C);
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(in) & 15) == 0, "ma_split_bf16x3: in not 16-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out) & 7) == 0, "ma_split_bf16x3: out not 8-byte aligned");
   const int64_t total = (int64_t)rows * (C / 4);
   split_bf16x3_kernel<<<grid_for(total, 256, device_sm_count() * 16), 256, 0, static_cast<cudaStream_t>(stream)>>>(
       in, ld_in, static_cast<__nv_bfloat16*>(out), rows, C);
@@ -858,6 +879,8 @@ extern "C" int ma_linear_rows_f32(const float* x, int64_t ldx, const float* w, i
                  ldo >= N, "ma_linear_rows_f32: needs 1 <= rows <= %d, K %% 4 == 0, strides %% 4 == 0 (rows=%d N=%d K=%d)",
              LIN_ROWS_MAX, rows, N, K);
   MA_REQUIRE(((reinterpret_cast<uintptr_t>(x) | reinterpret_cast<uintptr_t>(w)) & 15) == 0, "ma_linear_rows_f32: x / w not 16-byte aligned");
+  MA_REQUIRE(ldx >= K, "ma_linear_rows_f32: ldx (%lld) below K = %d", (long long)ldx, K);
+  MA_REQUIRE(ldw >= K, "ma_linear_rows_f32: ldw (%lld) below K = %d", (long long)ldw, K);
   MA_REQUIRE(act == MA_ACT_NONE || act == MA_ACT_RELU || act == MA_ACT_GELU, "ma_linear_rows_f32: bad activation %d", act);
   const size_t smem = (size_t)rows * K * sizeof(float);
   MA_REQUIRE(smem <= 48 * 1024, "ma_linear_rows_f32: rows * K = %d floats do not fit 48 KB of shared memory", rows * K);
@@ -872,6 +895,8 @@ extern "C" int ma_decode_dense(const float* raw, int ld_raw, const float* pose_r
   MA_REQUIRE(raw && pose_raw && scale_raw && pts3d && pts3d_cam && rays && depth && conf && logits && mask && cam_trans &&
                  cam_quats && scale_out && n > 0 && HW > 0 && ld_raw >= 6,
              "ma_decode_dense: bad arguments");
+  MA_REQUIRE(ld_raw % 4 != 0 || (reinterpret_cast<uintptr_t>(raw) & 15) == 0,
+             "ma_decode_dense: raw not 16-byte aligned (ld_raw %% 4 == 0 takes the float4 loads)");
   DecodeParams p{raw, ld_raw, pose_raw, scale_raw, pts3d, pts3d_cam, rays, depth, conf, logits, mask, cam_trans, cam_quats,
                  scale_out, n, HW};
   dim3 grid(grid_for(HW, 256, 1024), n);

@@ -87,26 +87,56 @@ def test_bilinear_align_corners_matches_torch(n, Hin, Win, C, Ho, Wo, virt):
     assert (out.float() - ref).abs().max().item() < 2e-2 * ref.abs().max().item()
 
 
-@pytest.mark.parametrize("rows,N,K,act", [(8, 768, 768, "relu"), (1, 768, 768, "gelu"), (8, 7, 768, None), (1, 1, 768, None),
-                                          (16, 128, 8, "gelu"), (3, 1024, 512, None), (12, 77, 1024, "relu")])
-def test_linear_rows_f32_matches_torch(rows, N, K, act):
+LINEAR_ROWS = [(8, 768, 768, "relu"), (1, 768, 768, "gelu"), (8, 7, 768, None), (1, 1, 768, None), (16, 128, 8, "gelu"),
+               (3, 1024, 512, None), (12, 77, 1024, "relu")]
+# (rows, N, K, act, ldx - K, ldo - N, bias): row-strided x (NaN padding) and out (sentinel padding), no bias, K = 4, and
+# rows * K = 16 * 768 floats, exactly the 48 KB of shared memory the kernel stages x in
+LINEAR_ROWS_STRIDED = [(16, 40, 768, "gelu", 4, 3, True), (16, 9, 768, None, 8, 0, False), (5, 33, 4, "relu", 4, 1, False),
+                       (3, 100, 256, None, 0, 5, False)]
+
+
+@pytest.mark.parametrize("rows,N,K,act,ldx_pad,ldo_pad,bias", [
+    *(pytest.param(*c, 0, 0, True, id="-".join(map(str, c))) for c in LINEAR_ROWS),
+    *(pytest.param(*c, id="-".join(map(str, c[:4])) + f"-ldx+{c[4]}-ldo+{c[5]}" + ("" if c[6] else "-nobias"))
+      for c in LINEAR_ROWS_STRIDED)])
+def test_linear_rows_f32_matches_torch(rows, N, K, act, ldx_pad, ldo_pad, bias):
     """ma_linear_rows_f32 (the pooled MLPs of the pose / scale heads and the per-view global encoders): plain fp32 Linear on up
-    to 16 rows against torch (float64 accumulation as the yardstick)."""
+    to 16 rows against torch (float64 accumulation as the yardstick).  Per element: lanes stride over K in float4 steps, so
+    each output is a chain of 4 ceil(K / 128) FMAs, 5 shuffle adds and the bias: D = 4 ceil(K / 128) + 7 and
+    |y - ref| <= D u (|x| |w|^T + |b|) (x 1.13 through GELU) + 2e-7 |pre-GELU| (the erf approximation) + u |ref|."""
     import torch.nn.functional as F
 
-    from mapanything_b200 import ops
+    from mapanything_b200 import _lib, ops
     from mapanything_b200._lib import MA_ACT_GELU, MA_ACT_NONE, MA_ACT_RELU
 
     g = torch.Generator(device="cuda").manual_seed(rows * 1000 + N + K)
-    x = torch.randn(rows, K, device="cuda", generator=g)
+    xbuf = torch.full((rows + 1, K + ldx_pad), float("nan"), device="cuda")
+    xbuf[:rows, :K] = torch.randn(rows, K, device="cuda", generator=g)
+    x = xbuf[:rows, :K]
     w = torch.randn(N, K, device="cuda", generator=g) * K ** -0.5
-    b = torch.randn(N, device="cuda", generator=g)
-    out = torch.full((rows, N), float("nan"), device="cuda")
-    ops.linear_rows_f32(x, w, b, out, {"relu": MA_ACT_RELU, "gelu": MA_ACT_GELU, None: MA_ACT_NONE}[act])
-    ref = x.double() @ w.double().t() + b.double()
-    ref = F.relu(ref) if act == "relu" else F.gelu(ref) if act == "gelu" else ref
+    b = torch.randn(N, device="cuda", generator=g) if bias else None
+    obuf = torch.full((rows, N + ldo_pad), -77.0, device="cuda")
+    out = obuf[:, :N]
+    code = {"relu": MA_ACT_RELU, "gelu": MA_ACT_GELU, None: MA_ACT_NONE}[act]
+    if ldx_pad or ldo_pad:   # ops.linear_rows_f32 takes contiguous tensors only
+        _lib.check(_lib.load().ma_linear_rows_f32(x.data_ptr(), x.stride(0), w.data_ptr(), w.stride(0), b.data_ptr() if bias else None,
+                                                  code, out.data_ptr(), out.stride(0), rows, N, K,
+                                                  torch.cuda.current_stream().cuda_stream), "ma_linear_rows_f32")
+    else:
+        ops.linear_rows_f32(x, w, b, out, code)
+    pre = x.double() @ w.double().t() + (b.double() if bias else 0.0)
+    mag = x.double().abs() @ w.double().abs().t() + (b.double().abs() if bias else 0.0)
+    ref = F.relu(pre) if act == "relu" else F.gelu(pre) if act == "gelu" else pre
     assert torch.isfinite(out).all()
     assert (out.double() - ref).abs().max().item() < 2e-5 * max(1.0, ref.abs().max().item())
+    u = 2.0 ** -24
+    bound = (4 * -(-K // 128) + 7) * u * mag * (1.13 if act == "gelu" else 1.0) + u * ref.abs()
+    if act == "gelu":
+        bound = bound + 2e-7 * pre.abs()
+    ratio = ((out.double() - ref).abs() / bound).max().item()
+    print(f"\n[linear_rows_f32] rows={rows} N={N} K={K} act={act}: worst err/bound {ratio:.3g}", end="")
+    assert ratio <= 1.0, ratio
+    assert (obuf[:, N:] == -77.0).all(), "ldo padding written"
 
 
 def test_token_mean_f32_matches_torch():

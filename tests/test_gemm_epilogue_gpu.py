@@ -295,6 +295,15 @@ def test_split3_bit_exact_on_strided_input():
 
     g = torch.Generator(device="cuda").manual_seed(3)
     buf = torch.randn(300, 136, device="cuda", generator=g) * torch.exp(torch.randn(300, 136, device="cuda", generator=g) * 4)
+    # rows 0-59: +-0, fp32 subnormals, magnitudes near 1e30 and exact bf16 rounding ties (low 16 bits 0x8000: halfway
+    # between two bf16 values, with an even and an odd bf16 neighbour below) at normal, subnormal and ~1e30 magnitudes
+    base = torch.tensor([1.0, -3.0, 1e30, -7e29, 1.5e-38, 2.5e-39, -1e-40, 0.1], device="cuda")
+    bits = base.view(torch.int32)
+    ties = torch.cat([((bits & -0x20000) | 0x8000).view(torch.float32), ((bits & -0x20000) | 0x18000).view(torch.float32)])
+    special = torch.cat([torch.tensor([0.0, -0.0, 1e-45, -1e-45, 1e-40, -3e-39, 1.1e-38, 1e30, -1e30, 3.3e30, -9.9e29],
+                                      device="cuda"), ties])
+    buf[:60, :special.numel()] = special
+    buf[:60, 60:60 + special.numel()] = special.flip(0)
     x = buf[:, :120]   # ld_in = 136 > C
     got = ops.split3(x)
     hi = x.bfloat16()
