@@ -316,7 +316,8 @@ int ma_pose_to_quat_trans(const float* poses, float* quats, float* trans, int B,
 
 /* nn.PixelUnshuffle(patch) of an NHWC fp32 map (n,H,W,cin) (ray directions model.py:803-811 / depth :946-971) written as
  * the split-bf16 activation [hi | lo | hi] of an NHWC token map (n,H/p,W/p,3*cpad), channel k = c*p*p + dy*p + dx zero
- * padded to cpad (multiple of 8).  mode 1 (depth): v /= factor[i]; v = v/max(|v|,1e-8) * log1p(|v|) (geometry.py:1666-1679). */
+ * padded to cpad (multiple of 8).  mode 1 (depth): v /= factor[i]; v = v/max(|v|,1e-8) * log1p(|v|) (geometry.py:1666-1679).
+ * patch must be positive and divide H and W; cpad >= cin*patch*patch. */
 int ma_unshuffle_split(const float* in, void* out, int n, int H, int W, int cin, int patch, int cpad, int mode,
                        const float* factor, void* stream);
 
@@ -332,7 +333,8 @@ int ma_pose_inputs(const float* quats, const float* trans, const uint8_t* has_po
 
 /* In-place fusion adds on the fp32 encoder features feat [V*N][C] (model.py:820-825, :1003-1008, :1124-1129):
  * feat[v*N+t] += dense_a[a_slot[v]*N+t] + dense_b[b_slot[v]*N+t] + sum_j gw[j*V+v] * g_j[v]; slot -1 / NULL = absent;
- * g3 (depth-scale features) has one row per b_slot and is read at g3[b_slot[v]]. */
+ * g3 (depth-scale features) has one row per b_slot and is read at g3[b_slot[v]].  C % 4 == 0; the kernel moves float4, so
+ * feat and each of dense_a, dense_b, g0..g3 that is present must be 16-byte aligned. */
 int ma_fuse_add(float* feat, int V, int N, int C, const float* dense_a, const int* a_slot, const float* dense_b,
                 const int* b_slot, const float* g0, const float* g1, const float* g2, const float* g3, const float* gw,
                 void* stream);
@@ -392,19 +394,24 @@ int ma_intrinsics_from_rays(const float* rays, float* K, int n, int H, int W, vo
 /* camera_poses (n,4,4) from quats (n,4, xyzw) and translations (n,3) (inference.py:364-379). */
 int ma_pose_matrices(const float* quats, const float* trans, float* out, int n, void* stream);
 
-/* Edge mask (inference.py:418-454 + geometry.py:1717-1780, :2031-2072, :2129-2188), float32-exact with numpy:
- * mask_out = mask_in & ~(depth_edge & normal_edge).  depth_z is read with an element stride (pass pts3d_cam + 2,
+/* Edge mask (inference.py:418-454 + geometry.py:1717-1780, :2031-2072, :2129-2188): mask_out = mask_in & ~(depth_edge &
+ * normal_edge).  Normals, normal mask and depth edge are float32-exact with numpy; the neighbour angles use CUDA's acosf,
+ * which can differ from numpy's float32 arccos by a few ulp, so only a pixel whose pooled angle lies that close to the
+ * threshold can differ from numpy.  depth_z is read with an element stride (pass pts3d_cam + 2,
  * stride 3).  Workspaces per pixel: ws_normals 3 floats, ws_nmask 1 byte, ws_angle 1 float, ws_depth_edge 1 byte. */
 int ma_edge_mask(const float* pts3d, const float* depth_z, int depth_stride, const uint8_t* mask_in, uint8_t* mask_out,
                  float* ws_normals, uint8_t* ws_nmask, float* ws_angle, uint8_t* ws_depth_edge, int n, int H, int W,
                  float normal_tol_deg, float depth_rtol, void* stream);
 
-/* out[px, c] = in[px*in_stride + in_offset + c] * mask[px], c < width (inference.py:457-476). */
+/* out[px, c] = in[px*in_stride + in_offset + c] * mask[px], c < width (inference.py:457-476).  The columns read must lie
+ * within one pixel: 0 <= in_offset and in_offset + width <= in_stride (depth_z from pts3d_cam: stride 3, offset 2, width 1). */
 int ma_apply_mask(const float* in, int in_stride, int in_offset, const uint8_t* mask, float* out, int64_t pixels, int width,
                   void* stream);
 
 /* Confidence mask (inference.py:393-415): per image thr = torch.quantile(conf, q) (linear interpolation, float32
- * arithmetic of torch) by exact radix selection, mask = conf > thr (1 byte bool).  thr_out [n] optional. */
+ * arithmetic of torch: its lerp rounds once, as an FMA) by exact radix selection, mask = conf > thr (1 byte bool).
+ * An image holding a NaN gets a NaN threshold and an all-False mask, as torch.quantile propagates NaN.  thr_out [n]
+ * optional. */
 int ma_quantile_mask(const float* conf, uint8_t* mask, float* thr_out, int n, int64_t per_image, float q, void* stream);
 
 /* depthmap_to_camera_frame / depthmap_to_world_frame (geometry.py:18-114; what every demo calls on infer()'s depth_z,

@@ -310,6 +310,7 @@ extern "C" int ma_unshuffle_split(const float* in, void* out, int n, int H, int 
                                   const float* factor, void* stream) {
   using namespace ma;
   MA_REQUIRE(in && out, "ma_unshuffle_split: null pointer");
+  MA_REQUIRE(patch > 0, "ma_unshuffle_split: patch must be positive, got %d", patch);
   MA_REQUIRE(n > 0 && H % patch == 0 && W % patch == 0 && cin > 0, "ma_unshuffle_split: bad shape");
   MA_REQUIRE(cpad % 8 == 0 && cpad >= cin * patch * patch, "ma_unshuffle_split: cpad must be a multiple of 8 >= cin*p*p");
   MA_REQUIRE(mode == 0 || (mode == 1 && factor), "ma_unshuffle_split: mode 1 needs the per-view factor");
@@ -344,6 +345,11 @@ extern "C" int ma_fuse_add(float* feat, int V, int N, int C, const float* dense_
   MA_REQUIRE(feat && V > 0 && N > 0 && C > 0 && C % 4 == 0, "ma_fuse_add: bad arguments");
   MA_REQUIRE((!dense_a || a_slot) && (!dense_b || b_slot), "ma_fuse_add: dense addend without its slot table");
   MA_REQUIRE(!(g0 || g1 || g2 || g3) || gw, "ma_fuse_add: global addends need their gate table");
+  // float4 loads and stores: every row operand that is present must be 16-byte aligned (C % 4 == 0 keeps its rows so)
+  const struct { const void* ptr; const char* name; } rows[] = {{feat, "feat"}, {dense_a, "dense_a"}, {dense_b, "dense_b"},
+                                                               {g0, "g0"}, {g1, "g1"}, {g2, "g2"}, {g3, "g3"}};
+  for (const auto& r : rows)
+    MA_REQUIRE(reinterpret_cast<uintptr_t>(r.ptr) % 16 == 0, "ma_fuse_add: %s not 16-byte aligned", r.name);
   FuseParams p;
   p.feat = feat; p.dense_a = dense_a; p.a_slot = a_slot; p.dense_b = dense_b; p.b_slot = b_slot;
   p.g[0] = g0; p.g[1] = g1; p.g[2] = g2; p.g[3] = g3; p.gw = gw;

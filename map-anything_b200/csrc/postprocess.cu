@@ -8,6 +8,8 @@
 // OUTPUT IS BOOLEAN: any rounding difference can flip a pixel.  Reference functions:
 //   points_to_normals geometry.py:1717-1780, normals_edge :2129-2188 (including its transposed mask window),
 //   depth_edge :2031-2072, max_pool_2d :1905-2028, mask combination inference.py:418-476.
+// The one exception is the neighbour angle: CUDA's acosf can differ from numpy's float32 arccos by a few ulp, so a pixel
+// whose pooled angle lies within that distance of the threshold can differ from numpy.
 #include <math_constants.h>
 
 #include "host_common.h"
@@ -277,9 +279,12 @@ __global__ void mask_and_kernel(const uint8_t* __restrict__ a, const uint8_t* __
 // ----------------------------------------------------------------------------------------------
 // Per-image confidence quantile mask (reference inference.py:393-415): thr = torch.quantile(conf, q) with linear
 // interpolation, mask = conf > thr.  One block per image: exact order statistics by a 4 x 8-bit radix select over the
-// order-preserving integer image of the floats (no sort), then torch's lerp in float32:
+// order-preserving integer image of the floats (no sort), then torch's lerp in float32, each branch one FMA rounding as
+// in ATen's lerp:
 //   rank = q * (n - 1) (float32), lo = floor(rank), w = rank - lo,
-//   thr = w < 0.5 ? a + w (b - a) : b - (b - a)(1 - w)      with a, b = the lo-th / ceil(rank)-th smallest values.
+//   thr = w < 0.5 ? fma(w, b - a, a) : fma(w - 1, b - a, b)      with a, b = the lo-th / ceil(rank)-th smallest values
+// (w - 1 is exact for w in [0.5, 1)).  As in torch.quantile, an image holding a NaN gets a NaN threshold (an all-False
+// mask).
 // ----------------------------------------------------------------------------------------------
 __device__ __forceinline__ uint32_t float_to_ordered(float f) {
   const uint32_t u = __float_as_uint(f);
@@ -292,7 +297,7 @@ __device__ __forceinline__ float ordered_to_float(uint32_t u) {
 __global__ void quantile_mask_kernel(const float* __restrict__ conf, uint8_t* __restrict__ mask, float* __restrict__ thr_out,
                                      int64_t per_image, float q) {
   __shared__ uint32_t hist[256];
-  __shared__ uint32_t s_prefix, s_k, s_next, s_cnt_le;
+  __shared__ uint32_t s_prefix, s_k, s_next, s_cnt_le, s_nan;
   const float* x = conf + (int64_t)blockIdx.x * per_image;
   const float rank = q * static_cast<float>(per_image - 1);  // float32 like torch (q and n - 1 as float32 tensors)
   const float lo_f = floorf(rank);
@@ -300,7 +305,7 @@ __global__ void quantile_mask_kernel(const float* __restrict__ conf, uint8_t* __
   const uint32_t k_lo = static_cast<uint32_t>(lo_f);
   const bool need_hi = ceilf(rank) != lo_f;
 
-  if (threadIdx.x == 0) { s_prefix = 0u; s_k = k_lo; }
+  if (threadIdx.x == 0) { s_prefix = 0u; s_k = k_lo; s_nan = 0u; }
   __syncthreads();
   uint32_t less_total = 0;  // (thread 0) number of elements strictly below the selected value so far
   for (int pass = 0; pass < 4; ++pass) {
@@ -310,7 +315,9 @@ __global__ void quantile_mask_kernel(const float* __restrict__ conf, uint8_t* __
     const uint32_t prefix = s_prefix;
     const uint32_t pmask = pass == 0 ? 0u : (0xffffffffu << (shift + 8));
     for (int64_t i = threadIdx.x; i < per_image; i += blockDim.x) {
-      const uint32_t u = float_to_ordered(x[i]);
+      const float xi = x[i];
+      if (pass == 0 && xi != xi) s_nan = 1u;
+      const uint32_t u = float_to_ordered(xi);
       if ((u & pmask) == prefix) atomicAdd(&hist[(u >> shift) & 0xffu], 1u);
     }
     __syncthreads();
@@ -345,7 +352,7 @@ __global__ void quantile_mask_kernel(const float* __restrict__ conf, uint8_t* __
     }
   }
   const float diff = b - a;
-  const float thr = w < 0.5f ? __fadd_rn(a, __fmul_rn(w, diff)) : __fsub_rn(b, __fmul_rn(diff, __fsub_rn(1.0f, w)));
+  const float thr = s_nan ? CUDART_NAN_F : w < 0.5f ? __fmaf_rn(w, diff, a) : __fmaf_rn(w - 1.0f, diff, b);
   if (threadIdx.x == 0 && thr_out) thr_out[blockIdx.x] = thr;
   uint8_t* m = mask + (int64_t)blockIdx.x * per_image;
   for (int64_t i = threadIdx.x; i < per_image; i += blockDim.x) m[i] = x[i] > thr ? 1 : 0;
@@ -442,6 +449,8 @@ extern "C" int ma_edge_mask(const float* pts3d, const float* depth_z, int depth_
 extern "C" int ma_apply_mask(const float* in, int in_stride, int in_offset, const uint8_t* mask, float* out, int64_t pixels,
                              int width, void* stream) {
   MA_REQUIRE(in && mask && out && pixels > 0 && width > 0 && in_stride >= width, "ma_apply_mask: bad arguments");
+  MA_REQUIRE(in_offset >= 0 && in_offset <= in_stride - width,
+             "ma_apply_mask: in_offset %d + width %d must lie in [0, in_stride %d]", in_offset, width, in_stride);
   const int64_t total = pixels * width;
   const int grid = static_cast<int>((total + 255) / 256 > 148 * 16 ? 148 * 16 : (total + 255) / 256);
   apply_mask_kernel<<<grid, 256, 0, static_cast<cudaStream_t>(stream)>>>(in, in_stride, in_offset, mask, out, pixels, width);
