@@ -62,6 +62,11 @@ int ma_last_gemm_block(void);
  * attention_fwd_v2_kernel (longer key ranges, kv split); 0 before the first launch.  Lets tests and tools see which kernel
  * a shape reaches; no reference counterpart. */
 int ma_last_attention_kernel(void);
+/* Which form of the horizontal resampling pass the last ma_resample_h_u8rgb call of THIS thread launched: 1 =
+ * resample_h_kernel (byte loads, any window length), 1000 + KMAX = resample_h_vec_kernel<KMAX> (word loads, windows up to
+ * KMAX taps), 2000 + NW4 = resample_h_dp4a_kernel<NW4> (dp4a on packed coefficients, windows up to 4 * NW4 taps); 0 before
+ * the first launch.  Lets tests see which instantiation a call reaches; no reference counterpart. */
+int ma_last_resample_kernel(void);
 
 /* ---- GEMM: Y = epilogue(X . W^T) ------------------------------------------------------------
  * Replaces every nn.Linear / 1x1 conv / im2col'ed conv on the path (cuBLASLt / cuDNN calls in the
@@ -355,7 +360,8 @@ int ma_resample_coeffs(int in_size, int out_size, int filter, int* ksize_out, in
 /* Horizontal pass over n frames of the same size.  src: device u8 RGB, interleaved; row / frame strides in bytes;
  * source rows [y0, y0+rows) and source columns [sx0, sx1) are read (sx0/sx1 = the window span of output columns
  * [x0, x0+cols)); bounds / coeffs: device copies of the tables for the horizontal axis (ksize taps, out_size columns); packed: optional, see ma_resample_pack_coeffs.
- * tmp: device u8 [n][rows][cols][3]. */
+ * tmp: device u8 [n][rows][cols][3].  src may sit at any byte address; y0 and sx0 must be >= 0 and bounds, coeffs and
+ * packed 4-byte aligned.  The staged span sx1 - sx0 may be at most 68,264 pixels (a row of it lives in shared memory). */
 int ma_resample_h_u8rgb(const uint8_t* src, int64_t src_row_stride, int64_t src_frame_stride, int n, int y0, int rows,
                         int sx0, int sx1, const int32_t* bounds, const int32_t* coeffs, const uint32_t* packed, int ksize,
                         int out_size, int x0, int cols, uint8_t* tmp, void* stream);
@@ -367,18 +373,21 @@ int ma_resample_pack_coeffs(const int32_t* coeffs, int ksize, int out_size, uint
 
 /* Vertical pass + crop + normalise.  tmp: [n][rows][cols][3] u8 whose row 0 is source row y0; output rows
  * [top, top+th) of the resampled image (out_size rows; bounds / coeffs: the vertical axis' tables, ksize taps).  out_chw: fp32 (n, 3, th, cols) = ((u/255) - mean) / std in
- * torchvision's rounding order (mean / std: 3 HOST floats), may be NULL; out_u8: u8 [n][th][cols][3], may be NULL. */
+ * torchvision's rounding order (mean / std: 3 HOST floats), may be NULL; out_u8: u8 [n][th][cols][3], may be NULL.
+ * bounds, coeffs and out_chw must be 4-byte aligned; th and n at most 65535. */
 int ma_resample_v_norm_u8rgb(const uint8_t* tmp, int n, int rows, int cols, int y0, const int32_t* bounds,
                              const int32_t* coeffs, int ksize, int out_size, int top, int th, const float* mean_host,
                              const float* std_host, float* out_chw, uint8_t* out_u8, void* stream);
 
 /* preprocess_inputs() (image.py:335-675) resizes depth maps with cv2.resize(INTER_NEAREST) and slices the crop
  * (cropping.py:248-255, :339): out[y][x] = src[y_idx[y]][x_idx[x]], th x tw; y_idx / x_idx: device int32 source offsets
- * of the cropped window (OpenCV resizeNN: min(floor(i * (1 / (dst / src))), src - 1), computed on the host). */
+ * of the cropped window (OpenCV resizeNN: min(floor(i * (1 / (dst / src))), src - 1), computed on the host).
+ * src, y_idx, x_idx and out must be 4-byte aligned; th at most 65535. */
 int ma_gather_rows_cols_f32(const float* src, int64_t src_row_stride, const int32_t* y_idx, const int32_t* x_idx, int th,
                             int tw, float* out, void* stream);
 
-/* Float image -> bytes as image.py:503-506 does with torch: (in * scale).clamp(0, 255).byte(); n elements. */
+/* Float image -> bytes as image.py:503-506 does with torch for an fp32 tensor: (in * scale).clamp(0, 255).byte(); n elements.
+ * in must be 4-byte aligned. */
 int ma_f32_to_u8(const float* in, int64_t n, float scale, uint8_t* out, void* stream);
 
 /* ---- infer() post-processing (reference mapanything/utils/inference.py:294-480, host numpy there) ---- */

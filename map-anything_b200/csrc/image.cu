@@ -266,13 +266,24 @@ __global__ void f32_to_u8_kernel(const float* __restrict__ in, int64_t n, float 
   out[i] = static_cast<uint8_t>(static_cast<int>(v));  // truncation, like the C cast behind .byte()
 }
 
+// Which form of the horizontal pass this thread launched last: 1 = resample_h_kernel, 1000 + KMAX = resample_h_vec_kernel<KMAX>,
+// 2000 + NW4 = resample_h_dp4a_kernel<NW4>; 0 before the first launch.
+thread_local int g_last_resample_kernel = 0;
+
 }  // namespace ma
+
+extern "C" int ma_last_resample_kernel(void) { return ma::g_last_resample_kernel; }
 
 using namespace ma;
 
 extern "C" int ma_gather_rows_cols_f32(const float* src, int64_t src_row_stride, const int32_t* y_idx, const int32_t* x_idx,
                                        int th, int tw, float* out, void* stream) {
   MA_REQUIRE(src && y_idx && x_idx && out && th > 0 && tw > 0, "ma_gather_rows_cols_f32: bad arguments (th=%d tw=%d)", th, tw);
+  MA_REQUIRE(th <= 65535, "ma_gather_rows_cols_f32: th=%d above 65535 (one grid row per output row)", th);
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(src) & 3) == 0, "ma_gather_rows_cols_f32: src not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(y_idx) & 3) == 0, "ma_gather_rows_cols_f32: y_idx not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(x_idx) & 3) == 0, "ma_gather_rows_cols_f32: x_idx not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out) & 3) == 0, "ma_gather_rows_cols_f32: out not 4-byte aligned");
   dim3 grid((tw + 127) / 128, th);
   gather_rows_cols_f32_kernel<<<grid, 128, 0, static_cast<cudaStream_t>(stream)>>>(src, src_row_stride, y_idx, x_idx, tw, out);
   MA_CHECK_CUDA(cudaGetLastError());
@@ -281,6 +292,7 @@ extern "C" int ma_gather_rows_cols_f32(const float* src, int64_t src_row_stride,
 
 extern "C" int ma_f32_to_u8(const float* in, int64_t n, float scale, uint8_t* out, void* stream) {
   MA_REQUIRE(in && out && n > 0, "ma_f32_to_u8: bad arguments");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(in) & 3) == 0, "ma_f32_to_u8: in not 4-byte aligned");
   f32_to_u8_kernel<<<static_cast<unsigned>((n + 255) / 256), 256, 0, static_cast<cudaStream_t>(stream)>>>(in, n, scale, out);
   MA_CHECK_CUDA(cudaGetLastError());
   return MA_OK;
@@ -352,6 +364,7 @@ static int launch_h_vec(const uint8_t* src, int64_t row_stride, int64_t frame_st
     MA_CHECK_CUDA(cudaFuncSetAttribute(resample_h_vec_kernel<KMAX>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     configured = 200 * 1024;
   }
+  g_last_resample_kernel = 1000 + KMAX;
   resample_h_vec_kernel<KMAX><<<dim3(rows, n), 256, smem, stream>>>(src, row_stride, frame_stride, y0, sx0, sx1, bounds, coeffs,
                                                                     out_size, x0, cols, tmp);
   MA_CHECK_CUDA(cudaGetLastError());
@@ -371,6 +384,7 @@ static int launch_h_dp4a(const uint8_t* src, int64_t row_stride, int64_t frame_s
     MA_CHECK_CUDA(cudaFuncSetAttribute(resample_h_dp4a_kernel<NW4>, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024));
     configured = 200 * 1024;
   }
+  g_last_resample_kernel = 2000 + NW4;
   resample_h_dp4a_kernel<NW4><<<dim3(rows, n), 256, smem, stream>>>(src, row_stride, frame_stride, y0, sx0, sx1, bounds, packed,
                                                                     out_size, x0, cols, tmp, plane_words);
   MA_CHECK_CUDA(cudaGetLastError());
@@ -403,6 +417,11 @@ extern "C" int ma_resample_h_u8rgb(const uint8_t* src, int64_t src_row_stride, i
   MA_REQUIRE(src && bounds && coeffs && tmp && n > 0 && n <= 65535 && rows > 0 && cols > 0 && sx1 > sx0 && x0 >= 0 &&
                  x0 + cols <= out_size && ksize > 0,
              "ma_resample_h_u8rgb: bad arguments (n=%d rows=%d cols=%d ksize=%d)", n, rows, cols, ksize);
+  MA_REQUIRE(sx0 >= 0, "ma_resample_h_u8rgb: sx0=%d is negative", sx0);
+  MA_REQUIRE(y0 >= 0, "ma_resample_h_u8rgb: y0=%d is negative", y0);
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(bounds) & 3) == 0, "ma_resample_h_u8rgb: bounds not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(coeffs) & 3) == 0, "ma_resample_h_u8rgb: coeffs not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(packed) & 3) == 0, "ma_resample_h_u8rgb: packed not 4-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
   static const bool byte_loads = [] {  // MA_RESAMPLE_BYTE_LOADS=1: the first kernel (byte loads, any window length), for A/B runs
     const char* e = getenv("MA_RESAMPLE_BYTE_LOADS");
@@ -445,6 +464,7 @@ extern "C" int ma_resample_h_u8rgb(const uint8_t* src, int64_t src_row_stride, i
       configured = 200 * 1024;
     }
   }
+  g_last_resample_kernel = 1;
   resample_h_kernel<<<dim3(rows, n), 256, smem, st>>>(src, src_row_stride, src_frame_stride, y0, sx0, sx1, bounds, coeffs, out_size,
                                                      x0, cols, tmp);
   MA_CHECK_CUDA(cudaGetLastError());
@@ -458,6 +478,10 @@ extern "C" int ma_resample_v_norm_u8rgb(const uint8_t* tmp, int n, int rows, int
                  top + th <= out_size && (out_chw || out_u8),
              "ma_resample_v_norm_u8rgb: bad arguments (n=%d cols=%d th=%d)", n, cols, th);
   MA_REQUIRE(!out_chw || (mean_host && std_host), "ma_resample_v_norm_u8rgb: mean / std missing");
+  MA_REQUIRE(th <= 65535, "ma_resample_v_norm_u8rgb: th=%d above 65535 (one grid row per output row)", th);
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(bounds) & 3) == 0, "ma_resample_v_norm_u8rgb: bounds not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(coeffs) & 3) == 0, "ma_resample_v_norm_u8rgb: coeffs not 4-byte aligned");
+  MA_REQUIRE((reinterpret_cast<uintptr_t>(out_chw) & 3) == 0, "ma_resample_v_norm_u8rgb: out_chw not 4-byte aligned");
   const float m0 = mean_host ? mean_host[0] : 0.f, m1 = mean_host ? mean_host[1] : 0.f, m2 = mean_host ? mean_host[2] : 0.f;
   const float s0 = std_host ? std_host[0] : 1.f, s1 = std_host ? std_host[1] : 1.f, s2 = std_host ? std_host[2] : 1.f;
   dim3 grid((cols + 127) / 128, th, n);

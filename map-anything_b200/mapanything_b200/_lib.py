@@ -84,6 +84,7 @@ SIGNATURES = {
     "ma_set_stream_k": (_i, [_i]),
     "ma_last_gemm_block": (_i, []),
     "ma_last_attention_kernel": (_i, []),
+    "ma_last_resample_kernel": (_i, []),
     "ma_gemm_bf16": (_i, [_p, _i64, _p, _i64, _i, _i, _i, C.POINTER(GemmEpilogue), _i, _p]),
     "ma_conv3x3_bf16": (_i, [_p, _i, _i, _i, _i, _p, _i64, _i, C.POINTER(GemmEpilogue), _i, _p]),
     "ma_attention_fwd": (_i, [_p, _i64, _i64, _i, _p, _i64, _i64, _i, _p, _i64, _i, _p, _i64, _i, _i, _i, _i, _i, _i64,

@@ -339,8 +339,12 @@ def _camera_matrix_of_crop(K: np.ndarray, input_resolution, output_resolution, s
 
 
 def _image_to_device_u8(img, view_idx: int, dev: torch.device, up: _Uploader) -> torch.Tensor:
-    """The image forms preprocess_inputs accepts (image.py:493-521) as a CUDA uint8 (H, W, 3) tensor.  Host inputs are
-    converted with the reference's own expressions; CUDA float tensors with ma_f32_to_u8."""
+    """The image forms preprocess_inputs accepts (image.py:493-521) as a CUDA uint8 (H, W, 3) tensor.  Tensors are converted
+    as the reference does, (img * 255).clamp(0, 255).byte() when img.max() <= 1 else img.clamp(0, 255).byte(), evaluated in
+    the tensor's own dtype: host tensors with that expression before the upload, CUDA fp32 tensors with ma_f32_to_u8 (the same
+    fp32 multiply, clamp and truncation), CUDA uint8 tensors as they are unless they hold only 0s and 1s, and every other
+    CUDA dtype with the expression on the device (a fp16 image rounds img * 255 to fp16 and a fp64 image keeps fp64, so an
+    fp32 kernel would give other bytes)."""
     import PIL.Image
 
     if isinstance(img, torch.Tensor):
@@ -351,13 +355,15 @@ def _image_to_device_u8(img, view_idx: int, dev: torch.device, up: _Uploader) ->
                 return up.upload((img * 255).clamp(0, 255).byte().numpy())
             return up.upload(img.clamp(0, 255).byte().numpy())
         img = img.to(dev)
+        in_unit_range = bool(img.max() <= 1.0)
         if img.dtype == torch.uint8:
-            return img.contiguous()
-        x = img.contiguous().float()
+            return (img * 255 if in_unit_range else img).contiguous()
+        if img.dtype != torch.float32:
+            return ((img * 255).clamp(0, 255) if in_unit_range else img.clamp(0, 255)).byte().contiguous()
+        x = img.contiguous()
         out = torch.empty(x.shape, device=dev, dtype=torch.uint8)
-        scale = 255.0 if float(x.max()) <= 1.0 else 1.0
-        check(_lib.load().ma_f32_to_u8(x.data_ptr(), x.numel(), scale, out.data_ptr(), torch.cuda.current_stream().cuda_stream),
-              "ma_f32_to_u8")
+        check(_lib.load().ma_f32_to_u8(x.data_ptr(), x.numel(), 255.0 if in_unit_range else 1.0, out.data_ptr(),
+                                       torch.cuda.current_stream().cuda_stream), "ma_f32_to_u8")
         ops._count()
         return out
     if isinstance(img, np.ndarray):
