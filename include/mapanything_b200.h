@@ -390,6 +390,58 @@ int ma_gather_rows_cols_f32(const float* src, int64_t src_row_stride, const int3
  * in must be 4-byte aligned. */
 int ma_f32_to_u8(const float* in, int64_t n, float scale, uint8_t* out, void* stream);
 
+/* ---- load_images(): baseline JPEG decoding on the GPU ------------------------------------------------------------
+ * The reference decodes every file with exif_transpose(PIL.Image.open(f)).convert("RGB") (image.py:134-332), i.e.
+ * libjpeg-turbo's default decode: JDCT_ISLOW integer IDCT, fancy upsampling, no merged upsampler, table-driven
+ * YCbCr -> RGB.  These entry points reproduce that decode bit for bit for sequential Huffman 8-bit frames with one
+ * component or three YCbCr components sampled 4:4:4, 4:2:2, 4:2:0 or 4:4:0; the caller decodes every other file, and
+ * every frame ma_jpeg_decode reports, with Pillow. */
+#define MA_JPEG_SUBSEQ_BYTES 128 /* entropy-coded bytes per subsequence of the parallel Huffman decode */
+
+typedef struct ma_jpeg_info {
+  int32_t width, height;       /* frame size before EXIF orientation */
+  int32_t ncomp;               /* 1 (grayscale) or 3 (YCbCr) */
+  int32_t h_samp, v_samp;      /* luma sampling factors (chroma is 1x1); 1x1 for grayscale */
+  int32_t restart_interval;    /* MCUs per restart interval, 0 = none */
+  int32_t nsegments;           /* restart intervals of the scan */
+  int32_t nsubseq;             /* subsequences of MA_JPEG_SUBSEQ_BYTES */
+  int64_t nblocks;             /* 8x8 coefficient blocks of the scan */
+  int64_t plane_bytes;         /* bytes of the frame's sample planes in the workspace */
+  int64_t blob_bytes;          /* size of the device blob ma_jpeg_parse writes */
+} ma_jpeg_info;
+
+/* HOST function (no CUDA): reads the markers of a JPEG file (file_host, size bytes): SOI, SOF0 / SOF1, DQT, DHT, DRI,
+ * APP0 (JFIF), APP14 (Adobe), other APPn / COM skipped, one SOS, entropy-coded data, EOI.  Fills *info; with
+ * blob_host != NULL also writes the self-contained device blob (header with the Huffman lookup + canonical tables, the
+ * quantisation tables in natural order, restart-interval and subsequence tables, and the entropy-coded bytes with the
+ * FF00 stuffing and RSTn markers removed), which needs blob_capacity >= info->blob_bytes; with a smaller capacity the
+ * call still fills *info and returns MA_ERR_INVALID, so the caller can retry with info->blob_bytes.  With blob_capacity
+ * >= size + 16384 the entropy-coded data is read once, straight into the blob.  Returns MA_ERR_INVALID with a
+ * message for: no SOI; a truncated segment or a stream that does not end in EOI; any SOF other than SOF0 / SOF1
+ * (progressive, lossless, arithmetic); precision other than 8; 2 or 4 or more components; three components that are not
+ * YCbCr (Adobe transform != 1, or 'R','G','B' ids without JFIF) or not sampled as above; a zero frame height (DNL);
+ * quantisation or Huffman table indices above 3, a table class above 1, or a scan that refers to a missing table; a
+ * Huffman table that is not a valid prefix code (more codes of a length than fit, a code of all 1-bits, more than 256
+ * symbols) or a DC symbol above 15;
+ * a scan that does not cover every component in frame order, or that is not Ss = 0, Se = 63, Ah = Al = 0; restart
+ * markers out of sequence, without DRI, or not one per restart interval; a second scan or any other marker. */
+int ma_jpeg_parse(const uint8_t* file_host, int64_t size, ma_jpeg_info* info, uint8_t* blob_host, int64_t blob_capacity);
+
+/* Device workspace ma_jpeg_decode needs for these n frames (infos: HOST array). */
+int ma_jpeg_workspace(const ma_jpeg_info* infos, int n, int64_t* bytes);
+
+/* Decodes n frames in one set of launches.  blobs: device copy of the blobs of ma_jpeg_parse, frame i at byte offset
+ * blob_offsets_host[i] (16-byte aligned; blobs 16-byte aligned); infos_host: their infos.  out_host[i]: device pointer
+ * of frame i's packed RGB output, (H', W', 3) bytes where (W', H') is the frame size after orientation_host[i] (EXIF
+ * orientation 1-8; 5-8 swap width and height; other values = 1).  workspace: at least ma_jpeg_workspace bytes,
+ * 256-byte aligned.  status: device int32[n], 4-byte aligned, written with 0 for a frame decoded exactly, else a
+ * nonzero bit set (1: the entropy-coded data is invalid or holds the wrong number of blocks; 2: the parallel Huffman
+ * decode did not synchronise; 4: coefficients outside the range in which every libjpeg-turbo islow IDCT agrees); the
+ * output of such a frame is undefined.  n at most 65535. */
+int ma_jpeg_decode(const uint8_t* blobs, const int64_t* blob_offsets_host, const ma_jpeg_info* infos_host, int n,
+                   uint8_t* const* out_host, const int32_t* orientation_host, void* workspace, int64_t workspace_bytes,
+                   int32_t* status, void* stream);
+
 /* ---- infer() post-processing (reference mapanything/utils/inference.py:294-480, host numpy there) ---- */
 
 /* img_no_norm: clip(img * std + mean, 0, 1), (n,3,H,W) -> (n,H,W,3) fp32 (image.py:93-131). mean/std: 3 HOST floats. */

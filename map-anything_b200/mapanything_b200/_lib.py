@@ -71,6 +71,13 @@ class DecodeSpec(C.Structure):
                 ("use_factored", C.c_int), ("conf_vmin", C.c_float)]
 
 
+class JpegInfo(C.Structure):
+    """ma_jpeg_info (include/mapanything_b200.h)."""
+    _fields_ = [("width", C.c_int32), ("height", C.c_int32), ("ncomp", C.c_int32), ("h_samp", C.c_int32),
+                ("v_samp", C.c_int32), ("restart_interval", C.c_int32), ("nsegments", C.c_int32), ("nsubseq", C.c_int32),
+                ("nblocks", C.c_int64), ("plane_bytes", C.c_int64), ("blob_bytes", C.c_int64)]
+
+
 MA_REP = {"pointmap": 0, "raymap+depth": 1, "raydirs+depth+pose": 2, "campointmap+pose": 3, "pointmap+raydirs+depth+pose": 4}
 MA_PTS = {"linear": 0, "exp": 1, "z_exp": 2}
 
@@ -129,6 +136,10 @@ SIGNATURES = {
     "ma_gather_rows_cols_f32": (_i, [_p, _i64, _p, _p, _i, _i, _p, _p]),
     "ma_f32_to_u8": (_i, [_p, _i64, _f, _p, _p]),
     "ma_resample_v_norm_u8rgb": (_i, [_p, _i, _i, _i, _i, _p, _p, _i, _i, _i, _i, _p, _p, _p, _p, _p]),
+    "ma_jpeg_parse": (_i, [_p, _i64, C.POINTER(JpegInfo), _p, _i64]),
+    "ma_jpeg_workspace": (_i, [C.POINTER(JpegInfo), _i, C.POINTER(_i64)]),
+    "ma_jpeg_decode": (_i, [_p, C.POINTER(_i64), C.POINTER(JpegInfo), _i, C.POINTER(_p), C.POINTER(C.c_int32), _p, _i64, _p,
+                            _p]),
 }
 
 _lib = None

@@ -3,7 +3,8 @@ resize / crop / normalise on the GPU.
 
 The reference decodes every file with Pillow, resizes it with PIL.Image.resize (LANCZOS when shrinking, BICUBIC when
 enlarging; cropping.py:188-275), centre-crops (cropping.py:385-467) and normalises with torchvision (image.py:291-296),
-all on the host.  Here the file is still DECODED on the host (Pillow), then the raw RGB bytes go to the device once and
+all on the host.  Here baseline JPEG files are decoded on the GPU (csrc/jpeg.cu, bit for bit Pillow's libjpeg-turbo
+decode; only the compressed stream is uploaded) and every other file with Pillow, whose RGB bytes are uploaded; then
 two integer kernels (csrc/image.cu) reproduce Pillow's 8-bit resampling bit for bit, fused with the crop and the
 normalisation: the returned views hold `img` as a CUDA fp32 (1, 3, H, W) tensor that `MapAnything.infer` consumes without
 another host->device copy.  There is no host fallback for the resize.
@@ -182,6 +183,96 @@ class _Uploader:
         return dst
 
 
+def jpeg_parse(data: bytes, with_blob: bool = True):
+    """ma_jpeg_parse: (JpegInfo, uint8 blob or None), or None when the file is not a baseline frame the GPU decodes."""
+    lib = _lib.load()
+    info = _lib.JpegInfo()
+    buf = np.frombuffer(data, np.uint8)
+    if not with_blob:
+        return (info, None) if lib.ma_jpeg_parse(buf.ctypes.data, buf.size, C.byref(info), None, 0) == _lib.MA_OK else None
+    # one pass over the file: a blob of this capacity takes the unstuffed data directly (the tables after it are about a
+    # tenth of it; a file with more, e.g. a restart marker every few bytes, is parsed again into a blob of the exact size)
+    blob = np.empty(buf.size + buf.size // 2 + (1 << 16), np.uint8)
+    info.blob_bytes = 0
+    if lib.ma_jpeg_parse(buf.ctypes.data, buf.size, C.byref(info), blob.ctypes.data, blob.size) != _lib.MA_OK:
+        if info.blob_bytes <= blob.size:
+            return None
+        blob = np.empty(info.blob_bytes, np.uint8)
+        check(lib.ma_jpeg_parse(buf.ctypes.data, buf.size, C.byref(info), blob.ctypes.data, blob.size), "ma_jpeg_parse")
+    return info, blob[:info.blob_bytes]
+
+
+class _JpegBatch:
+    """Frames waiting for one ma_jpeg_decode call: their blobs, infos, output slots and EXIF orientations.  The batch is
+    decoded when its device workspace would pass `budget` bytes (coefficients + sample planes: ~130 B per pixel of a
+    4:4:4 frame), so the memory it takes stays bounded like the slabs'."""
+
+    def __init__(self, up: "_Uploader", budget: int = 1 << 30):
+        self.up, self.budget = up, budget
+        self.items: list = []   # (blob, info, out tensor, orientation, payload)
+        self.ws_bytes = 0
+
+    @staticmethod
+    def _ws(info) -> int:
+        return 128 * info.nblocks + info.plane_bytes + 32 * info.nsubseq
+
+    def add(self, blob, info, out: torch.Tensor, orientation: int, payload) -> list:
+        """Queues a frame; decodes the pending ones first when it would pass the budget (returns flush()'s list)."""
+        failed = self.flush() if self.items and self.ws_bytes + self._ws(info) > self.budget else []
+        self.items.append((blob, info, out, orientation, payload))
+        self.ws_bytes += self._ws(info)
+        return failed
+
+    def flush(self) -> list:
+        """Decodes the pending frames; returns the payloads of frames the decoder reported (to be decoded by Pillow)."""
+        if not self.items:
+            return []
+        items, self.items, self.ws_bytes = self.items, [], 0
+        n = len(items)
+        offs = np.cumsum([0] + [b.size for b, *_ in items])
+        cat = np.empty(int(offs[-1]), np.uint8)
+        for (b, *_), o in zip(items, offs):
+            cat[o:o + b.size] = b
+        d_blobs = self.up.upload(cat)
+        infos = (_lib.JpegInfo * n)(*[it[1] for it in items])
+        offsets = (C.c_int64 * n)(*[int(o) for o in offs[:-1]])
+        outs = (C.c_void_p * n)(*[it[2].data_ptr() for it in items])
+        orient = (C.c_int32 * n)(*[it[3] for it in items])
+        lib = _lib.load()
+        ws_bytes = C.c_int64(0)
+        check(lib.ma_jpeg_workspace(infos, n, C.byref(ws_bytes)), "ma_jpeg_workspace")
+        ws = torch.empty(ws_bytes.value, dtype=torch.uint8, device=self.up.device)
+        status = torch.empty(n, dtype=torch.int32, device=self.up.device)
+        check(lib.ma_jpeg_decode(d_blobs.data_ptr(), offsets, infos, n, outs, orient, ws.data_ptr(), ws_bytes.value,
+                                 status.data_ptr(), torch.cuda.current_stream().cuda_stream), "ma_jpeg_decode")
+        ops._count(30)
+        st = status.cpu().numpy()
+        ops.JPEG_ROUTES["gpu"] += int((st == 0).sum())
+        return [it[4] for it, s in zip(items, st) if s != 0]
+
+
+def _open_for_gpu(path: str):
+    """(blob, info, orientation) when the file goes to the GPU decoder: Pillow's header-only open reports a JPEG in mode
+    RGB or L, and ma_jpeg_parse accepts it (baseline sequential Huffman, 8-bit, grayscale or YCbCr 4:4:4 / 4:2:2 /
+    4:2:0 / 4:4:0).  The EXIF orientation is read through Pillow (getexif, with its XMP fallback) like exif_transpose."""
+    import PIL.Image
+
+    try:
+        with PIL.Image.open(path) as im:
+            if im.format != "JPEG" or im.mode not in ("RGB", "L"):
+                return None
+            orientation = im.getexif().get(0x0112, 1)
+    except Exception:  # noqa: BLE001  (Pillow's own route reports the error)
+        return None
+    with open(path, "rb") as fh:
+        data = fh.read()
+    parsed = jpeg_parse(data)
+    if parsed is None:
+        return None
+    info, blob = parsed
+    return blob, info, orientation if orientation in (2, 3, 4, 5, 6, 7, 8) else 1
+
+
 _RESIZE_MODES = ["fixed_mapping", "longest_side", "square", "fixed_size"]
 
 
@@ -259,40 +350,70 @@ def load_images(
 
     exts = [".jpg", ".jpeg", ".png"] + ([".heic", ".heif"] if heif_support_enabled else [])
     exts = tuple(exts)
-    # first pass: decode on the host (Pillow, like the reference), start the uploads, collect aspect ratios
+    # first pass: decode baseline JPEGs on the GPU and every other file on the host (Pillow, like the reference), start
+    # the uploads, collect aspect ratios
     up = _Uploader(dev)
+    jpegs = _JpegBatch(up)
     loaded, aspect_ratios = [], []
     slabs: Dict[Tuple[int, int], List[list]] = {}   # (W, H) -> [[device tensor (cap, H, W, 3), frames used], ...]
     slab_bytes = 256 << 20                          # frames per slab = what fits 256 MB (at least 1, at most 64)
+
+    def slot(W1: int, H1: int, path: str) -> torch.Tensor:
+        # frames of one size are uploaded side by side, so the resize runs as one batched launch per slab
+        lst = slabs.setdefault((W1, H1), [])
+        if not lst or lst[-1][1] == lst[-1][0].shape[0]:
+            cap = max(1, min(64, slab_bytes // (H1 * W1 * 3)))
+            lst.append([torch.empty(cap, H1, W1, 3, dtype=torch.uint8, device=dev), 0])
+        slab = lst[-1]
+        loaded.append([path, (W1, H1), len(lst) - 1, slab[1], W1, H1])
+        slab[1] += 1
+        aspect_ratios.append(W1 / H1)
+        return slab[0][slab[1] - 1]
+
+    def pillow_decode(path: str):
+        if bayer_format:
+            import cv2
+
+            color_bayer = cv2.imread(os.path.join(root, path), cv2.IMREAD_UNCHANGED)
+            img = PIL.Image.fromarray(cv2.cvtColor(color_bayer, cv2.COLOR_BAYER_RG2BGR))
+            return exif_transpose(img).convert("RGB")
+        return exif_transpose(PIL.Image.open(os.path.join(root, path))).convert("RGB")
+
+    def redo_with_pillow(entries: list) -> None:
+        # frames the GPU decoder reported: Pillow decodes them into the same slot, or the file is skipped like any
+        # other file Pillow cannot read
+        for entry in entries:
+            path, key, si, fi = entry[:4]
+            try:
+                up.upload(np.asarray(pillow_decode(path)), slabs[key][si][0][fi])
+                ops.JPEG_ROUTES["pillow"] += 1
+            except Exception as e:  # noqa: BLE001
+                if verbose:
+                    print(f"Warning: Could not load {path}: {e}")
+                k = next(i for i, x in enumerate(loaded) if x is entry)
+                del loaded[k], aspect_ratios[k]
+
     with torch.cuda.device(dev):
         for i, path in enumerate(folder_content):
             if i % stride != 0 or not path.lower().endswith(exts):
                 continue
+            gpu = None if bayer_format else _open_for_gpu(os.path.join(root, path))
+            if gpu is not None:
+                blob, info, orientation = gpu
+                W1, H1 = (info.height, info.width) if orientation >= 5 else (info.width, info.height)
+                out = slot(W1, H1, path)
+                redo_with_pillow(jpegs.add(blob, info, out, orientation, loaded[-1]))
+                continue
             try:
-                if bayer_format:
-                    import cv2
-
-                    color_bayer = cv2.imread(os.path.join(root, path), cv2.IMREAD_UNCHANGED)
-                    img = PIL.Image.fromarray(cv2.cvtColor(color_bayer, cv2.COLOR_BAYER_RG2BGR))
-                    img = exif_transpose(img).convert("RGB")
-                else:
-                    img = exif_transpose(PIL.Image.open(os.path.join(root, path))).convert("RGB")
+                img = pillow_decode(path)
                 W1, H1 = img.size
-                arr = np.asarray(img)
-                # frames of one size are uploaded side by side, so the resize runs as one batched launch per slab
-                lst = slabs.setdefault((W1, H1), [])
-                if not lst or lst[-1][1] == lst[-1][0].shape[0]:
-                    cap = max(1, min(64, slab_bytes // (H1 * W1 * 3)))
-                    lst.append([torch.empty(cap, H1, W1, 3, dtype=torch.uint8, device=dev), 0])
-                slab = lst[-1]
-                up.upload(arr, slab[0][slab[1]])
-                loaded.append((path, (W1, H1), len(lst) - 1, slab[1], W1, H1))
-                slab[1] += 1
-                aspect_ratios.append(W1 / H1)
+                up.upload(np.asarray(img), slot(W1, H1, path))
+                ops.JPEG_ROUTES["pillow"] += 1
             except Exception as e:  # noqa: BLE001  (the reference skips unreadable files the same way)
                 if verbose:
                     print(f"Warning: Could not load {path}: {e}")
                 continue
+        redo_with_pillow(jpegs.flush())
         if not loaded:
             raise ValueError("No valid images found")
         target_size = _target_size(aspect_ratios, resize_mode, size, patch_size, resolution_set, verbose)

@@ -17,6 +17,8 @@ from ._lib import (MA_ACT_GELU, MA_ACT_NONE, MA_ACT_RELU, MA_ATTN_MAX_SEGMENTS, 
                    MA_ATTN_STATE_OUT, MA_BF16, MA_F32, AttnExt, GemmEpilogue, check)
 
 LAUNCHES = 0
+# files load_images decoded on the GPU (ma_jpeg_decode) and with Pillow
+JPEG_ROUTES = {"gpu": 0, "pillow": 0}
 PROFILE = None
 # weight data_ptr -> (algorithmic N, algorithmic K) for packed weights whose stored shape is larger than the reference layer's:
 # K zero-padded for TMA alignment (patch embed 588 -> 640, conv channels to multiples of 8) or tripled by the split-bf16
