@@ -11,8 +11,10 @@
 //                          coefficients and their byte planes
 //   * resample_h_dp4a_kernel  one block per source row: the row is staged in shared memory with 4-byte coalesced loads and
 //                          split into R / G / B byte planes; every thread produces output pixels of that row with dp4a on
-//                          byte-split coefficients.  resample_h_vec_kernel (32-bit loads + PRMT) and resample_h_kernel
-//                          (byte loads, any window length) are the earlier forms, kept as fallbacks / for A/B runs
+//                          byte-split coefficients.  Runs when the caller passes the packed coefficients, the window has
+//                          at most 64 taps and the staged span fits shared memory.  Otherwise resample_h_vec_kernel
+//                          (32-bit loads + PRMT) runs for windows of at most 64 taps, and resample_h_kernel (byte loads,
+//                          any window length) for longer windows or spans too wide for the other two
 //   * resample_v_norm_kernel  thread per output pixel of the CROPPED target: vertical pass over the 8-bit
 //                          intermediate (taps are row-contiguous across a warp), byte clamp, (u/255 - mean)/std in the
 //                          rounding order of torchvision, planar fp32 (3,H,W) output = the model's `img` layout
@@ -20,7 +22,6 @@
 // By bytes this is HBM work (a 1920x1080 frame: 6.2 MB in, 1.7 MB intermediate, 1.8 MB out); in practice the integer
 // pipes bound it (25-tap LANCZOS windows at this reduction), see DESIGN.md section 5 for the measured forms.
 #include <math.h>
-#include <stdlib.h>
 
 #include <vector>
 
@@ -423,16 +424,8 @@ extern "C" int ma_resample_h_u8rgb(const uint8_t* src, int64_t src_row_stride, i
   MA_REQUIRE((reinterpret_cast<uintptr_t>(coeffs) & 3) == 0, "ma_resample_h_u8rgb: coeffs not 4-byte aligned");
   MA_REQUIRE((reinterpret_cast<uintptr_t>(packed) & 3) == 0, "ma_resample_h_u8rgb: packed not 4-byte aligned");
   cudaStream_t st = static_cast<cudaStream_t>(stream);
-  static const bool byte_loads = [] {  // MA_RESAMPLE_BYTE_LOADS=1: the first kernel (byte loads, any window length), for A/B runs
-    const char* e = getenv("MA_RESAMPLE_BYTE_LOADS");
-    return e && e[0] == '1';
-  }();
   const int64_t row_bytes = static_cast<int64_t>(sx1 - sx0) * 3;
-  static const bool no_dp4a = [] {  // MA_RESAMPLE_DP4A=0: ignore the packed coefficients (A/B runs)
-    const char* e = getenv("MA_RESAMPLE_DP4A");
-    return e && e[0] == '0';
-  }();
-  if (packed && !no_dp4a && !byte_loads && ksize <= 64 && row_bytes + 1024 <= 180 * 1024) {
+  if (packed && ksize <= 64 && row_bytes + 1024 <= 180 * 1024) {
 #define MA_H_DP4A(W) \
   case W:            \
     return launch_h_dp4a<W>(src, src_row_stride, src_frame_stride, n, y0, rows, sx0, sx1, bounds, packed, out_size, x0, cols, tmp, st)
@@ -443,7 +436,7 @@ extern "C" int ma_resample_h_u8rgb(const uint8_t* src, int64_t src_row_stride, i
     }
 #undef MA_H_DP4A
   }
-  if (!byte_loads && ksize <= 64 && row_bytes + 512 <= 200 * 1024) {
+  if (ksize <= 64 && row_bytes + 512 <= 200 * 1024) {
 #define MA_H_VEC(K) \
   case K / 4:       \
     return launch_h_vec<K>(src, src_row_stride, src_frame_stride, n, y0, rows, sx0, sx1, bounds, coeffs, out_size, x0, cols, tmp, st)

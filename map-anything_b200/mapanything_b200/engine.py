@@ -21,6 +21,11 @@ from . import ops
 from .ops import MA_ACT_GELU, MA_ACT_NONE, MA_ACT_RELU
 
 
+# views per DPT pass (bounds the activation scratch: ~0.6 GB per view at 518 px).  8 instead of 4: same-box A/B at 8 views
+# 311.1 vs 301.6 views/s (fewer, larger launches)
+DPT_CHUNK = 8
+
+
 def _bf16(t: torch.Tensor) -> torch.Tensor:
     return t.detach().to(torch.bfloat16).contiguous()
 
@@ -172,6 +177,8 @@ class BlockW:
 class Engine:
     """Owns the packed weights of one MapAnything module on one CUDA device."""
 
+    encoder_streams = 1   # not read by the package; bench.py pins it to 1 around its instrumented pass
+
     def __init__(self, model: nn.Module):
         self.device = next(model.parameters()).device
         if self.device.type != "cuda":
@@ -228,18 +235,8 @@ class Engine:
         if self.head_type == "dpt+pose":
             self._init_pose(model)
         self.scale_mlp = [Lin3(m.weight, m.bias) for m in model.scale_head.mlp if isinstance(m, nn.Linear)]
-        import os
-
-        # view groups of the encoder on separate CUDA streams: +1 % before programmatic dependent launch existed, equal with
-        # it, and now slower than one stream (same-box A/B at 8 views: 327-328 views/s with two, 332 with one, 335 with one
-        # and the persistent two-stream attention kernel, which wants all views in one launch)
-        self.encoder_streams = max(1, int(os.environ.get("MA_ENCODER_STREAMS", "1")))
         self.sm_count = torch.cuda.get_device_properties(self.device).multi_processor_count
-        # views per DPT pass (bounds the activation scratch: ~0.6 GB per view at 518 px).  8 instead of 4: same-box A/B at 8
-        # views 311.1 vs 301.6 views/s (fewer, larger launches); MA_DPT_CHUNK overrides for A/B runs
-        self.dpt_chunk_default = max(1, int(os.environ.get("MA_DPT_CHUNK", "8")))
-        self.dpt_chunk = self.dpt_chunk_default
-        self.proj_block_n = int(os.environ.get("MA_PROJ_BN", "0"))   # A/B knob: tile code of the attention-projection GEMMs
+        self.dpt_chunk = DPT_CHUNK   # views per DPT pass; the model lowers it for memory_efficient_inference
         # measurement aid (bench.py `strong` record): when a list, every sharded global block appends the CUDA events that
         # bracket its wait for the K/V all-gather on the compute stream
         self.ag_wait_events = None
@@ -265,12 +262,9 @@ class Engine:
         reg = model.dpt_regressor_head
         self.reg1, self.reg2, self.reg3 = _conv3x3(reg.conv1), _conv3x3(reg.conv2[0]), _conv1x1(reg.conv2[2])
         # the last 1x1 conv (hidden -> 6) as the epilogue of the 3x3 conv in front of it (ma_gemm_epilogue.head_*): fp32
-        # weights [8][128] (the kernel form needs hidden = 128 and <= 8 outputs; MA_FUSED_HEAD=0 keeps the separate kernel)
-        import os as _os2
-
-        self.reg3_fused = None
+        # weights [8][128] (the kernel form needs hidden = 128 and <= 8 outputs; other heads run the 1x1 conv separately)
         w3 = reg.conv2[2].weight.detach().reshape(reg.conv2[2].weight.shape[0], -1)
-        if w3.shape[1] == 128 and w3.shape[0] <= 8 and self.reg2.n == 128 and _os2.environ.get("MA_FUSED_HEAD", "1") != "0":
+        if w3.shape[1] == 128 and w3.shape[0] <= 8 and self.reg2.n == 128:
             hw = torch.zeros(8, 128, device=self.device, dtype=torch.float32)
             hb = torch.zeros(8, device=self.device, dtype=torch.float32)
             hw[:w3.shape[0]] = w3.float()
@@ -280,30 +274,26 @@ class Engine:
 
     def _init_pose(self, model):
         ph = model.pose_head
-        self.pose_relu_after_skip = bool(getattr(ph, "final_relu_after_skip", True))
-        self.pose_blocks = []
-        for rb in ph.res_conv:
-            if not isinstance(rb.head_skip, nn.Identity):
-                raise ValueError("pose head with a projecting skip is not part of the released config")
-            # pose + scale heads run in split-bf16 (~fp32) precision: their outputs are normalised / exponentiated and
-            # the reference computes them with autocast disabled (model.py:1599)
-            cin = rb.res_conv2.weight.shape[1]
-            self.pose_blocks.append((
-                Lin3(rb.res_conv1.weight, rb.res_conv1.bias),
-                Lin3(rb.res_conv2.weight.detach().permute(0, 2, 3, 1), rb.res_conv2.bias, group=cin),
-                Lin3(rb.res_conv3.weight, rb.res_conv3.bias),
-            ))
-        # MA_POSE_HEAD=bf16 (default): the three convolutions of each ResConvBlock run with plain bf16 operands (fp32
+        if not all(isinstance(rb.head_skip, nn.Identity) for rb in ph.res_conv):
+            raise ValueError("pose head with a projecting skip is not part of the released config")
+        # The pose and scale heads run in split-bf16 (~fp32) precision: their outputs are normalised / exponentiated and
+        # the reference computes them with autocast disabled (model.py:1599).  The exception are the three convolutions of
+        # each ResConvBlock of the released wiring, relu(skip + conv3(y)): they run with plain bf16 operands (fp32
         # accumulate, fp32 residual chain) -- they act on 1369 tokens per view whose average is what the MLPs see, so bf16
         # rounding averages out (measured: rotation / translation error vs the fp32 oracle unchanged, DESIGN.md section 4),
-        # and the split-bf16 form cost 3x the MMA work (1.05 ms of a 26 ms step).  The pooled MLPs and the output layer,
-        # whose results are normalised / exponentiated, stay in split-bf16 (~fp32).  MA_POSE_HEAD=split restores round 1.
-        import os as _os
-
-        self.pose_bf16 = _os.environ.get("MA_POSE_HEAD", "bf16") != "split"
-        self.pose_blocks_bf16 = [(
-            Lin(rb.res_conv1.weight, rb.res_conv1.bias), _conv3x3(rb.res_conv2), Lin(rb.res_conv3.weight, rb.res_conv3.bias),
-        ) for rb in ph.res_conv]
+        # and the split-bf16 form cost 3x the MMA work (1.05 ms of a 26 ms step).  The other wiring, skip + relu(conv3(y)),
+        # keeps split-bf16 blocks.
+        self.pose_relu_after_skip = bool(getattr(ph, "final_relu_after_skip", True))
+        if self.pose_relu_after_skip:
+            self.pose_blocks = [(
+                Lin(rb.res_conv1.weight, rb.res_conv1.bias), _conv3x3(rb.res_conv2), Lin(rb.res_conv3.weight, rb.res_conv3.bias),
+            ) for rb in ph.res_conv]
+        else:
+            self.pose_blocks = [(
+                Lin3(rb.res_conv1.weight, rb.res_conv1.bias),
+                Lin3(rb.res_conv2.weight.detach().permute(0, 2, 3, 1), rb.res_conv2.bias, group=rb.res_conv2.weight.shape[1]),
+                Lin3(rb.res_conv3.weight, rb.res_conv3.bias),
+            ) for rb in ph.res_conv]
         self.pose_mlp = [Lin3(ph.more_mlps[0].weight, ph.more_mlps[0].bias), Lin3(ph.more_mlps[2].weight, ph.more_mlps[2].bias)]
         self.pose_out = Lin3(torch.cat([ph.fc_t.weight, ph.fc_rot.weight], 0), torch.cat([ph.fc_t.bias, ph.fc_rot.bias], 0))
 
@@ -410,7 +400,7 @@ class Engine:
         else:
             ops.attention(qkv[:, :dim], qkv[:, dim:2 * dim], qkv[:, 2 * dim:], a, num_heads=heads, num_seqs=num_seqs,
                           q_len=seq_len, kv_len=seq_len, q_seq_stride=seq_stride, kv_seq_stride=seq_stride, scale=scale)
-        ops.gemm(a, bw.proj.w, xr, bias=bw.proj.b, colscale=bw.ls1, residual=xr, block_n=self.proj_block_n)
+        ops.gemm(a, bw.proj.w, xr, bias=bw.proj.b, colscale=bw.ls1, residual=xr)
         ops.layernorm(xr, h, bw.n2w, bw.n2b)
         f = self._lin(h, bw.fc1, act=MA_ACT_GELU)
         ops.gemm(f, bw.fc2.w, xr, bias=bw.fc2.b, colscale=bw.ls2, residual=xr)
@@ -482,38 +472,16 @@ class Engine:
         pos0 = pos[0].contiguous()
         imgs = imgs.contiguous()
         feat = self._empty(n * N, self.C, dtype=torch.float32)
-        # The encoder is independent per view: run it as `groups` batches of views on separate CUDA streams, issued
-        # block by block in turn.  Every kernel here is a persistent grid over all SMs whose last wave leaves SMs idle
-        # (2.3 - 5.2 waves per launch at 8 views); the other group's next kernel fills that tail.
-        groups = self.encoder_streams if n >= 2 * self.encoder_streams else 1
-        main = torch.cuda.current_stream()
-        bounds = [(g * n) // groups for g in range(groups + 1)]
-        streams = [main] if groups == 1 else self._side_streams(groups)
-        xs = []
-        for g in range(groups):
-            lo, ng = bounds[g], bounds[g + 1] - bounds[g]
-            if groups > 1:
-                streams[g].wait_stream(main)
-            with torch.cuda.stream(streams[g]):
-                a = self._empty(ng * N, self.kpad)
-                ops.patchify(imgs[lo:lo + ng], a, p)
-                x = self._empty(ng * (N + 1), self.C, dtype=torch.float32)
-                ops.gemm(a, self.patch_embed.w, x, bias=self.patch_embed.b, residual=pos[1:], residual_row_mod=N,
-                         rows_per_group_in=N, rows_per_group_out=N + 1, row_offset_out=1)
-                ops.set_rows(x, self.cls, pos0, groups=ng, group_stride=N + 1, row_offset=0)
-            xs.append(x)
+        a = self._empty(n * N, self.kpad)
+        ops.patchify(imgs, a, p)
+        x = self._empty(n * (N + 1), self.C, dtype=torch.float32)
+        ops.gemm(a, self.patch_embed.w, x, bias=self.patch_embed.b, residual=pos[1:], residual_row_mod=N,
+                 rows_per_group_in=N, rows_per_group_out=N + 1, row_offset_out=1)
+        ops.set_rows(x, self.cls, pos0, groups=n, group_stride=N + 1, row_offset=0)
         for bw in self.enc_blocks:
-            for g in range(groups):
-                ng = bounds[g + 1] - bounds[g]
-                with torch.cuda.stream(streams[g]):
-                    self._block(xs[g], bw, ng * (N + 1), self.enc_heads, ng, N + 1, N + 1)
-        for g in range(groups):
-            lo, ng = bounds[g], bounds[g + 1] - bounds[g]
-            with torch.cuda.stream(streams[g]):
-                ops.layernorm(xs[g], feat[lo * N:(lo + ng) * N], self.enc_nw, self.enc_nb, rows=ng * N, rows_per_group=N,
-                              in_group_stride=N + 1, in_row_offset=1, out_group_stride=N, out_row_offset=0)
-            if groups > 1:
-                main.wait_stream(streams[g])
+            self._block(x, bw, n * (N + 1), self.enc_heads, n, N + 1, N + 1)
+        ops.layernorm(x, feat, self.enc_nw, self.enc_nb, rows=n * N, rows_per_group=N,
+                      in_group_stride=N + 1, in_row_offset=1, out_group_stride=N, out_row_offset=0)
         return feat
 
     def _lin3(self, x32: torch.Tensor, lin: "Lin3", out: torch.Tensor, act: int = MA_ACT_NONE) -> torch.Tensor:
@@ -523,11 +491,6 @@ class Engine:
         if lin.w32 is not None and rows <= ops.LINEAR_ROWS_MAX and rows * k * 4 <= 48 * 1024 and k % 4 == 0:
             return ops.linear_rows_f32(x32, lin.w32, lin.b, out, act)
         return ops.gemm(ops.split3(x32), lin.w, out, bias=lin.b, act=act)
-
-    def _side_streams(self, k: int):
-        if len(getattr(self, "_streams", [])) < k:
-            self._streams = [torch.cuda.Stream(device=self.device) for _ in range(k)]
-        return self._streams[:k]
 
     # ------------------------------------------------------------------------------------------ stage 2
     def fuse_norm(self, feat: torch.Tensor) -> torch.Tensor:
@@ -718,13 +681,13 @@ class Engine:
         ops.bilinear_ac(o, up, virtual_hw=up_virtual)
         return up
 
-    def pose_head(self, x32: torch.Tensor, n: int, hp: int, wp: int, out: torch.Tensor, x16: Optional[torch.Tensor] = None):
+    def pose_head(self, x32: torch.Tensor, n: int, hp: int, wp: int, out: torch.Tensor, x16: torch.Tensor):
         """x32 fp32 [n*N][D] (final info-sharing features; x16 = the same in bf16) -> out fp32 [n][7] = (t | q)."""
         N = hp * wp
         D = x32.shape[1]
-        if self.pose_bf16 and self.pose_relu_after_skip and x16 is not None:
+        if self.pose_relu_after_skip:
             xb = x16
-            for c1, c2, c3 in self.pose_blocks_bf16:
+            for c1, c2, c3 in self.pose_blocks:
                 u = self._lin(xb, c1, act=MA_ACT_RELU)
                 u2 = self._conv3(u.view(n, hp, wp, c1.n), c2, act=MA_ACT_RELU).reshape(n * N, c2.n)
                 xn = self._empty(n * N, c3.n, dtype=torch.float32)
@@ -744,7 +707,7 @@ class Engine:
         return out
 
     def _pose_blocks_split(self, x32: torch.Tensor, n: int, hp: int, wp: int) -> torch.Tensor:
-        """ResConvBlocks in split-bf16 (~fp32) precision."""
+        """ResConvBlocks skip + relu(conv3(y)) in split-bf16 (~fp32) precision."""
         N = hp * wp
         for c1, c2, c3 in self.pose_blocks:
             u = self._empty(n * N, c1.n, dtype=torch.float32)
@@ -753,8 +716,7 @@ class Engine:
             u2 = self._empty(n * N, c2.n, dtype=torch.float32)
             ops.conv3x3(us, c2.w, u2, bias=c2.b, act=MA_ACT_RELU)
             xn = self._empty(n * N, c3.n, dtype=torch.float32)
-            ops.gemm(ops.split3(u2), c3.w, xn, bias=c3.b, residual=x32, act=MA_ACT_RELU,
-                     act_after_residual=self.pose_relu_after_skip)
+            ops.gemm(ops.split3(u2), c3.w, xn, bias=c3.b, residual=x32, act=MA_ACT_RELU)
             x32 = xn
         return x32
 
@@ -803,20 +765,18 @@ class Engine:
             g1u = self._empty(n, H, W, g1.shape[3])
             ops.bilinear_ac(g1, g1u)
             rawv = raw[s * H * W:(s + n) * H * W]
-            if self.reg3_fused is not None and raw.shape[1] == 8:
+            if self.reg3_fused is not None:
                 ops.conv3x3_head(g1u, self.reg2.w, self.reg2.b, MA_ACT_RELU, self.reg3_fused[0], self.reg3_fused[1], rawv)
-                if with_pose:
-                    self.pose_head(final32[s * N:(s + n) * N], n, hp, wp, pose_raw[s:s + n], x16=t[3])
-                continue
-            g2 = self._conv3(g1u, self.reg2, act=MA_ACT_RELU)
-            g2f = g2.reshape(n * H * W, -1)
-            if self.reg3.n <= 8 and self.reg3.k <= 256 and self.reg3.k % 8 == 0:
-                ops.head_linear_small(g2f, self.reg3.w, self.reg3.b, rawv)   # 128 -> 6 per pixel: streaming kernel
             else:
-                ops.gemm(g2f, self.reg3.w, rawv[:, :self.reg3.n], bias=self.reg3.b)
-            # pose head on the final info-sharing features (split-bf16 precision)
+                g2 = self._conv3(g1u, self.reg2, act=MA_ACT_RELU)
+                g2f = g2.reshape(n * H * W, -1)
+                if self.reg3.n <= 8 and self.reg3.k <= 256 and self.reg3.k % 8 == 0:
+                    ops.head_linear_small(g2f, self.reg3.w, self.reg3.b, rawv)   # <= 8 outputs per pixel: streaming kernel
+                else:
+                    ops.gemm(g2f, self.reg3.w, rawv[:, :self.reg3.n], bias=self.reg3.b)
+            # pose head on the final info-sharing features
             if with_pose:
-                self.pose_head(final32[s * N:(s + n) * N], n, hp, wp, pose_raw[s:s + n], x16=t[3])
+                self.pose_head(final32[s * N:(s + n) * N], n, hp, wp, pose_raw[s:s + n], t[3])
         return raw, pose_raw
 
     def scale_head(self, tok_feat32: torch.Tensor) -> torch.Tensor:

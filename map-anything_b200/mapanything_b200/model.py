@@ -22,7 +22,7 @@ import torch.nn as nn
 
 from . import ops
 from . import params as P
-from .engine import Engine
+from .engine import DPT_CHUNK, Engine
 from .inference import (
     postprocess_model_outputs_for_inference,
     validate_input_views_for_inference,
@@ -552,8 +552,7 @@ class MapAnything(nn.Module, PyTorchModelHubMixin):
         if height % p or width % p:
             raise AssertionError(f"Input image size ({height}, {width}) must be a multiple of the patch size {p}")
         eng = self.engine()
-        eng.dpt_chunk = min(self._compute_adaptive_minibatch_size(), eng.dpt_chunk_default) if memory_efficient_inference \
-            else eng.dpt_chunk_default
+        eng.dpt_chunk = min(self._compute_adaptive_minibatch_size(), DPT_CHUNK) if memory_efficient_inference else DPT_CHUNK
         hp, wp = height // p, width // p
         N = hp * wp
         plan, comm = None, self._shard_comm

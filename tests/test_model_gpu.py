@@ -95,8 +95,17 @@ def _assert_within(ours, what, floor=None, factor=2.0):
         assert ours[k] <= bound, f"{what}: {k} = {ours[k]:.4g} exceeds {bound:.4g}"
 
 
-def test_stages_tiny_config():
-    """Stage by stage on the toy-width model with the hard weights (localises a failure to one kernel family)."""
+def _tiny_relu_before_skip():
+    from oracle.config import tiny_config
+
+    cfg = tiny_config()
+    cfg["pred_head_config"]["pose_head"]["final_relu_after_skip"] = False
+    return cfg
+
+
+def test_stages_tiny_config_both_pose_wirings():
+    """Stage by stage on the toy-width model with the hard weights (localises a failure to one kernel family); the pose
+    head under both ResConvBlock wirings, each of which runs its own form of the blocks (bf16 / split-bf16)."""
     from oracle.config import tiny_config
 
     oracle, model = _build(tiny_config, seed=0)
@@ -140,17 +149,21 @@ def test_stages_tiny_config():
         e = _rel(pose_raw, ref["pose_raw"])
         print(f"pose head raw rel err (oracle fp32 features in; bf16 convs, split-bf16 pooled MLPs) {e:.3e}")
         assert e < 2e-3   # 25 tokens per view here; the bf16 rounding of the convs averages over 1369 tokens at full size
-        eng.pose_bf16 = False   # round-1 form: every pose-head layer in split-bf16 (~fp32)
-        _, pose_split = eng.dpt_and_pose(otaps, V, hp, hp, 70, 70, final32=otaps32[3])
-        eng.pose_bf16 = True
-        e = _rel(pose_split, ref["pose_raw"])
-        print(f"pose head raw rel err, MA_POSE_HEAD=split {e:.3e}")
-        assert e < 1e-4
         scale_raw = eng.scale_head(ref["scale_token_feat"].reshape(1, -1).cuda().contiguous())
         ref_scale = oracle.scale_head(ref["scale_token_feat"]).reshape(-1)
         e = (scale_raw.cpu() - ref_scale).abs().max().item()
         print(f"scale head log-scale abs err {e:.3e}")
         assert e < 1e-4
+    # the wiring skip + relu(conv3(y)) runs every pose-head layer in split-bf16 (~fp32)
+    oracle, model = _build(_tiny_relu_before_skip, seed=0)
+    with torch.no_grad():
+        _, ref = oracle(views, return_internals=True)
+        otaps32 = [nchw(ref[k], ref[k].shape[1]).cuda().contiguous() for k in ("fused", "tap1", "tap2", "final")]
+        otaps = [t.bfloat16().contiguous() for t in otaps32]
+        _, pose_split = model.engine().dpt_and_pose(otaps, V, hp, hp, 70, 70, final32=otaps32[3])
+    e = _rel(pose_split, ref["pose_raw"])
+    print(f"pose head raw rel err, split-bf16 ResConvBlocks (oracle fp32 features in) {e:.3e}")
+    assert e < 1e-4
 
 
 def test_forward_tiny_reference_style_init_stated_tolerance():
